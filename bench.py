@@ -3,7 +3,7 @@
 bench.py -- belief x alpha backups/sec of the PBVI backup on the olfactory-navigation POMDP (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--beliefs B] [--alphas V]
-                    [--legs backup,solve,configs] [--scaling weak|strong] [--headline late|young|dense]
+                    [--legs backup,solve,configs] [--scaling weak|strong] [--headline late|young|dense] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...          (one rank per GPU)
 
 Workload (config.workload): BASELINE.json configs[2] -- the 22021-state toroidal olfactory model (A=6, O=3, R=1),
@@ -30,6 +30,8 @@ the ranks exchange + merge their generating tuples (pomdp_pbvi_exploration_b200.
                over the ranks at N > 1 (`PBVI_Solver.solve(group=...)`).
 `configs`      the other BASELINE configs (tiger, 4x4 grid, synthetic sparse sweep, sea-robin size), each with its own parity sample.
 --impl reference runs the CPU oracle as the reference arm on the b200 arm's alphas.
+--dump-outputs DIR writes the value function the last timed step of the headline point returned (dump_outputs()).  Every input is
+generated from fixed seeds, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -61,7 +63,9 @@ NCU_TRAFFIC_BYTES_PER_LAUNCH = {'young': 0.2400e9, 'late': 10.4627e9, 'dense': N
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=10,
+                    help='timed steps of the value-function point the line reports; the other points run max(3, steps // 2), '
+                         'the host-buffer leg runs steps')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--beliefs', type=int, default=10000, help='beliefs per GPU (weak scaling) or in total (--scaling strong)')
@@ -76,7 +80,14 @@ def parse_args():
     ap.add_argument('--only-point', default=None, help='measure one value-function point only (ncu passes)')
     ap.add_argument('--save-workload', default=None, help='write the synthetic beliefs / alphas to this .pt file')
     ap.add_argument('--load-workload', default=None, help='read them back instead of regenerating (ncu passes: no setup kernels)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write the value function the last timed backup step returned to DIR/*.npy (float64, at most 64 MB in all)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or (args.legs and 'backup' not in args.legs.split(','))):
+        ap.error('--dump-outputs needs the backup leg of --impl b200')
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -381,6 +392,31 @@ def host_tables(model) -> dict:
     return {'reach': model.reachable_states, 'rto': model.reachable_transitional_observation_table, 'rbar': model.expected_rewards_table}
 
 
+def dump_outputs(directory: str, vf, max_bytes: int = 64 << 20) -> dict:
+    """
+    Writes the ValueFunction a timed backup step returned, as float64 .npy files, so that two builds run with the same arguments can
+    be compared output for output:
+      actions.npy                      the action of every new alpha row;
+      alpha_vector_row_sums.npy        the sum over states of every new alpha row;
+      alpha_vector_array.npy           the rows themselves -- all of them, or, when they do not fit in `max_bytes` with the two
+                                       arrays above, a sample drawn with a fixed seed (sorted);
+      alpha_vector_array_rows.npy      the positions of those rows in the value function.
+    """
+    import torch
+    rows = vf.alpha_vector_array                         # summed and sampled where it lives: only the sampled rows are copied back
+    n, S = rows.shape
+    fit = max(0, (max_bytes - 4096 - 2 * n * 8) // ((S + 1) * 8))          # (4096: the four .npy headers)
+    pick = np.arange(n) if fit >= n else np.sort(np.random.default_rng(0).choice(n, fit, replace=False))
+    arrays = {'actions': np.asarray(vf.actions, dtype=np.float64), 'alpha_vector_row_sums': rows.sum(dim=1).cpu().numpy(),
+              'alpha_vector_array': rows[torch.as_tensor(pick, device=rows.device)].cpu().numpy(),
+              'alpha_vector_array_rows': pick.astype(np.float64)}
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + '.npy'), a)
+    return {'dir': directory, 'alpha_rows': n, 'alpha_rows_written': int(pick.size),
+            'bytes': int(sum(a.nbytes for a in arrays.values()))}
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def workload_config(args, world, headline=None, density=None):
     per_gpu = args.beliefs if args.scaling == 'weak' else -(-args.beliefs // world)
@@ -560,8 +596,8 @@ def run_b200(args):
         if args.only_point:
             order = [args.only_point]
         for name in order:
-            n_steps = args.steps if name == args.headline else max(3, args.steps // 2)
-            n_warm = args.warmup if name == args.headline else max(2, args.warmup // 2)
+            n_steps = args.steps if name == order[0] else max(3, args.steps // 2)        # order[0]: the point the line reports
+            n_warm = args.warmup if name == order[0] else max(2, args.warmup // 2)
             r = time_device_steps(make_step(vfs[name]), dev, n_steps, n_warm, barrier, sampler)
             r['steps'] = n_steps
             r['elapsed_ms'], r['score_ms'] = reduce_max([r['elapsed_ms'], r['score_ms']])
@@ -736,6 +772,8 @@ def run_b200(args):
         if rank == 0 and line is not None:
             line['configs'] = cfg
 
+    if args.dump_outputs and rank == 0:                   # (parse_args: the backup leg ran, `out` is its headline step's output)
+        line['dump_outputs'] = dump_outputs(args.dump_outputs, out)
     if rank == 0 and line is not None:
         emit(line)
     if world > 1:

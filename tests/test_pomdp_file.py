@@ -1,7 +1,7 @@
 """
 CPU tests of the Cassandra .POMDP reader / writer (pomdp_pbvi_exploration_b200.pomdp_file) against the tensors the
 reference's own loader + Model constructor produced (tests/golden/model_*.npz), on a hand-written tiger specification,
-on the reference's example files when its mount is present (authoring container only), and on round trips.
+on the reference's example files when a checkout of the reference is named by PBVI_REFERENCE_ROOT, and on round trips.
 """
 import os
 
@@ -11,7 +11,10 @@ import pytest
 from conftest import load_golden
 from pomdp_pbvi_exploration_b200.pomdp_file import load_POMDP_file, parse_POMDP, save_POMDP_file
 
-EXAMPLES = '/root/reference/Experiments/Example Models'
+# the example files ship with the reference (PimLb/POMDP_PBVI_Exploration), not with this repository
+EXAMPLES = os.path.join(os.environ.get('PBVI_REFERENCE_ROOT', ''), 'Experiments', 'Example Models')
+needs_examples = pytest.mark.skipif(not os.path.isabs(EXAMPLES) or not os.path.isdir(EXAMPLES),
+                                    reason="needs the reference's example .POMDP files: set PBVI_REFERENCE_ROOT to a checkout of the reference")
 
 TIGER = """
 # tiger: listen / open-left / open-right; hearing accuracy 0.85
@@ -67,7 +70,7 @@ def test_tiger_specification_matches_reference_tensors(tmp_path):
     _check_against_golden(model, 'tiger')
 
 
-@pytest.mark.skipif(not os.path.isdir(EXAMPLES), reason='reference example files only exist in the authoring container')
+@needs_examples
 @pytest.mark.parametrize('fname,tag', [('tiger.95.POMDP', 'tiger'), ('4x4.95.POMDP', 'grid4x4'), ('4x4.95-no_loop.POMDP', 'grid4x4_noloop'),
                                        ('tiger-grid.POMDP', 'tigergrid'), ('hallway.POMDP', 'hallway'), ('cheese.95.POMDP', 'cheese'),
                                        ('4x3.95.POMDP', 'grid4x3'), ('cit.POMDP', 'cit')])
@@ -77,7 +80,7 @@ def test_reference_example_files(fname, tag):
     _check_against_golden(model, tag)
 
 
-@pytest.mark.skipif(not os.path.isdir(EXAMPLES), reason='reference example files only exist in the authoring container')
+@needs_examples
 def test_every_example_file_parses_to_stochastic_tables():
     """All 18 bundled files parse (the reference's reader rejects parr95, saci-s12-a6-z5 and shuttle), rows are distributions."""
     files = sorted(f for f in os.listdir(EXAMPLES) if f.endswith('.POMDP'))
@@ -89,7 +92,9 @@ def test_every_example_file_parses_to_stochastic_tables():
         assert abs(spec["start"].sum() - 1.0) < 1e-4, f
 
 
-@pytest.mark.parametrize('tag', ['grid4x4', 'hallway'])
+# every model whose dense tables the reference's loader stored: the reader must give back exactly the reference's tensors
+@pytest.mark.parametrize('tag', ['tiger', 'grid4x4', 'grid4x4_noloop', 'tigergrid', 'hallway', 'cheese', 'grid4x3', 'hanks', 'network',
+                                 'maze4x5x2'])
 def test_round_trip(tmp_path, tag):
     from pomdp_pbvi_exploration_b200 import Model
     m = load_golden('model_' + tag)
