@@ -217,6 +217,18 @@ PBVI_API int pbvi_vi_sweep(pbvi_model* m, const double* d_vopt, double gamma, do
  * d_keep[i] = 1 iff alpha_i is >= everywhere by no vector other than itself. */
 PBVI_API int pbvi_prune_dominated(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, void* stream);
 
+/* ---- LP-domination prune (ValueFunction.prune level 3; the reference's intended Lark / White filter, src/mdp.py:834-906, whose
+ * branch fails on the undefined `pruned_alpha_set` at :872) ----------------------------------------------------------------------
+ * d_keep[i] = 0 iff a convex combination of the other rows exceeds alpha_i by more than tol = 1e-9*max(1, max|alpha|) at every
+ * state (verified in FP64); d_bound[i] (nullable) = the verified bound behind the decision (witness margin lower bound m* for kept
+ * rows, certificate upper bound u for pruned ones); h_counts[4] (nullable) = {kept at a corner, kept by an LP witness, pruned,
+ * kept undecided}.  Rows must be pairwise distinct.  A row with a non-finite entry is kept (counted with the corners, bound NaN) and
+ * never used as a competitor.  Synchronises `stream`. */
+PBVI_API int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts, void* stream);
+/* instrumentation of the last pbvi_prune_lp call: h_out4 = {largest competitor set |J| reached, restricted LPs solved, simplex pivots,
+ * rows sent to the LP stage} */
+PBVI_API int pbvi_prune_lp_stats(const pbvi_model* m, int64_t* h_out4);
+
 /* ---- HSVI sawtooth upper bound (BeliefValueMapping.evaluate, src/pomdp.py:887-895) -----------------
  * d_out[q] = min(v0_q, min_i v0_q + (ub_value_i - ub_belief_i . corner) * min_{s: ub_belief_i[s] > 0} query_q[s]/ub_belief_i[s]) */
 PBVI_API int pbvi_sawtooth(pbvi_model* m, const double* d_corner, const double* d_ub_beliefs, const double* d_ub_values, int n_ub,

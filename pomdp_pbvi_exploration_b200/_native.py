@@ -50,6 +50,8 @@ SIGNATURES = {
     'pbvi_unpack_rows': [_P, _P, _P, _P, c_int, c_int, c_int, c_int64, _P, _P],
     'pbvi_vi_sweep': [_P, _P, c_double, _P, _P, _P],
     'pbvi_prune_dominated': [_P, _P, c_int, _P, _P],
+    'pbvi_prune_lp': [_P, _P, c_int, _P, _P, _P, _P],
+    'pbvi_prune_lp_stats': [_P, _P],
     'pbvi_sawtooth': [_P, _P, _P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_support_lists': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth_lists': [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int, _P, _P],
@@ -480,6 +482,23 @@ class DeviceModel:
         keep = torch.empty((al.shape[0],), dtype=torch.int32, device=self.device)
         self._call(self._lib.pbvi_prune_dominated(self._h, _ptr(al), al.shape[0], _ptr(keep), self._stream))
         return keep
+
+    def prune_lp(self, alphas):
+        """LP-domination prune of pairwise distinct rows (see `pbvi_prune_lp`): returns (keep [n] int32 CUDA tensor, bound [n] float64
+        CUDA tensor, counts int64 [4] = {kept at a corner, kept by an LP witness, pruned, kept undecided}).  Synchronises."""
+        al = self._beliefs(alphas)
+        n = al.shape[0]
+        keep = torch.empty((n,), dtype=torch.int32, device=self.device)
+        bound = torch.empty((n,), dtype=torch.float64, device=self.device)
+        counts = np.zeros(4, dtype=np.int32)
+        self._call(self._lib.pbvi_prune_lp(self._h, _ptr(al), n, _ptr(keep), _ptr(bound), counts.ctypes.data, self._stream))
+        return keep, bound, counts.astype(np.int64)
+
+    def prune_lp_stats(self) -> dict:
+        """Work of the last `prune_lp` call: largest competitor set, restricted LPs, simplex pivots, rows that reached the LP stage."""
+        out = np.zeros(4, dtype=np.int64)
+        _check(self._lib.pbvi_prune_lp_stats(self._h, out.ctypes.data))
+        return dict(max_competitors=int(out[0]), lps=int(out[1]), pivots=int(out[2]), lp_rows=int(out[3]))
 
     def sawtooth(self, corner, ub_beliefs, ub_values, queries) -> torch.Tensor:
         c, q = _f64(corner, self.device), self._beliefs(queries)

@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.environ.get('PBVI_B200_LIB', os.path.join(HERE, 'libpbvi_b200.so'))
-SOURCES = ['model.cu', 'backup.cu', 'belief.cu', 'misc.cu', 'hostpack.cu', 'comm.cu', 'hsvi.cu']
+SOURCES = ['model.cu', 'backup.cu', 'belief.cu', 'misc.cu', 'hostpack.cu', 'comm.cu', 'hsvi.cu', 'prune_lp.cu']
 HOST_SOURCES = ['hostpack_host.cpp']
 HEADERS = ['pbvi_common.cuh', 'score_kernel.cuh', os.path.join('..', '..', 'include', 'pbvi_b200.h')]
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')

@@ -184,6 +184,7 @@ struct pbvi_model {
     size_t h_pack_bytes = 0;
     void* h_io = nullptr;        // pinned staging for pageable alpha / output buffers of the same call (grow-only)
     size_t h_io_bytes = 0;
+    long long prune_lp_stats[4] = {0, 0, 0, 0};   // last pbvi_prune_lp: largest |J|, restricted LPs solved, simplex pivots, rows sent to the LP
 };
 
 namespace pbvi {

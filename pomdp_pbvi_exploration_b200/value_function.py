@@ -209,26 +209,36 @@ class ValueFunction:
     # ---- pruning -------------------------------------------------------------------------------
     def prune(self, level: int = 1) -> None:
         """
-        Level 1 is a no-op (duplicates never enter), level 2 removes pointwise-dominated vectors (reference
-        src/mdp.py:857-866) with the device kernel.  Level 3 (LP domination) is broken in the reference
-        (`pruned_alpha_set` undefined, src/mdp.py:872) and is not provided.
+        Level 1 is a no-op (duplicates never enter).  Level 2 removes pointwise-dominated vectors (reference src/mdp.py:857-866).
+
+        Level 3 first runs level 2, then removes the vectors that a convex combination of the others beats everywhere -- the LP
+        domination the reference intended (src/mdp.py:834-906; its branch fails on the undefined `pruned_alpha_set` at :872).  With
+        tau = 1e-9 * max(1, max |alpha|), alpha_i is removed only with a certificate: weights lambda >= 0 summing to 1 over the other
+        rows with sum_j lambda_j alpha_j[s] > alpha_i[s] + tau at every state, re-checked in FP64 from the rows.  Every other row
+        stays: rows with a witness belief (alpha_i . b - max_{j != i} alpha_j . b > -tau), near-ties, rows whose search ran out of
+        budget, and rows with a non-finite entry.  A removed row lies more than tau below another row at every belief, and following
+        the rows that beat it ends at a kept row, so max_v alpha_v . b over the kept rows equals the max over all rows at every
+        belief.  Kept rows keep their order, actions and row hashes; pruning the result again removes nothing.
         """
         if level < self._pruning_level or level > 3:
             log('Attempting to prune a value function to a level already reached. Returning \'self\'')
             return
-        if level >= 3:
-            raise NotImplementedError('prune level 3 raises NameError in the reference (src/mdp.py:872); not emulated')
         if level >= 2 and self._pruning_level < 2 and len(self) > 0:
-            keep = self.model.device.prune_dominated(self._array).cpu().numpy().astype(bool)
-            idx = np.flatnonzero(keep)
-            self._array = self._array[torch.as_tensor(idx, device=self._array.device)]
-            self._actions = self._actions[idx]
-            self._hashes = None if self._hashes is None else self.row_hashes[idx]
-            self._vector_list = None
-            self._mirror = None
-            self.uid, self.parent_uid, self.n_new = next(_UID), None, 0
-            self._buf = None
+            self._select_rows(self.model.device.prune_dominated(self._array))
+        if level >= 3 and self._pruning_level < 3 and len(self) > 0:
+            self._select_rows(self.model.device.prune_lp(self._array)[0])
         self._pruning_level = level
+
+    def _select_rows(self, keep: torch.Tensor) -> None:
+        """Keeps the rows flagged in `keep` (device int32 [n]) in their order, with their actions and hashes."""
+        idx = np.flatnonzero(keep.cpu().numpy())
+        self._array = self._array[torch.as_tensor(idx, device=self._array.device)]
+        self._actions = self._actions[idx]
+        self._hashes = None if self._hashes is None else self.row_hashes[idx]
+        self._vector_list = None
+        self._mirror = None
+        self.uid, self.parent_uid, self.n_new = next(_UID), None, 0
+        self._buf = None
 
     # ---- persistence (reference src/mdp.py:909-1036): column 0 `action`, then one column per state label ----------
     def _frame(self, path):
