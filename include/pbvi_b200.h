@@ -213,6 +213,13 @@ PBVI_API int pbvi_unpack_rows(pbvi_model* m, const uint32_t* d_bitmap, const int
  * d_alpha_out[a][s] = Rbar[s,a] + gamma * sum_r P[s,a,r] * d_vopt[reach[s,a,r]];  d_vopt_out[s] = max_a (nullable) */
 PBVI_API int pbvi_vi_sweep(pbvi_model* m, const double* d_vopt, double gamma, double* d_alpha_out, double* d_vopt_out, void* stream);
 
+/* ---- Fast Informed Bound sweep (Hauskrecht 2000; FIB_Solver) ------------------------------------------------------------------------
+ * d_out[a][s] = Rbar[s,a] + gamma * sum_o max_{a' < k} sum_r RTO[s,a,o,r] * d_in[a'][reach[s,a,r]]   for k input rows d_in [k][S],
+ * A output rows.  Fixed order (r ascending, then o ascending, no fma contraction): R = 1 models reproduce a NumPy restatement bit for bit.
+ * d_stats2 (nullable; needs k == A, rows paired by index) receives {max(out - in), max |out - in|} from the same launch (NaN wins).
+ * Enqueues on `stream`, does not synchronise. */
+PBVI_API int pbvi_fib_sweep(pbvi_model* m, const double* d_in, int k, double gamma, double* d_out, double* d_stats2, void* stream);
+
 /* ---- pointwise-domination prune (ValueFunction.prune level 2, src/mdp.py:857-866) -------------------
  * d_keep[i] = 1 iff alpha_i is >= everywhere by no vector other than itself. */
 PBVI_API int pbvi_prune_dominated(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, void* stream);
@@ -258,6 +265,18 @@ PBVI_API int pbvi_hsvi_level(pbvi_model* m, const double* d_b, const double* d_a
                              const double* d_ub_values, int n_ub, uint64_t* d_stored_keys, double* d_stored_vals, int n_stored,
                              int stored_capacity, double conv_term, int may_continue, double* d_next, double* d_succ, double* d_mass,
                              double* h_out8, void* stream);
+
+/* ---- point-based upper-bound backup of n beliefs (UpperBound.improve) ------------------------------------------------------------------
+ * The bound is min(F, sawtooth): F(b) = max_{a < k} d_fib[a] . b over k upper-bound rows d_fib [k][S] (FIB rows), and the sawtooth over the
+ * n_ub stored beliefs of the support lists (as for pbvi_sawtooth_lists; d_corner = max_a d_fib[a][s]).  For every belief b_i of d_b [n][S]:
+ *   d_u[i]      = max_a [ b_i.Rbar[:,a] + gamma * sum_{o: P(o|b_i,a) > 0} P(o|b_i,a) * min(F, sawtooth)(b_i^{ao}) ]   (o ascending)
+ *   d_cur[i]    = min(F, sawtooth)(b_i)           (nullable)
+ *   d_best_a[i] = the first maximising action     (nullable)
+ * Scratch (n*A*O*S successors, n*A*O*(n_ub+1) sawtooth terms) comes from the handle's arena: the caller sizes n.  Enqueues on `stream`,
+ * does not synchronise. */
+PBVI_API int pbvi_upper_backup(pbvi_model* m, const double* d_b, int n, const double* d_fib, int k, double gamma, const double* d_corner,
+                               const int32_t* d_idx, const double* d_val, const int32_t* d_count, const double* d_dot,
+                               const double* d_ub_values, int n_ub, double* d_u, double* d_cur, int32_t* d_best_a, void* stream);
 
 /* ---- SSEA novelty score (src/pomdp.py:1682-1686) --------------------------------------------------
  * d_out[j] = min_i || d_beliefs[i] - d_candidates[j] ||_2 */

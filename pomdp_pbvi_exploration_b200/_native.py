@@ -49,6 +49,8 @@ SIGNATURES = {
     'pbvi_pack_slabs_host': [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int64, _P],
     'pbvi_unpack_rows': [_P, _P, _P, _P, c_int, c_int, c_int, c_int64, _P, _P],
     'pbvi_vi_sweep': [_P, _P, c_double, _P, _P, _P],
+    'pbvi_fib_sweep': [_P, _P, c_int, c_double, _P, _P, _P],
+    'pbvi_upper_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_dominated': [_P, _P, c_int, _P, _P],
     'pbvi_prune_lp': [_P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_lp_stats': [_P, _P],
@@ -476,6 +478,30 @@ class DeviceModel:
         vnew = torch.empty((self.S,), dtype=torch.float64, device=self.device)
         self._call(self._lib.pbvi_vi_sweep(self._h, _ptr(v), float(gamma), _ptr(alpha), _ptr(vnew), self._stream))
         return alpha, vnew
+
+    def fib_sweep(self, rows, gamma: float, want_stats: bool = False):
+        """One Fast Informed Bound sweep (`pbvi_fib_sweep`): A output rows [A,S] from k input rows [k,S]; with `want_stats` (k == A)
+        also the device pair {max(out - rows), max |out - rows|} [2] computed by the same launch."""
+        U = self._beliefs(rows)
+        out = torch.empty((self.A, self.S), dtype=torch.float64, device=self.device)
+        stats = torch.empty((2,), dtype=torch.float64, device=self.device) if want_stats else None
+        self._call(self._lib.pbvi_fib_sweep(self._h, _ptr(U), U.shape[0], float(gamma), _ptr(out), _ptr(stats), self._stream))
+        return (out, stats) if want_stats else out
+
+    def upper_backup(self, beliefs, fib_rows, gamma: float, corner, idx, val, count, dot, ub_values, n_ub: int, want_action: bool = False):
+        """Point-based upper-bound backup of n beliefs (`pbvi_upper_backup`) against the rows `fib_rows` [k,S] and the sawtooth over the
+        first n_ub stored beliefs of the support lists: returns (u [n], cur [n]) CUDA float64 tensors (and the maximising action [n] int32
+        with `want_action`).  The caller sizes n: the call takes n*A*O*(S + n_ub + 1) doubles of scratch."""
+        b, F = self._beliefs(beliefs), self._beliefs(fib_rows)
+        n = b.shape[0]
+        u = torch.empty((n,), dtype=torch.float64, device=self.device)
+        cur = torch.empty((n,), dtype=torch.float64, device=self.device)
+        act = torch.empty((n,), dtype=torch.int32, device=self.device) if want_action else None
+        on = n_ub > 0
+        self._call(self._lib.pbvi_upper_backup(self._h, _ptr(b), n, _ptr(F), F.shape[0], float(gamma), _ptr(corner), _ptr(idx) if on else None,
+                                               _ptr(val) if on else None, _ptr(count) if on else None, _ptr(dot) if on else None,
+                                               _ptr(ub_values) if on else None, int(n_ub), _ptr(u), _ptr(cur), _ptr(act), self._stream))
+        return (u, cur, act) if want_action else (u, cur)
 
     def prune_dominated(self, alphas) -> torch.Tensor:
         al = self._beliefs(alphas)

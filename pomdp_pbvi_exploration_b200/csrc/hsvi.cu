@@ -304,6 +304,65 @@ __global__ void __launch_bounds__(256) hsvi_take_next_kernel(const double* __res
     next[s] = (a >= 0 && o >= 0) ? succ[((size_t)a * O + o) * S + s] : b[s];
 }
 
+// ---- point-based upper-bound backup over a slab of beliefs (pbvi_upper_backup) -----------------------------------------------------
+// rb[i][a] = b_i . Rbar[:,a]: reward_dot_kernel with a warp per (belief, action)
+__global__ void __launch_bounds__(256) reward_dots_kernel(const double* __restrict__ b, int n, int S, const int32_t* __restrict__ nzPtr,
+                                                          const int32_t* __restrict__ nzIdx, const double* __restrict__ nzVal, int A,
+                                                          double* __restrict__ rb) {
+    const int w = (blockIdx.x * 256 + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (w >= n * A) return;
+    const int i = w / A, a = w - i * A;
+    const double* bi = b + (size_t)i * S;
+    double part = 0.0;
+    for (int j = nzPtr[a] + lane; j < nzPtr[a + 1]; j += 32) part = fma(bi[nzIdx[j]], nzVal[j], part);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) part += __shfl_down_sync(0xffffffffu, part, off);
+    if (lane == 0) rb[w] = part;
+}
+
+// Thread per belief i:  u[i] = max_a [ rb[i][a] + gamma * sum_{o: P(o|b,a) > 0} P(o|b,a) * min(fib, saw)(b^{ao}) ]  (o ascending, products
+// and sums rounded one at a time, strict > so the first maximising action wins), cur[i] = min(fib, saw)(b_i), bestA[i] = that action.
+// Observations of probability zero are skipped: their successor is the 0/0 row.
+__global__ void __launch_bounds__(128) upper_q_kernel(const double* __restrict__ mass, const double* __restrict__ fibSucc,
+                                                      const double* __restrict__ sawSucc, const double* __restrict__ rb,
+                                                      const double* __restrict__ fibB, const double* __restrict__ sawB, int n, int A, int O,
+                                                      double gamma, double* __restrict__ u, double* __restrict__ cur, int32_t* __restrict__ bestA) {
+    const int i = blockIdx.x * 128 + threadIdx.x;
+    if (i >= n) return;
+    const size_t z0 = (size_t)i * A * O;
+    double maxQ = -INFINITY;
+    int best = -1;
+    for (int a = 0; a < A; a++) {
+        double acc = 0.0;
+        for (int o = 0; o < O; o++) {
+            const size_t z = z0 + (size_t)a * O + o;
+            const double p = mass[z];
+            if (p > 0.0) acc = __dadd_rn(acc, __dmul_rn(p, fmin(fibSucc[z], sawSucc[z])));
+        }
+        const double q = __dadd_rn(rb[(size_t)i * A + a], __dmul_rn(gamma, acc));
+        if (q > maxQ) { maxQ = q; best = a; }
+    }
+    u[i] = maxQ;
+    if (cur) cur[i] = fmin(fibB[i], sawB[i]);
+    if (bestA) bestA[i] = best;
+}
+
+// out[j] = max_v rows[j] . alphas[v] for any number of rows (few_rows_scores_kernel's grid is limited to 65535 row tiles per launch)
+static int few_rows_max_impl(pbvi_model* m, const double* d_rows, int n, const double* d_alphas, int nV, double* d_out, cudaStream_t st) {
+    PBVI_TAKE(scores, double, (size_t)n * nV);
+    constexpr int SLAB = 65535 * FR_B;
+    for (int j0 = 0; j0 < n; j0 += SLAB) {
+        const int nj = std::min(SLAB, n - j0);
+        few_rows_scores_kernel<<<dim3(ceil_div(nV, FR_A), ceil_div(nj, FR_B)), 256, 0, st>>>(d_rows + (size_t)j0 * m->S, nj, d_alphas, nV, m->S,
+                                                                                         scores + (size_t)j0 * nV);
+        m->last_launches++;
+    }
+    few_rows_max_kernel<<<n, 256, 0, st>>>(scores, nV, d_out);
+    m->last_launches++;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}
+
 }  // namespace pbvi
 
 using namespace pbvi;
@@ -394,5 +453,44 @@ extern "C" int pbvi_hsvi_level(pbvi_model* m, const double* d_b, const double* d
     PBVI_CUDA(cudaGetLastError());
     PBVI_CUDA(cudaMemcpyAsync(h_out8, outDev, sizeof(HsviOut), cudaMemcpyDeviceToHost, st));
     PBVI_CUDA(cudaStreamSynchronize(st));
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_upper_backup(pbvi_model* m, const double* d_b, int n, const double* d_fib, int k, double gamma, const double* d_corner,
+                                 const int32_t* d_idx, const double* d_val, const int32_t* d_count, const double* d_dot,
+                                 const double* d_ub_values, int n_ub, double* d_u, double* d_cur, int32_t* d_best_a, void* stream) {
+    PBVI_REQUIRE(n >= 0 && n_ub >= 0 && k > 0, "counts must be non-negative and k positive");
+    if (n > 0) {
+        PBVI_REQUIRE(d_b && d_fib && d_corner && d_u, "NULL pointer argument");
+        PBVI_REQUIRE(n_ub == 0 || (d_idx && d_val && d_count && d_dot && d_ub_values), "NULL pointer argument: support lists are required when n_ub > 0");
+    }
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    if (n == 0) return PBVI_OK;
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    m->last_launches = 0;
+    const int A = m->A, O = m->O, S = m->S;
+    const size_t nZ = (size_t)n * m->nZ;
+    PBVI_REQUIRE(nZ <= (size_t)INT32_MAX, "too many successors in one call: pass fewer beliefs");
+    PBVI_TAKE(succ, double, nZ * S);
+    PBVI_TAKE(mass, double, nZ);
+    PBVI_TAKE(fibSucc, double, nZ);
+    PBVI_TAKE(sawSucc, double, nZ);
+    PBVI_TAKE(rb, double, (size_t)n * A);
+    PBVI_TAKE(fibB, double, (size_t)n);
+    PBVI_TAKE(sawB, double, (size_t)n);
+    PBVI_TRY(belief_successors_impl(m, d_b, n, 1, succ, mass, st));
+    PBVI_TRY(few_rows_max_impl(m, succ, (int)nZ, d_fib, k, fibSucc, st));
+    PBVI_TRY(sawtooth_lists_impl(m, d_corner, d_idx, d_val, d_count, d_dot, d_ub_values, n_ub, succ, (int)nZ, mass, sawSucc, st));
+    reward_dots_kernel<<<ceil_div(n * A, 8), 256, 0, st>>>(d_b, n, S, m->rbarNzPtr, m->rbarNzIdx, m->rbarNzVal, A, rb);
+    m->last_launches++;
+    if (d_cur) {
+        PBVI_TRY(few_rows_max_impl(m, d_b, n, d_fib, k, fibB, st));
+        PBVI_TRY(sawtooth_lists_impl(m, d_corner, d_idx, d_val, d_count, d_dot, d_ub_values, n_ub, d_b, n, nullptr, sawB, st));
+    }
+    upper_q_kernel<<<ceil_div(n, 128), 128, 0, st>>>(mass, fibSucc, sawSucc, rb, fibB, sawB, n, A, O, gamma, d_u, d_cur, d_best_a);
+    m->last_launches++;
+    PBVI_CUDA(cudaGetLastError());
     return PBVI_OK;
 }

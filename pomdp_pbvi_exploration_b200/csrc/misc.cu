@@ -241,6 +241,94 @@ __global__ void __launch_bounds__(256) vi_sweep_kernel(const double* __restrict_
     if (voptOut) voptOut[s] = best;
 }
 
+// Fast Informed Bound sweep (Hauskrecht 2000), thread per (a, s):
+//     out[a][s] = Rbar[s,a] + gamma * sum_o max_{a' < k} sum_r RTO[s,a,o,r] * U[a'][reach[s,a,r]]
+// U is read through its transposed copy UT [S][k], so the k candidates of one landing state are contiguous.  Fixed order: r ascending
+// inside, then o ascending, products and sums rounded one at a time (no fma) as in vi_sweep_kernel -- R = 1 models reproduce a NumPy
+// restatement bit for bit.  With stats != nullptr (k == A, rows paired by index) every block also leaves max(out - U) and max |out - U|
+// (NaN wins) in part[block]; the last block to finish reduces the parts in block order into stats[2].
+constexpr int FIB_THREADS = 256;
+
+__global__ void __launch_bounds__(FIB_THREADS) fib_sweep_kernel(const double* __restrict__ UT, int k, const int32_t* __restrict__ reachK,
+                                                                const double* __restrict__ rtoK, const double* __restrict__ rbarT, double gamma,
+                                                                int S, int R, int A, int O, double* __restrict__ out,
+                                                                double2* __restrict__ part, unsigned int* __restrict__ done,
+                                                                double* __restrict__ stats) {
+    __shared__ double sh[2][FIB_THREADS / 32];
+    __shared__ bool s_last;
+    const int t = blockIdx.x * FIB_THREADS + threadIdx.x;
+    double dmax = -INFINITY, amax = 0.0;
+    bool nan = false;
+    if (t < A * S) {
+        const int a = t / S, s = t - a * S;
+        const size_t K = (size_t)S * R;
+        const size_t base = (size_t)s * R;
+        const int32_t* reach = reachK + (size_t)a * K + base;
+        double acc = 0.0;
+        for (int o = 0; o < O; o++) {
+            const double* rto = rtoK + ((size_t)a * O + o) * K + base;
+            double best = -INFINITY;
+            for (int ap = 0; ap < k; ap++) {
+                double inner = 0.0;
+                for (int r = 0; r < R; r++) {
+                    const double prod = __dmul_rn(rto[r], UT[(size_t)reach[r] * k + ap]);
+                    inner = (r == 0) ? prod : __dadd_rn(inner, prod);
+                }
+                best = (inner != inner || best != best) ? inner + best : fmax(best, inner);     // NaN wins (np.max)
+            }
+            acc = __dadd_rn(acc, best);
+        }
+        const double v = __dadd_rn(rbarT[(size_t)a * S + s], __dmul_rn(gamma, acc));
+        out[(size_t)a * S + s] = v;
+        if (stats) {
+            const double d = __dadd_rn(v, -UT[(size_t)s * k + a]);
+            nan = d != d;
+            dmax = d;
+            amax = fabs(d);
+        }
+    }
+    if (!stats) return;
+    // block reduction (NaN wins), then the last-block reduction of the per-block parts
+    const unsigned anyNan = __ballot_sync(0xffffffffu, nan);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        dmax = fmax(dmax, __shfl_down_sync(0xffffffffu, dmax, off));
+        amax = fmax(amax, __shfl_down_sync(0xffffffffu, amax, off));
+    }
+    if ((threadIdx.x & 31) == 0) {
+        sh[0][threadIdx.x >> 5] = anyNan ? NAN : dmax;
+        sh[1][threadIdx.x >> 5] = anyNan ? NAN : amax;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double m0 = -INFINITY, m1 = 0.0;
+        bool bn = false;
+        for (int w = 0; w < FIB_THREADS / 32; w++) {
+            bn |= sh[0][w] != sh[0][w];
+            m0 = fmax(m0, sh[0][w]);
+            m1 = fmax(m1, sh[1][w]);
+        }
+        part[blockIdx.x] = bn ? make_double2(NAN, NAN) : make_double2(m0, m1);
+        __threadfence();
+        s_last = atomicAdd(done, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x == 0) {
+        __threadfence();
+        const volatile double* pv = reinterpret_cast<volatile double*>(part);     // written by other blocks: bypass L1
+        double m0 = -INFINITY, m1 = 0.0;
+        bool bn = false;
+        for (int b = 0; b < (int)gridDim.x; b++) {
+            const double x = pv[2 * b], y = pv[2 * b + 1];
+            bn |= x != x;
+            m0 = fmax(m0, x);
+            m1 = fmax(m1, y);
+        }
+        stats[0] = bn ? NAN : m0;
+        stats[1] = bn ? NAN : m1;
+    }
+}
+
 // keep[i] = 1 iff exactly one vector (alpha_i itself, or none when it holds a NaN... the reference counts rows with
 // all(alpha_j >= alpha_i)) dominates alpha_i everywhere.  Block per i, early exit per j on the first losing coordinate block.
 __global__ void __launch_bounds__(256) prune_dominated_kernel(const double* __restrict__ alphas, int nV, int S, int32_t* __restrict__ keep) {
@@ -644,6 +732,32 @@ extern "C" int pbvi_vi_sweep(pbvi_model* m, const double* d_vopt, double gamma, 
     vi_sweep_kernel<<<ceil_div(m->S, 256), 256, 0, (cudaStream_t)stream>>>(d_vopt, m->reachK, m->probK, m->rbarT, gamma, m->S, m->R, m->A,
                                                                           d_alpha_out, d_vopt_out);
     m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_fib_sweep(pbvi_model* m, const double* d_in, int k, double gamma, double* d_out, double* d_stats2, void* stream) {
+    PBVI_REQUIRE(k > 0, "k must be positive");
+    PBVI_REQUIRE(d_in && d_out, "NULL pointer argument");
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_REQUIRE(!d_stats2 || k == m->A, "the residual statistics pair rows by index: they need k == A input rows");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    m->last_launches = 0;
+    const int S = m->S, nBlocks = ceil_div(m->A * S, FIB_THREADS);
+    PBVI_TAKE(UT, double, (size_t)S * k);
+    PBVI_TRY(transpose_alphas(m, d_in, k, k, UT, st));          // [k][S] -> [S][k]: the k candidates of a landing state are one line
+    double2* part = nullptr;
+    unsigned int* done = nullptr;
+    if (d_stats2) {
+        part = m->arena.take<double2>((size_t)nBlocks);
+        done = m->arena.take<unsigned int>(1);
+        if (!part || !done) return PBVI_ERR_OOM;
+        PBVI_CUDA(cudaMemsetAsync(done, 0, sizeof(unsigned int), st));
+    }
+    fib_sweep_kernel<<<nBlocks, FIB_THREADS, 0, st>>>(UT, k, m->reachK, m->rtoK, m->rbarT, gamma, S, m->R, m->A, m->O, d_out, part, done, d_stats2);
+    m->last_launches++;
     PBVI_CUDA(cudaGetLastError());
     return PBVI_OK;
 }
