@@ -86,6 +86,16 @@ PBVI_API int pbvi_backup_select(pbvi_model* m, const double* d_beliefs, int nB, 
 PBVI_API int pbvi_backup_assemble(pbvi_model* m, const double* d_alphas, int nV, double gamma, const int32_t* d_actions,
                          const int32_t* d_vsel, int n, double* d_out, uint64_t* d_hash, void* stream);
 
+/* pbvi_controller_sweep: one evaluation sweep of a finite-state controller (PolicyGraph) with n nodes, node i playing d_actions[i] and
+ * moving to node d_succ[i][o] on observation o:
+ *   d_out[i][s] = Rbar[s,a_i] + ((G_0 + G_1) + ...),  G_o = gamma * sum_r RTO[s,a_i,o,r] * d_in[succ_i[o]][reach[s,a_i,r]]
+ * i.e. bitwise the rows pbvi_backup_assemble(d_in, n, gamma, d_actions, d_succ) gives.  d_in [n][S] must be finite (zero-RTO terms
+ * are skipped as for finite alphas); indices are clamped into range.  d_stats3 (nullable) receives, from the same launch,
+ * {max(out - in), max(in - out), max |out - in|} over all n*S entries, rows paired by index (NaN wins).
+ * Enqueues on `stream`, does not synchronise. */
+PBVI_API int pbvi_controller_sweep(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions,
+                                   const int32_t* d_succ, double* d_out, double* d_stats3, void* stream);
+
 /* pbvi_backup: select + assemble for every belief (no dedup): d_out_alpha [nB][S], d_out_action [nB];
  * d_out_vstar [nB][A][O] and d_out_value [nB][A] may be NULL. */
 PBVI_API int pbvi_backup(pbvi_model* m, const double* d_beliefs, int nB, const double* d_alphas, int nV, double gamma,

@@ -29,6 +29,7 @@ SIGNATURES = {
     'pbvi_model_dims': [_P, POINTER(c_int), POINTER(c_int), POINTER(c_int), POINTER(c_int)],
     'pbvi_backup_select': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P],
     'pbvi_backup_assemble': [_P, _P, c_int, c_double, _P, _P, c_int, _P, _P, _P],
+    'pbvi_controller_sweep': [_P, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_backup_host': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P],
     'pbvi_backup_host_unique': [_P, _P, c_int, _P, c_int, c_double, _P, c_int, _P, POINTER(c_int), _P],
@@ -210,6 +211,19 @@ class DeviceModel:
         self._call(self._lib.pbvi_backup_assemble(self._h, _ptr(al), al.shape[0], float(gamma), _ptr(act), _ptr(vs), n, _ptr(out),
                                                   _ptr(keys), self._stream))
         return (out, keys) if with_hash else out
+
+    def controller_sweep(self, rows, gamma: float, actions, succ, want_stats: bool = False):
+        """One evaluation sweep of a finite-state controller (`pbvi_controller_sweep`): n rows [n,S] from the n node rows `rows`, node i
+        playing actions[i] and moving to succ[i][o]; with `want_stats` also the device triple {max(out - rows), max(rows - out),
+        max |out - rows|} [3] computed by the same launch."""
+        W = self._beliefs(rows)
+        act, sc = _i32(actions, self.device), _i32(succ, self.device)
+        n = W.shape[0]
+        assert act.shape == (n,) and sc.shape == (n, self.O)
+        out = torch.empty((n, self.S), dtype=torch.float64, device=self.device)
+        stats = torch.empty((3,), dtype=torch.float64, device=self.device) if want_stats else None
+        self._call(self._lib.pbvi_controller_sweep(self._h, _ptr(W), n, float(gamma), _ptr(act), _ptr(sc), _ptr(out), _ptr(stats), self._stream))
+        return (out, stats) if want_stats else out
 
     def backup(self, beliefs, alphas, gamma: float):
         """select + assemble for every belief, no dedup: (alpha [nB,S], action [nB], v* [nB,A,O], value [nB,A])."""

@@ -24,6 +24,37 @@ from .value_function import ValueFunction
 CHUNK_BYTES = 2 << 30        # per pbvi_upper_backup call: successors (n*A*O*S doubles) and sawtooth terms (n*A*O*(n_ub+1)) each stay below
 
 
+def certificate_contraction(model: Model, gamma: float, what: str) -> float:
+    """gamma' = gamma * max(1, m) with m = max_{s,a} sum_{o,r} RTO[s,a,o,r]: the factor by which a constant shift of every row passes through
+    one sweep at most.  The residual certificates (FIB_Solver: upper bound, PolicyGraph.evaluate: lower bound) need gamma' < 1;
+    otherwise this raises ValueError."""
+    rto = np.asarray(model.reachable_transitional_observation_table, dtype=np.float64)
+    m = float(np.max(rto.sum(axis=(2, 3))))
+    gamma_c = float(gamma) * max(1.0, m)
+    if not gamma_c < 1.0:
+        raise ValueError(f'gamma * max(1, max_(s,a) sum_(o,r) RTO) = {gamma_c} >= 1: the {what} certificate needs a contraction')
+    return gamma_c
+
+
+def belief_rows(model: Model, beliefs) -> torch.Tensor:
+    """A BeliefSet, a Belief, or an array / tensor of one or more rows as a contiguous CUDA float64 [n,S] tensor; non-finite rows raise
+    ValueError."""
+    if isinstance(beliefs, BeliefSet):
+        rows = beliefs.belief_array
+    elif isinstance(beliefs, Belief):
+        rows = beliefs.values[None, :]
+    else:
+        rows = beliefs if isinstance(beliefs, torch.Tensor) else torch.as_tensor(np.asarray(beliefs, dtype=np.float64))
+        if rows.dim() == 1:
+            rows = rows[None, :]
+    rows = rows.to(device=model.device.device, dtype=torch.float64).contiguous()
+    if rows.dim() != 2 or rows.shape[1] != model.state_count:
+        raise ValueError(f'beliefs must be [n, {model.state_count}], got {tuple(rows.shape)}')
+    if rows.shape[0] and not bool(torch.isfinite(rows).all()):
+        raise ValueError('belief rows must be finite')
+    return rows
+
+
 class FIB_Solver:
     """
     Fast Informed Bound value iteration (Hauskrecht 2000) on the device:
@@ -51,11 +82,7 @@ class FIB_Solver:
               history_tracking_level: int = 1):
         """Returns (ValueFunction with one row per action, byte-deduplicated; MDPSolverHistory)."""
         gamma = float(self.gamma)
-        rto = np.asarray(model.reachable_transitional_observation_table, dtype=np.float64)
-        m = float(np.max(rto.sum(axis=(2, 3))))
-        gamma_c = gamma * max(1.0, m)
-        if not gamma_c < 1.0:
-            raise ValueError(f'gamma * max(1, max_(s,a) sum_(o,r) RTO) = {gamma_c} >= 1: the FIB certificate needs a contraction')
+        gamma_c = certificate_contraction(model, gamma, 'FIB')
         dev = model.device
         A, S = model.action_count, model.state_count
         if initial_value_function is None:
@@ -152,20 +179,7 @@ class UpperBound:
         self._cap = cap
 
     def _rows_of(self, beliefs) -> torch.Tensor:
-        if isinstance(beliefs, BeliefSet):
-            rows = beliefs.belief_array
-        elif isinstance(beliefs, Belief):
-            rows = beliefs.values[None, :]
-        else:
-            rows = beliefs if isinstance(beliefs, torch.Tensor) else torch.as_tensor(np.asarray(beliefs, dtype=np.float64))
-            if rows.dim() == 1:
-                rows = rows[None, :]
-        rows = rows.to(device=self._F.device, dtype=torch.float64).contiguous()
-        if rows.dim() != 2 or rows.shape[1] != self.model.state_count:
-            raise ValueError(f'beliefs must be [n, {self.model.state_count}], got {tuple(rows.shape)}')
-        if rows.shape[0] and not bool(torch.isfinite(rows).all()):
-            raise ValueError('belief rows must be finite')
-        return rows
+        return belief_rows(self.model, beliefs)
 
     def _lists(self):
         n = self._n

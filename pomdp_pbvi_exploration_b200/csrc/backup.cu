@@ -15,6 +15,8 @@
 // pbvi_backup_assemble:
 //   action_order_kernel + assemble_grouped_kernel (R = 1) / assemble_kernel   alpha_a rows for (action, v*[O]) tuples in the
 //                             reference's operation order, no FMA contraction, 128-bit row keys accumulated on the way
+// pbvi_controller_sweep:
+//   controller_sweep_kernel   the same rows for the nodes of a finite-state controller against its own rows, plus a fused residual
 #include <algorithm>
 #include <thread>
 
@@ -433,6 +435,94 @@ __global__ void __launch_bounds__(256) assemble_kernel(const double* __restrict_
         for (int w = 0; w < 8; w++) { x += sh[0][w]; y += sh[1][w]; }
         atomicAdd(&hacc[(size_t)i * 2], x);
         atomicAdd(&hacc[(size_t)i * 2 + 1], y);
+    }
+}
+
+// ---- one evaluation sweep of a finite-state controller: out[i][s] = alpha_a entry of the tuple (actions[i], succ[i][.]) against the
+//      n rows `in` (the assemble kernel's arithmetic, so out is bitwise what pbvi_backup_assemble gives for the same tuples).  Block per
+//      (node i, 256 states), 1-D grid.  With stats != nullptr every block leaves {max d, -min d, max |d|} of d = out - in (rows paired by
+//      index; NaN wins) in part[block]; the last block to finish reduces the parts into stats[3].
+constexpr int CTRL_THREADS = 256;
+
+__device__ __forceinline__ void ctrl_reduce3(double& a, double& b, double& c, bool& nan, double (*sh)[CTRL_THREADS / 32], int* shn) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        a = fmax(a, __shfl_down_sync(0xffffffffu, a, off));
+        b = fmax(b, __shfl_down_sync(0xffffffffu, b, off));
+        c = fmax(c, __shfl_down_sync(0xffffffffu, c, off));
+    }
+    const unsigned anyNan = __ballot_sync(0xffffffffu, nan);
+    if ((threadIdx.x & 31) == 0) { sh[0][threadIdx.x >> 5] = a; sh[1][threadIdx.x >> 5] = b; sh[2][threadIdx.x >> 5] = c; shn[threadIdx.x >> 5] = anyNan != 0; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < CTRL_THREADS / 32; w++) {
+            a = fmax(a, sh[0][w]);
+            b = fmax(b, sh[1][w]);
+            c = fmax(c, sh[2][w]);
+            nan |= shn[w] != 0;
+        }
+        nan |= shn[0] != 0;
+    }
+}
+
+__global__ void __launch_bounds__(CTRL_THREADS) controller_sweep_kernel(const double* __restrict__ in, int n, const int32_t* __restrict__ actions,
+                                                                        const int32_t* __restrict__ succ, const int32_t* __restrict__ reachK,
+                                                                        const double* __restrict__ rtoK, const double* __restrict__ rbarT,
+                                                                        double gamma, int S, int R, int O, int A, int sBlocks, bool skipZero,
+                                                                        double* __restrict__ out, double* __restrict__ part,
+                                                                        unsigned int* __restrict__ done, double* __restrict__ stats) {
+    extern __shared__ int s_vsel[];
+    __shared__ double sh[3][CTRL_THREADS / 32];
+    __shared__ int shn[CTRL_THREADS / 32];
+    __shared__ bool s_last;
+    const int i = blockIdx.x / sBlocks, s = (blockIdx.x % sBlocks) * CTRL_THREADS + threadIdx.x;
+    const int a = min(max(actions[i], 0), A - 1);                      // indices are clamped: a bad node never reads out of bounds
+    for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), n - 1);
+    __syncthreads();
+    double up = -INFINITY, down = -INFINITY, amax = 0.0;
+    bool nan = false;
+    if (s < S) {
+        const double v = alpha_a_entry(in, S, R, O, s_vsel, reachK + (size_t)a * S * R, rtoK + (size_t)a * O * S * R, rbarT + (size_t)a * S,
+                                       gamma, s, skipZero);
+        out[(size_t)i * S + s] = v;
+        if (stats) {
+            const double d = __dadd_rn(v, -in[(size_t)i * S + s]);
+            nan = d != d;
+            up = d;
+            down = -d;
+            amax = fabs(d);
+        }
+    }
+    if (!stats) return;
+    ctrl_reduce3(up, down, amax, nan, sh, shn);
+    if (threadIdx.x == 0) {
+        const size_t b = blockIdx.x;
+        part[3 * b] = nan ? NAN : up;
+        part[3 * b + 1] = nan ? NAN : down;
+        part[3 * b + 2] = nan ? NAN : amax;
+        __threadfence();
+        s_last = atomicAdd(done, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    const volatile double* pv = part;                                  // written by other blocks: bypass L1
+    up = down = -INFINITY;
+    amax = 0.0;
+    nan = false;
+    for (unsigned b = threadIdx.x; b < gridDim.x; b += CTRL_THREADS) {
+        const double x = pv[3 * (size_t)b], y = pv[3 * (size_t)b + 1], z = pv[3 * (size_t)b + 2];
+        nan |= x != x;
+        up = fmax(up, x);
+        down = fmax(down, y);
+        amax = fmax(amax, z);
+    }
+    __syncthreads();                                                   // sh / shn are reused
+    ctrl_reduce3(up, down, amax, nan, sh, shn);
+    if (threadIdx.x == 0) {
+        stats[0] = nan ? NAN : up;
+        stats[1] = nan ? NAN : down;
+        stats[2] = nan ? NAN : amax;
     }
 }
 
@@ -964,6 +1054,36 @@ extern "C" int pbvi_backup_assemble(pbvi_model* m, const double* d_alphas, int n
     PBVI_TRY(enter_call(m, (cudaStream_t)stream));
     m->last_launches = 0;
     return assemble_impl(m, d_alphas, nV, gamma, d_actions, d_vsel, (size_t)m->O, 0, n, d_out, d_hash, (cudaStream_t)stream);
+}
+
+extern "C" int pbvi_controller_sweep(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions, const int32_t* d_succ,
+                                     double* d_out, double* d_stats3, void* stream) {
+    PBVI_REQUIRE(d_in && d_actions && d_succ && d_out, "NULL pointer argument");
+    PBVI_REQUIRE(n >= 1, "need n >= 1 controller nodes");
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    const int sBlocks = ceil_div(m->S, CTRL_THREADS);
+    PBVI_REQUIRE((long long)n * sBlocks <= 0x7fffffffLL, "too many controller nodes in one call");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    m->last_launches = 0;
+    const unsigned nBlocks = (unsigned)((long long)n * sBlocks);
+    double* part = nullptr;
+    unsigned int* done = nullptr;
+    if (d_stats3) {
+        part = m->arena.take<double>((size_t)nBlocks * 3);
+        done = m->arena.take<unsigned int>(1);
+        if (!part || !done) return PBVI_ERR_OOM;
+        PBVI_CUDA(cudaMemsetAsync(done, 0, sizeof(unsigned int), st));
+    }
+    // the rows are finite (the caller's contract), so zero-RTO terms are skipped exactly as pbvi_backup_assemble skips them for finite alphas
+    const bool skipZero = fabs(gamma) <= 1.79769313486231570e308;
+    controller_sweep_kernel<<<nBlocks, CTRL_THREADS, m->O * sizeof(int), st>>>(d_in, n, d_actions, d_succ, m->reachK, m->rtoK, m->rbarT, gamma,
+                                                                               m->S, m->R, m->O, m->A, sBlocks, skipZero, d_out, part, done,
+                                                                               d_stats3);
+    m->last_launches++;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
 }
 
 extern "C" int pbvi_backup(pbvi_model* m, const double* d_beliefs, int nB, const double* d_alphas, int nV, double gamma,
