@@ -96,6 +96,14 @@ PBVI_API int pbvi_backup_assemble(pbvi_model* m, const double* d_alphas, int nV,
 PBVI_API int pbvi_controller_sweep(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions,
                                    const int32_t* d_succ, double* d_out, double* d_stats3, void* stream);
 
+/* pbvi_controller_evaluate: up to max_sweeps sweeps W <- T_pi W of pbvi_controller_sweep from W = d_in in one persistent cooperative
+ * launch, stopping after the first sweep whose max |out - in| is below tol or NaN.  d_out [n][S] receives the last iterate (d_in is not
+ * written and must not be d_out), d_changes [max_sweeps] (nullable) each sweep's max |out - in|, *h_sweeps the number of sweeps run.
+ * k sweeps give bitwise the rows and change values of k pbvi_controller_sweep calls.  Synchronises `stream` once, at the end. */
+PBVI_API int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions,
+                                      const int32_t* d_succ, double tol, int max_sweeps, double* d_out, double* d_changes,
+                                      int* h_sweeps, void* stream);
+
 /* pbvi_backup: select + assemble for every belief (no dedup): d_out_alpha [nB][S], d_out_action [nB];
  * d_out_vstar [nB][A][O] and d_out_value [nB][A] may be NULL. */
 PBVI_API int pbvi_backup(pbvi_model* m, const double* d_beliefs, int nB, const double* d_alphas, int nV, double gamma,
@@ -233,6 +241,12 @@ PBVI_API int pbvi_fib_sweep(pbvi_model* m, const double* d_in, int k, double gam
 /* ---- pointwise-domination prune (ValueFunction.prune level 2, src/mdp.py:857-866) -------------------
  * d_keep[i] = 1 iff alpha_i is >= everywhere by no vector other than itself. */
 PBVI_API int pbvi_prune_dominated(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, void* stream);
+
+/* pbvi_first_dominating_row: domination of one row set by another (the improvement step of policy iteration on a controller).
+ * d_first[i] = the smallest j with d_new[j][s] >= d_old[i][s] at every state s (a NaN on either side fails), or -1; rows have length S.
+ * Equal rows dominate.  Enqueues on `stream`, does not synchronise. */
+PBVI_API int pbvi_first_dominating_row(pbvi_model* m, const double* d_new, int n_new, const double* d_old, int n_old, int32_t* d_first,
+                                       void* stream);
 
 /* ---- LP-domination prune (ValueFunction.prune level 3; the reference's intended Lark / White filter, src/mdp.py:834-906, whose
  * branch fails on the undefined `pruned_alpha_set` at :872) ----------------------------------------------------------------------

@@ -30,6 +30,7 @@ SIGNATURES = {
     'pbvi_backup_select': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P],
     'pbvi_backup_assemble': [_P, _P, c_int, c_double, _P, _P, c_int, _P, _P, _P],
     'pbvi_controller_sweep': [_P, _P, c_int, c_double, _P, _P, _P, _P, _P],
+    'pbvi_controller_evaluate': [_P, _P, c_int, c_double, _P, _P, c_double, c_int, _P, _P, POINTER(c_int), _P],
     'pbvi_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_backup_host': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P],
     'pbvi_backup_host_unique': [_P, _P, c_int, _P, c_int, c_double, _P, c_int, _P, POINTER(c_int), _P],
@@ -53,6 +54,7 @@ SIGNATURES = {
     'pbvi_fib_sweep': [_P, _P, c_int, c_double, _P, _P, _P],
     'pbvi_upper_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_dominated': [_P, _P, c_int, _P, _P],
+    'pbvi_first_dominating_row': [_P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_prune_lp': [_P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_lp_stats': [_P, _P],
     'pbvi_sawtooth': [_P, _P, _P, _P, c_int, _P, c_int, _P, _P],
@@ -224,6 +226,28 @@ class DeviceModel:
         stats = torch.empty((3,), dtype=torch.float64, device=self.device) if want_stats else None
         self._call(self._lib.pbvi_controller_sweep(self._h, _ptr(W), n, float(gamma), _ptr(act), _ptr(sc), _ptr(out), _ptr(stats), self._stream))
         return (out, stats) if want_stats else out
+
+    def controller_evaluate(self, rows, gamma: float, actions, succ, tol: float, max_sweeps: int):
+        """Up to `max_sweeps` controller sweeps in one persistent launch (`pbvi_controller_evaluate`), stopping after the first whose
+        max |out - in| is below `tol` or NaN: returns (last iterate [n,S], per-sweep max |out - in| [k] CUDA float64, k).  Synchronises."""
+        W = self._beliefs(rows)
+        act, sc = _i32(actions, self.device), _i32(succ, self.device)
+        n = W.shape[0]
+        assert act.shape == (n,) and sc.shape == (n, self.O)
+        out = torch.empty((n, self.S), dtype=torch.float64, device=self.device)
+        changes = torch.empty((max(int(max_sweeps), 1),), dtype=torch.float64, device=self.device)
+        k = c_int(0)
+        self._call(self._lib.pbvi_controller_evaluate(self._h, _ptr(W), n, float(gamma), _ptr(act), _ptr(sc), float(tol), int(max_sweeps),
+                                                      _ptr(out), _ptr(changes), byref(k), self._stream))
+        return out, changes[:k.value], k.value
+
+    def first_dominating_row(self, new_rows, old_rows) -> torch.Tensor:
+        """For every row of `old_rows`, the first row of `new_rows` that is >= it at every state, or -1 (`pbvi_first_dominating_row`):
+        int32 [n_old] CUDA tensor."""
+        Y, X = self._beliefs(new_rows), self._beliefs(old_rows)
+        first = torch.empty((X.shape[0],), dtype=torch.int32, device=self.device)
+        self._call(self._lib.pbvi_first_dominating_row(self._h, _ptr(Y), Y.shape[0], _ptr(X), X.shape[0], _ptr(first), self._stream))
+        return first
 
     def backup(self, beliefs, alphas, gamma: float):
         """select + assemble for every belief, no dedup: (alpha [nB,S], action [nB], v* [nB,A,O], value [nB,A])."""

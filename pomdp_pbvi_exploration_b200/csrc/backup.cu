@@ -17,10 +17,16 @@
 //                             reference's operation order, no FMA contraction, 128-bit row keys accumulated on the way
 // pbvi_controller_sweep:
 //   controller_sweep_kernel   the same rows for the nodes of a finite-state controller against its own rows, plus a fused residual
+// pbvi_controller_evaluate:
+//   controller_evaluate_kernel   persistent cooperative launch: the sweeps of controller_sweep_kernel until the change test stops them
 #include <algorithm>
 #include <thread>
 
+#include <cooperative_groups.h>
+
 #include "score_kernel.cuh"
+
+namespace cg = cooperative_groups;
 
 namespace pbvi {
 
@@ -255,6 +261,9 @@ __device__ __forceinline__ double block_sum_256(double v, double* sh) {
 // that is zero, and Rbar + (+-0.0) is the same double unless Rbar is -0.0 -- in which case nothing is skipped.  So the
 // result is bit-identical while most gathers of a sparse observation model (2 of 3 observations impossible from most states of
 // the olfactory model) are never issued.
+// Coherent: the alpha rows were written earlier in the same launch (controller_evaluate_kernel), so they are gathered with ld.global.cg
+// instead of through the read-only data cache, which is not kept coherent with writes during a launch.
+template <bool Coherent = false>
 __device__ __forceinline__ double alpha_a_entry(const double* __restrict__ alphas, int S, int R, int O, const int* vsel,
                                                 const int32_t* __restrict__ reach, const double* __restrict__ rtoA,
                                                 const double* __restrict__ rbarA, double gamma, int s, bool skipZero) {
@@ -268,7 +277,7 @@ __device__ __forceinline__ double alpha_a_entry(const double* __restrict__ alpha
         for (int r = 0; r < R; r++) {
             const size_t k = (size_t)s * R + r;
             const double w = rto[k];
-            const double prod = (skip && w == 0.0) ? 0.0 : __dmul_rn(w, arow[reach[k]]);
+            const double prod = (skip && w == 0.0) ? 0.0 : __dmul_rn(w, Coherent ? __ldcg(arow + reach[k]) : arow[reach[k]]);
             inner = (r == 0) ? prod : __dadd_rn(inner, prod);
         }
         const double term = __dmul_rn(gamma, inner);
@@ -523,6 +532,85 @@ __global__ void __launch_bounds__(CTRL_THREADS) controller_sweep_kernel(const do
         stats[0] = nan ? NAN : up;
         stats[1] = nan ? NAN : down;
         stats[2] = nan ? NAN : amax;
+    }
+}
+
+// ---- up to maxSweeps evaluation sweeps in one cooperative launch (pbvi_controller_evaluate).  Blocks stride over the (node, 256-state)
+//      items of controller_sweep_kernel with the same arithmetic; sweep k reads in0 (k = 0) or the rows sweep k-1 wrote, and writes
+//      bufA (k even) or bufB (k odd).  Each block leaves max |d| of its items (NaN wins) in part[k & 1][block]; after the one grid
+//      barrier of the sweep every block reduces all partials itself and so reaches the same stop decision (change < tol or NaN, or the
+//      last sweep).  The two parities keep a block that has already entered sweep k+1 from overwriting slots of sweep k that a slower
+//      block is still reading: slots of parity k & 1 are written again only after the barrier of sweep k+1, which every block passes
+//      only after its reads.  A maximum is exact in any order, so the change values are bitwise those of pbvi_controller_sweep's stats.
+//      When the last sweep wrote bufB, the blocks copy it into bufA (its writes are visible after the barrier).
+__device__ __forceinline__ double ctrl_reduce_max(double v, bool nan, double* sh, int* shn) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, off));
+    const unsigned anyNan = __ballot_sync(0xffffffffu, nan);
+    __syncthreads();                                                   // sh / shn of the previous use have been read
+    if ((threadIdx.x & 31) == 0) { sh[threadIdx.x >> 5] = v; shn[threadIdx.x >> 5] = anyNan != 0; }
+    __syncthreads();
+    bool n = false;
+#pragma unroll
+    for (int w = 0; w < CTRL_THREADS / 32; w++) {
+        v = fmax(v, sh[w]);
+        n |= shn[w] != 0;
+    }
+    return n ? NAN : v;
+}
+
+__global__ void __launch_bounds__(CTRL_THREADS) controller_evaluate_kernel(const double* __restrict__ in0, int n, const int32_t* __restrict__ actions,
+                                                                           const int32_t* __restrict__ succ, const int32_t* __restrict__ reachK,
+                                                                           const double* __restrict__ rtoK, const double* __restrict__ rbarT,
+                                                                           double gamma, int S, int R, int O, int A, int sBlocks, bool skipZero,
+                                                                           double tol, int maxSweeps, double* bufA, double* bufB, double* part,
+                                                                           double* __restrict__ changes, int* __restrict__ sweepsOut) {
+    extern __shared__ int s_vsel[];
+    __shared__ double sh[CTRL_THREADS / 32];
+    __shared__ int shn[CTRL_THREADS / 32];
+    cg::grid_group grid = cg::this_grid();
+    const int items = n * sBlocks;
+    int k = 0;
+    for (;; k++) {
+        // rows written earlier in this launch are read with ld.global.cg, never through the read-only data cache
+        const double* src = (k == 0) ? in0 : ((k & 1) ? bufA : bufB);
+        double* dst = (k & 1) ? bufB : bufA;
+        double amax = 0.0;
+        bool nan = false;
+        for (int it = blockIdx.x; it < items; it += gridDim.x) {
+            const int i = it / sBlocks, s = (it % sBlocks) * CTRL_THREADS + threadIdx.x;
+            const int a = min(max(actions[i], 0), A - 1);
+            __syncthreads();                                           // s_vsel of the previous item has been used
+            for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), n - 1);
+            __syncthreads();
+            if (s < S) {
+                const double v = alpha_a_entry<true>(src, S, R, O, s_vsel, reachK + (size_t)a * S * R, rtoK + (size_t)a * O * S * R,
+                                                     rbarT + (size_t)a * S, gamma, s, skipZero);
+                dst[(size_t)i * S + s] = v;
+                const double d = __dadd_rn(v, -__ldcg(src + (size_t)i * S + s));
+                nan |= d != d;
+                amax = fmax(amax, fabs(d));
+            }
+        }
+        const double mine = ctrl_reduce_max(amax, nan, sh, shn);
+        double* slots = part + (size_t)(k & 1) * gridDim.x;
+        if (threadIdx.x == 0) slots[blockIdx.x] = mine;
+        grid.sync();
+        amax = 0.0;
+        nan = false;
+        for (unsigned b = threadIdx.x; b < gridDim.x; b += CTRL_THREADS) {
+            const double x = __ldcg(slots + b);
+            nan |= x != x;
+            amax = fmax(amax, x);
+        }
+        const double change = ctrl_reduce_max(amax, nan, sh, shn);
+        if (changes && blockIdx.x == 0 && threadIdx.x == 0) changes[k] = change;
+        if (!(change >= tol) || k + 1 == maxSweeps) break;           // converged, NaN, or out of sweeps: the same decision in every block
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) *sweepsOut = k + 1;
+    if (k & 1) {
+        const size_t total = (size_t)n * S;
+        for (size_t e = (size_t)blockIdx.x * CTRL_THREADS + threadIdx.x; e < total; e += (size_t)gridDim.x * CTRL_THREADS) bufA[e] = __ldcg(bufB + e);
     }
 }
 
@@ -1083,6 +1171,46 @@ extern "C" int pbvi_controller_sweep(pbvi_model* m, const double* d_in, int n, d
                                                                                d_stats3);
     m->last_launches++;
     PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions, const int32_t* d_succ,
+                                        double tol, int max_sweeps, double* d_out, double* d_changes, int* h_sweeps, void* stream) {
+    PBVI_REQUIRE(d_in && d_actions && d_succ && d_out && h_sweeps, "NULL pointer argument");
+    PBVI_REQUIRE(n >= 1, "need n >= 1 controller nodes");
+    PBVI_REQUIRE(max_sweeps >= 1, "need max_sweeps >= 1");
+    PBVI_REQUIRE(tol == tol, "tol must not be NaN");
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    const int sBlocks = ceil_div(m->S, CTRL_THREADS);
+    PBVI_REQUIRE((long long)n * sBlocks <= 0x7fffffffLL, "too many controller nodes in one call");
+    PBVI_REQUIRE(d_in != d_out, "d_in and d_out must be different buffers");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    m->last_launches = 0;
+    const size_t smem = (size_t)m->O * sizeof(int);
+    int perSM = 0;
+    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, controller_evaluate_kernel, CTRL_THREADS, smem));
+    if (perSM < 1) {
+        set_error("pbvi_controller_evaluate: the kernel cannot be resident with %zu bytes of shared memory", smem);
+        return PBVI_ERR_UNSUPPORTED;
+    }
+    // every block must be resident for the grid barrier; a grid larger than the work would only add blocks to each barrier
+    const int nBlocks = (int)std::min<long long>((long long)perSM * m->sm_count, (long long)n * sBlocks);
+    PBVI_TAKE(bufB, double, (size_t)n * m->S);
+    PBVI_TAKE(part, double, (size_t)2 * nBlocks);
+    PBVI_TAKE(d_sweeps, int, 1);
+    const bool skipZero = fabs(gamma) <= 1.79769313486231570e308;   // as pbvi_controller_sweep
+    int S = m->S, R = m->R, O = m->O, A = m->A;
+    void* args[] = {(void*)&d_in, (void*)&n, (void*)&d_actions, (void*)&d_succ, (void*)&m->reachK, (void*)&m->rtoK, (void*)&m->rbarT,
+                    (void*)&gamma, (void*)&S, (void*)&R, (void*)&O, (void*)&A, (void*)&sBlocks, (void*)&skipZero, (void*)&tol,
+                    (void*)&max_sweeps, (void*)&d_out, (void*)&bufB, (void*)&part, (void*)&d_changes, (void*)&d_sweeps};
+    PBVI_CUDA(cudaLaunchCooperativeKernel((const void*)controller_evaluate_kernel, dim3(nBlocks), dim3(CTRL_THREADS), args, smem, st));
+    m->last_launches++;
+    int sweeps = 0;
+    PBVI_CUDA(cudaMemcpyAsync(&sweeps, d_sweeps, sizeof(int), cudaMemcpyDeviceToHost, st));
+    PBVI_CUDA(cudaStreamSynchronize(st));
+    *h_sweeps = sweeps;
     return PBVI_OK;
 }
 

@@ -352,6 +352,53 @@ __global__ void __launch_bounds__(256) prune_dominated_kernel(const double* __re
     if (threadIdx.x == 0) keep[i] = (count == 1) ? 1 : 0;
 }
 
+// first[i] = the smallest j with Y_j[s] >= X_i[s] at every state (a NaN on either side is a violation), or -1.  Block per (32 old rows
+// x 32 new rows) tile; both tiles pass through shared memory DOM_KS states at a time, and each thread carries four (j, i) pairs, i =
+// lane, j = warp + 8 q, so a warp reads one broadcast Y value and 32 consecutive X values per state.  A pair drops out at its first
+// violating state and the block stops when none is left.  first[] starts at -1 (all ones) and the tiles meet through an unsigned
+// atomicMin, so the result does not depend on the order of the blocks; a pair whose j is not below the best j already found for its i is
+// dropped at the start.
+constexpr int DOM_T = 32, DOM_KS = 32;
+
+__global__ void __launch_bounds__(256) first_dominating_row_kernel(const double* __restrict__ Y, int nNew, const double* __restrict__ X, int nOld,
+                                                                   int S, int32_t* first) {
+    __shared__ double xs[DOM_KS][DOM_T + 1], ys[DOM_KS][DOM_T + 1];
+    const int i0 = blockIdx.x * DOM_T, j0 = blockIdx.y * DOM_T;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int i = i0 + lane;
+    const unsigned best = (i < nOld) ? *(volatile unsigned*)(first + i) : 0u;
+    unsigned alive = 0;
+#pragma unroll
+    for (int q = 0; q < 4; q++) {
+        const int j = j0 + warp + 8 * q;
+        if (i < nOld && j < nNew && (unsigned)j < best) alive |= 1u << q;
+    }
+    for (int s0 = 0; s0 < S; s0 += DOM_KS) {
+        if (!__syncthreads_or(alive != 0)) return;                     // also: the tiles of the previous chunk have been read
+#pragma unroll
+        for (int u = 0; u < DOM_T * DOM_KS / 256; u++) {
+            const int r = warp + 8 * u, s = s0 + lane;
+            xs[lane][r] = (i0 + r < nOld && s < S) ? X[(size_t)(i0 + r) * S + s] : 0.0;
+            ys[lane][r] = (j0 + r < nNew && s < S) ? Y[(size_t)(j0 + r) * S + s] : 0.0;
+        }
+        __syncthreads();
+        const int ks = min(DOM_KS, S - s0);
+        for (int c = 0; c < ks && alive; c++) {
+            const double x = xs[c][lane];
+#pragma unroll
+            for (int q = 0; q < 4; q++)
+                if (!(ys[c][warp + 8 * q] >= x)) alive &= ~(1u << q);
+        }
+    }
+    // the lowest surviving j of this thread, then of the block per i: the atomic keeps the lowest over all tiles
+#pragma unroll
+    for (int q = 0; q < 4; q++)
+        if (alive & (1u << q)) {
+            atomicMin((unsigned*)(first + i), (unsigned)(j0 + warp + 8 * q));
+            break;
+        }
+}
+
 // Sawtooth upper bound:  v0_q = q . corner;  terms[q][i] = v0_q + (ub_value_i - ub_belief_i . corner) * min_{s: ub_belief_i[s] > 0} q[s] / ub_belief_i[s];
 // terms[q][nUb] = v0_q;  row_min_kernel then takes out[q] = min_i terms[q][i].
 // One block per STORED belief i, for all queries: b_i is read from HBM once (the first version, one block per (i, q), re-read
@@ -769,6 +816,24 @@ extern "C" int pbvi_prune_dominated(pbvi_model* m, const double* d_alphas, int n
     PBVI_REQUIRE(d_alphas && d_keep, "NULL pointer argument");
     PBVI_CUDA(cudaSetDevice(m->device));
     prune_dominated_kernel<<<nV, 256, 0, (cudaStream_t)stream>>>(d_alphas, nV, m->S, d_keep);
+    m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_first_dominating_row(pbvi_model* m, const double* d_new, int n_new, const double* d_old, int n_old, int32_t* d_first,
+                                         void* stream) {
+    PBVI_REQUIRE(n_new >= 0 && n_old >= 0, "n_new and n_old must be non-negative");
+    PBVI_REQUIRE(n_old == 0 || (d_old && d_first && (n_new == 0 || d_new)), "NULL pointer argument");
+    PBVI_REQUIRE(n_new <= 65535 * DOM_T, "n_new above 65535 * 32 (grid.y)");
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    if (n_old == 0) return PBVI_OK;
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_CUDA(cudaMemsetAsync(d_first, 0xFF, (size_t)n_old * sizeof(int32_t), st));
+    m->last_launches = 0;
+    if (n_new == 0) return PBVI_OK;
+    first_dominating_row_kernel<<<dim3(ceil_div(n_old, DOM_T), ceil_div(n_new, DOM_T)), 256, 0, st>>>(d_new, n_new, d_old, n_old, m->S, d_first);
     m->last_launches = 1;
     PBVI_CUDA(cudaGetLastError());
     return PBVI_OK;

@@ -5,7 +5,8 @@ Finite-state controllers (policy graphs) extracted from a value function, and th
                       V_n = Rbar_{a_n} + gamma * sum_o sum_r RTO[., a_n, o, r] * V_{sigma(n,o)}[reach[., a_n, r]]
                   and max_n V_n . b is the value of a policy that can be executed, hence a lower bound on V*(b) at every belief and for
                   every model, whatever the signs of its rewards.  `evaluate` iterates that fixed point on the device (one
-                  `pbvi_controller_sweep` launch per sweep) and certifies the returned rows with a residual shift.
+                  persistent `pbvi_controller_evaluate` launch) and certifies the returned rows with a residual shift; `improve`
+                  raises that bound by point-based policy iteration on the controller.
 
 The file formats of `save` / `load` are pomdp-solve's: `.pg` ("id action succ_0 ... succ_{O-1}" per node) and `.alpha` (an action line, a
 values line and a blank line per node).
@@ -22,6 +23,28 @@ from .bounds import belief_rows, certificate_contraction
 from .model import Model, log
 from .solver import MDPSolverHistory
 from .value_function import ValueFunction
+
+
+def reachable_subgraph(actions, successors, roots) -> tuple:
+    """
+    The part of a controller that can run from the nodes `roots`: returns (kept node indices ascending, their actions, their successors
+    renumbered to positions in the kept list).  Kept nodes keep their relative order, and every successor of a kept node is kept
+    (whatever the observation, an impossible one included), so the rows of the kept nodes need no re-evaluation.
+    """
+    act = np.asarray(actions, dtype=np.int64).reshape(-1)
+    succ = np.asarray(successors, dtype=np.int64)
+    seen = np.zeros(act.shape[0], dtype=bool)
+    stack = sorted({int(r) for r in np.asarray(roots).reshape(-1)})
+    seen[stack] = True
+    while stack:
+        for t in succ[stack.pop()].tolist():
+            if not seen[t]:
+                seen[t] = True
+                stack.append(t)
+    keep = np.flatnonzero(seen)
+    renumber = np.full(act.shape[0], -1, dtype=np.int64)
+    renumber[keep] = np.arange(len(keep))
+    return keep, act[keep], renumber[succ[keep]]
 
 
 class PolicyGraph:
@@ -143,8 +166,9 @@ class PolicyGraph:
         """
         Certified node values: returns (rows [N, S] CUDA float64, MDPSolverHistory with `sweeps`, `final_change`, `residual`, `shift`).
 
-        Iterates W <- T_pi W (`pbvi_controller_sweep`, one scalar read back per sweep) from the source rows (the Rbar rows of the node
-        actions for a graph without them) until max |T_pi W - W| < eps * gamma / (1 - gamma) or `max_sweeps` sweeps.  Certificate, the
+        Iterates W <- T_pi W (`pbvi_controller_evaluate`: every sweep in one persistent launch, synchronised once) from the source rows
+        (the Rbar rows of the node actions for a graph without them; the start `improve` sets) until max |T_pi W - W| <
+        eps * gamma / (1 - gamma) or `max_sweeps` sweeps.  Certificate, the
         mirror image of FIB_Solver's: with e = max(W - T_pi W) and gamma' = gamma * max(1, max_{s,a} sum_{o,r} RTO) the returned rows are
         W - max(e, 0) / (1 - gamma').  A constant shift c >= 0 passes through T_pi as at most gamma' * c, so they satisfy W <= T_pi W; they
         are re-checked with one more sweep, and while rounding leaves a positive residual e' the rows are lowered again by
@@ -167,16 +191,17 @@ class PolicyGraph:
         history = MDPSolverHistory(1, self.model, gamma, eps, None)
         tol = eps * gamma / (1.0 - gamma)
         change = float('nan')
-        for _ in range(max_sweeps):
+        if max_sweeps >= 1:
+            # the whole iteration is one persistent launch; the sweeps are not timed one by one, so each gets an even share of the wall time
             start = time.perf_counter()
-            W_new, stats = dev.controller_sweep(W, gamma, act, succ, want_stats=True)
-            change = float(stats[2])                                       # one scalar D2H per sweep = the convergence test
-            W = W_new
-            history.add(time.perf_counter() - start, change, None)
+            W, changes, k = dev.controller_evaluate(W, gamma, act, succ, tol, max_sweeps)
+            changes = changes.cpu().numpy().tolist()
+            per_sweep = (time.perf_counter() - start) / k
+            for c in changes:
+                history.add(per_sweep, c, None)
+            change = changes[-1]
             if change != change:
                 raise ValueError('the controller iterates are not finite')
-            if change < tol:
-                break
         residual = float(dev.controller_sweep(W, gamma, act, succ, want_stats=True)[1][1])
         if residual != residual:
             raise ValueError('the controller iterates are not finite')
@@ -201,6 +226,100 @@ class PolicyGraph:
         if print_progress:
             log(f'PolicyGraph: {len(self)} nodes, {history.sweeps} sweeps, residual max(W - TW) = {residual:.3e}, certificate shift {shift:.3e}')
         return self.rows, history
+
+    # ---- improvement -------------------------------------------------------------------------------------------------------
+    def improve(self, beliefs, iterations: int = 1, eps: float = 1e-6) -> tuple:
+        """
+        Point-based policy iteration (Hansen 1998; Ji et al. 2007) over B = b0 followed by the rows of `beliefs`: returns (PolicyGraph,
+        list of per-iteration stats dicts).  Needs an evaluated graph (`rows`, `gamma`).  Each iteration, with W the certified node rows:
+
+          1. backup: `backup_select(B, W)` gives at each b the tuple t_b = (a*_b, v*[b, a*_b, :]), a controller node that plays a*_b and
+             moves to node v*[b, a*_b, o] on o (an impossible observation scores zero everywhere, so it leads to node 0).  Distinct tuples
+             in order of first occurrence; a tuple equal to a node's (action, successors) is that node (the first such).
+          2. rows: Y = `backup_assemble(W)` of the tuples that are not nodes yet.
+          3. Hansen's rule (`first_dominating_row(Y, W)`): an old node dominated by some Y_j takes tuple j's action and successors and keeps
+             its index -- unless some t_b is that node, which stays as it is; a tuple that dominated no node is appended.  The start of the
+             next evaluation is X = W on the old nodes and Y_j on the appended ones.
+          4. `evaluate(gamma, eps)` from X, with its certificate.
+          5. prune: only the nodes reachable from the argmax nodes at B (`max_values` on the certified rows) are kept, renumbered in their
+             old order (`reachable_subgraph`).  Kept nodes point to kept nodes only, so their rows are a subset and stay certified.
+        An iteration that appends and overwrites nothing is the policy-iteration fixed point at B: the graph comes back unchanged.
+
+        Why the bound rises: successors always name old nodes, and X equals W on every old node.  So (T_new X)_n is (T_old W)_n >= W_n
+        (the certificate) for an untouched node, Y_j >= W_n for an overwritten one and Y_j = X_n for an appended one: X <= T_new X.  T_new
+        is monotone and a contraction, so the new controller's value V satisfies V >= T_new X >= X.  Every t_b is played by some node m
+        with (T_new X)_m = Y_{t_b}, so at every b in B the new value is >= the backup value Y_{t_b} . b >= (T_old W)_n . b >= W_n . b for
+        the old argmax node n at b: the old value.  All of this holds in exact arithmetic; the certified rows of step 4 can lie below V
+        by their shift, and that is what a caller sees at most as a fall.  Pruning keeps the argmax nodes of B and everything they reach.
+
+        Stats per iteration: nodes_before, nodes_after, appended, overwritten, pruned, sweeps, value_b0 (certified), shift and
+        seconds {select, assemble, dominance, evaluate, prune}.
+        """
+        self._require_rows()
+        if self.gamma is None:
+            raise ValueError('improve needs the gamma of evaluate: call evaluate(gamma) first')
+        m, gamma = self.model, self.gamma
+        dev = m.device
+        B = belief_rows(m, m.start_probabilities)
+        if beliefs is not None:
+            B = torch.cat([B, belief_rows(m, beliefs)])
+        pg, all_stats = self, []
+        for _ in range(int(iterations)):
+            W, N = pg.rows, len(pg)
+            sec = {}
+            t0 = time.perf_counter()
+            vstar, _, astar = dev.backup_select(B, W, gamma, want_value=False)
+            idx = torch.arange(B.shape[0], device=astar.device)
+            tuples = torch.cat([astar[:, None], vstar[idx, astar.long()]], dim=1).cpu().numpy().astype(np.int64)   # [nB, 1 + O]
+            sec['select'] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            node_of = {}
+            for n in range(N - 1, -1, -1):                                 # the first node with a given tuple wins
+                node_of[(int(pg.actions[n]), *pg.successors[n].tolist())] = n
+            in_use, new = set(), {}
+            for t in map(tuple, tuples.tolist()):
+                if t in node_of:
+                    in_use.add(node_of[t])
+                elif t not in new:
+                    new[t] = len(new)
+            new_t = np.asarray(list(new), dtype=np.int64).reshape(-1, 1 + m.observation_count)
+            Y = dev.backup_assemble(W, gamma, new_t[:, 0], new_t[:, 1:]) if len(new_t) else None
+            torch.cuda.synchronize(dev.device)
+            sec['assemble'] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            dom = dev.first_dominating_row(Y, W).cpu().numpy() if Y is not None else np.full(N, -1)
+            sec['dominance'] = time.perf_counter() - t0
+            actions, successors = pg.actions.copy(), pg.successors.copy()
+            used = np.zeros(len(new_t), dtype=bool)
+            overwritten = 0
+            for n in range(N):
+                j = int(dom[n])
+                if j >= 0 and n not in in_use:
+                    actions[n], successors[n] = new_t[j, 0], new_t[j, 1:]
+                    used[j] = True
+                    overwritten += 1
+            app = np.flatnonzero(~used)
+            stats = dict(nodes_before=N, appended=int(len(app)), overwritten=overwritten)
+            if len(app) == 0 and overwritten == 0:
+                stats.update(nodes_after=N, pruned=0, sweeps=0, value_b0=float(pg.value(B[:1])[0][0]), shift=0.0,
+                             seconds=dict(sec, evaluate=0.0, prune=0.0))
+                all_stats.append(stats)
+                break
+            t0 = time.perf_counter()
+            nxt = PolicyGraph(m, np.concatenate([actions, new_t[app, 0]]), np.concatenate([successors, new_t[app, 1:]]))
+            nxt._initial = torch.cat([W, Y[torch.as_tensor(app, device=W.device)]]).contiguous() if len(app) else W
+            rows, hist = nxt.evaluate(gamma, eps)
+            sec['evaluate'] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            roots = dev.max_values(B, rows)[1].cpu().numpy()
+            keep, k_act, k_succ = reachable_subgraph(nxt.actions, nxt.successors, roots)
+            pg = PolicyGraph(m, k_act, k_succ, rows=rows[torch.as_tensor(keep, device=rows.device)])
+            pg.gamma = gamma
+            sec['prune'] = time.perf_counter() - t0
+            stats.update(nodes_after=len(pg), pruned=len(nxt) - len(pg), sweeps=hist.sweeps, value_b0=float(pg.value(B[:1])[0][0]),
+                         shift=hist.shift, seconds=sec)
+            all_stats.append(stats)
+        return pg, all_stats
 
     def _require_rows(self) -> torch.Tensor:
         if self.rows is None:
