@@ -302,7 +302,27 @@ PBVI_API int pbvi_upper_backup(pbvi_model* m, const double* d_b, int n, const do
                                const int32_t* d_idx, const double* d_val, const int32_t* d_count, const double* d_dot,
                                const double* d_ub_values, int n_ub, double* d_u, double* d_cur, int32_t* d_best_a, void* stream);
 
-/* ---- SSEA novelty score (src/pomdp.py:1682-1686) --------------------------------------------------
+/* ---- one level of K gap-driven trials (GapSolver) -----------------------------------------------------------------------------------
+ * For every trial belief b_k of d_b [K][S], with the upper bound of pbvi_upper_backup (d_fib [k][S], corner values, support lists) and
+ * the lower bound max_n d_lower[n] . b over N rows d_lower [N][S]:
+ *   Q*_k, a*_k  = pbvi_upper_backup's d_u / d_best_a on the same inputs (bitwise: the same launches)
+ *   U_o = min(F, sawtooth)(b_k^{a* o}), L_o = max_n d_lower[n] . b_k^{a* o} and e_o = P_o * ((U_o - L_o) - theta) for every o with
+ *   P_o = P(o|b_k,a*) > 0 (one rounding per operation; L through the pbvi_max_values path on the O successors of a* only);
+ *   o*_k        = without d_uniform or with d_uniform[k] < 0: the first argmax of e over {o : e_o > 0};
+ *                 otherwise drawn from that set with weights e_o by NumPy's rule with the uniform d_uniform[k] (as pbvi_perseus_walk
+ *                 draws an observation: cdf = cumsum(w), cdf /= cdf[-1], searchsorted(cdf, u, 'right'));
+ *                 -1 when no e_o is positive (the trial ends).
+ * d_out4 [K][4] receives {a*, o*, Q*, e_{o*}} as doubles (with o* = -1: the largest e_o of a possible o, -inf when there is none);
+ * d_next [K][S] the next belief b_k^{a* o*}, bitwise pbvi_belief_update(b_k, a*, o*, normalise = 1) (b_k itself when o* = -1);
+ * d_U / d_L [K][O] (nullable, together) U_o and L_o, NaN for impossible observations.  d_uniform [K] is a device array (nullable).
+ * Scratch from the handle's arena: K*A*O*S successors, K*A*O*(n_ub + 1) sawtooth terms and K*O*S rows for L: the caller sizes K.
+ * Enqueues on `stream`, does not synchronise. */
+PBVI_API int pbvi_gap_trial_step(pbvi_model* m, const double* d_b, int K, const double* d_lower, int N, const double* d_fib, int k,
+                                 double gamma, const double* d_corner, const int32_t* d_idx, const double* d_val, const int32_t* d_count,
+                                 const double* d_dot, const double* d_ub_values, int n_ub, double theta, const double* d_uniform,
+                                 double* d_out4, double* d_next, double* d_U, double* d_L, void* stream);
+
+/* ---- SSEA novelty score (src/pomdp.py:1682-1686)--------------------------------------------------
  * d_out[j] = min_i || d_beliefs[i] - d_candidates[j] ||_2 */
 PBVI_API int pbvi_min_l2_distance(pbvi_model* m, const double* d_beliefs, int nB, const double* d_candidates, int nC, double* d_out,
                          void* stream);

@@ -61,6 +61,7 @@ SIGNATURES = {
     'pbvi_support_lists': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth_lists': [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_hsvi_level': [_P, _P, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_double, c_int, _P, _P, _P, _P, _P],
+    'pbvi_gap_trial_step': [_P, _P, c_int, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, c_double, _P, _P, _P, _P, _P, _P],
     'pbvi_min_l2_distance': [_P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_ger_scores': [_P, _P, _P, _P, c_int, c_double, c_double, _P, _P],
     'pbvi_comm_unique_id': [_P],
@@ -605,6 +606,26 @@ class DeviceModel:
                                              float(conv_term), int(bool(may_continue)), _ptr(next_out), _ptr(succ), _ptr(mass), out.ctypes.data,
                                              self._stream))
         return succ, mass, out[:4], out[4:].view(np.int64)
+
+    def gap_trial_step(self, beliefs, lower_rows, fib_rows, gamma: float, corner, idx, val, count, dot, ub_values, n_ub: int, theta: float,
+                       uniforms=None, want_bounds: bool = False):
+        """One level of K gap-driven trials (`pbvi_gap_trial_step`): returns (out [K,4] CUDA float64 = {a*, o*, Q*, e_{o*}} per trial, next
+        beliefs [K,S]), and with `want_bounds` also (U [K,O], L [K,O]).  `uniforms` [K] (None: the argmax rule everywhere; a negative
+        entry: the argmax rule for that trial).  The caller sizes K: the call takes K*A*O*(S + n_ub + 1) doubles of scratch."""
+        b, X, F = self._beliefs(beliefs), self._beliefs(lower_rows), self._beliefs(fib_rows)
+        K = b.shape[0]
+        u = None if uniforms is None else _f64(uniforms, self.device).reshape(-1)
+        assert u is None or u.shape == (K,)
+        out = torch.empty((K, 4), dtype=torch.float64, device=self.device)
+        nxt = torch.empty((K, self.S), dtype=torch.float64, device=self.device)
+        U = torch.empty((K, self.O), dtype=torch.float64, device=self.device) if want_bounds else None
+        L = torch.empty((K, self.O), dtype=torch.float64, device=self.device) if want_bounds else None
+        on = n_ub > 0
+        self._call(self._lib.pbvi_gap_trial_step(self._h, _ptr(b), K, _ptr(X), X.shape[0], _ptr(F), F.shape[0], float(gamma), _ptr(corner),
+                                                 _ptr(idx) if on else None, _ptr(val) if on else None, _ptr(count) if on else None,
+                                                 _ptr(dot) if on else None, _ptr(ub_values) if on else None, int(n_ub), float(theta), _ptr(u),
+                                                 _ptr(out), _ptr(nxt), _ptr(U), _ptr(L), self._stream))
+        return (out, nxt, U, L) if want_bounds else (out, nxt)
 
     def min_l2_distance(self, beliefs, candidates) -> torch.Tensor:
         b, c = self._beliefs(beliefs), self._beliefs(candidates)

@@ -494,3 +494,140 @@ extern "C" int pbvi_upper_backup(pbvi_model* m, const double* d_b, int n, const 
     PBVI_CUDA(cudaGetLastError());
     return PBVI_OK;
 }
+
+// ---- one level of K gap-driven trials (pbvi_gap_trial_step) ---------------------------------------------------------------------
+namespace pbvi {
+// rows[k*O + o] = the successor b_k^{a*_k o} (block per row); zeros for an impossible observation, whose successor is the 0/0 row: the
+// lower bounds of these rows go through the score kernel, and a NaN row would switch its zero-skipping off for the whole call
+__global__ void __launch_bounds__(256) gap_gather_kernel(const double* __restrict__ succ, const double* __restrict__ mass,
+                                                         const int32_t* __restrict__ bestA, int O, int nZ, int S, double* __restrict__ rows) {
+    const int r = blockIdx.x;
+    const int k = r / O, o = r - k * O, a = bestA[k];
+    const size_t z = (size_t)k * nZ + (size_t)max(a, 0) * O + o;
+    const bool live = a >= 0 && mass[z] > 0.0;
+    const double* src = succ + z * S;
+    double* dst = rows + (size_t)r * S;
+    for (int s = threadIdx.x; s < S; s += 256) dst[s] = live ? src[s] : 0.0;
+}
+
+// e_o = P_o * ((U_o - L_o) - theta), one rounding per operation; a NaN excess counts as not positive
+__device__ __forceinline__ double gap_excess(double p, double u, double l, double theta) {
+    return __dmul_rn(p, __dadd_rn(__dadd_rn(u, -l), -theta));
+}
+
+// Thread per trial k: the excess of every possible observation of a*_k and the choice of o*_k.  Without a uniform (or u_k < 0) the
+// first maximiser of e over {e > 0}; otherwise o ~ e over that set by NumPy's rule (w = max(e, 0) over all o, cdf = cumsum(w) with
+// sequential adds, cdf /= cdf[-1], searchsorted(cdf, u, 'right')), capped at the last positive weight so that a uniform outside [0, 1)
+// cannot pick an observation of weight 0.  No positive excess: o*_k = -1.  out4[k] = {a*, o*, Q*, e_{o*}}; with o* = -1, e is the
+// largest excess of a possible observation (-inf when there is none).
+__global__ void __launch_bounds__(128) gap_choose_kernel(const double* __restrict__ mass, const double* __restrict__ fibSucc,
+                                                         const double* __restrict__ sawSucc, const double* __restrict__ lower,
+                                                         const int32_t* __restrict__ bestA, const double* __restrict__ q, int K, int A, int O,
+                                                         double theta, const double* __restrict__ uniform, double* __restrict__ out4,
+                                                         int32_t* __restrict__ bestO, double* __restrict__ uOut, double* __restrict__ lOut) {
+    const int k = blockIdx.x * 128 + threadIdx.x;
+    if (k >= K) return;
+    const int a = bestA[k];                 // -1 only when every Q is NaN: no observation is possible then
+    const size_t z0 = (size_t)k * A * O + (size_t)max(a, 0) * O;
+    double best = 0.0, top = -INFINITY, tot = 0.0;
+    int arg = -1, lastPos = -1;
+    for (int o = 0; o < O; o++) {
+        const double p = a >= 0 ? mass[z0 + o] : 0.0;
+        double u = __longlong_as_double(0x7ff8000000000000ll), l = u;
+        if (p > 0.0) {
+            u = fmin(fibSucc[z0 + o], sawSucc[z0 + o]);
+            l = lower[(size_t)k * O + o];
+            const double e = gap_excess(p, u, l, theta);
+            top = fmax(top, e);
+            if (e > best) { best = e; arg = o; }
+            if (e > 0.0) { tot = __dadd_rn(tot, e); lastPos = o; }
+        }
+        if (uOut) { uOut[(size_t)k * O + o] = u; lOut[(size_t)k * O + o] = l; }
+    }
+    double eStar = top;
+    if (arg >= 0) {
+        eStar = best;
+        const double uk = uniform ? uniform[k] : -1.0;
+        if (uk >= 0.0) {
+            double run = 0.0;
+            int idx = 0;
+            for (int o = 0; o < O; o++) {
+                const double p = mass[z0 + o];
+                if (p > 0.0) {
+                    const double e = gap_excess(p, fmin(fibSucc[z0 + o], sawSucc[z0 + o]), lower[(size_t)k * O + o], theta);
+                    if (e > 0.0) run = __dadd_rn(run, e);
+                }
+                if (__ddiv_rn(run, tot) <= uk) idx++;
+            }
+            arg = min(idx, lastPos);
+            eStar = gap_excess(mass[z0 + arg], fmin(fibSucc[z0 + arg], sawSucc[z0 + arg]), lower[(size_t)k * O + arg], theta);
+        }
+    }
+    out4[(size_t)k * 4 + 0] = a;
+    out4[(size_t)k * 4 + 1] = arg;
+    out4[(size_t)k * 4 + 2] = q[k];
+    out4[(size_t)k * 4 + 3] = eStar;
+    bestO[k] = arg;
+}
+
+// next[k] = b_k^{a*_k o*_k}, the row pbvi_belief_update(b_k, a*_k, o*_k, normalise = 1) gives (same projection and pairwise normaliser);
+// b_k itself when the trial ends (o*_k = -1).  Block per trial.
+__global__ void __launch_bounds__(256) gap_next_kernel(const double* __restrict__ succ, const double* __restrict__ b,
+                                                       const int32_t* __restrict__ bestA, const int32_t* __restrict__ bestO, int O, int nZ,
+                                                       int S, double* __restrict__ next) {
+    const int k = blockIdx.x;
+    const int o = bestO[k];
+    const double* src = o >= 0 ? succ + ((size_t)k * nZ + (size_t)bestA[k] * O + o) * S : b + (size_t)k * S;
+    double* dst = next + (size_t)k * S;
+    for (int s = threadIdx.x; s < S; s += 256) dst[s] = src[s];
+}
+}  // namespace pbvi
+
+extern "C" int pbvi_gap_trial_step(pbvi_model* m, const double* d_b, int K, const double* d_lower, int N, const double* d_fib, int k,
+                                   double gamma, const double* d_corner, const int32_t* d_idx, const double* d_val, const int32_t* d_count,
+                                   const double* d_dot, const double* d_ub_values, int n_ub, double theta, const double* d_uniform,
+                                   double* d_out4, double* d_next, double* d_U, double* d_L, void* stream) {
+    PBVI_REQUIRE(K >= 0 && n_ub >= 0, "counts must be non-negative");
+    PBVI_REQUIRE(N >= 1 && k >= 1, "N >= 1 lower rows and k >= 1 FIB rows are required");
+    PBVI_REQUIRE(theta == theta, "theta is NaN");
+    PBVI_REQUIRE((d_U == nullptr) == (d_L == nullptr), "d_U and d_L go together");
+    if (K > 0) {
+        PBVI_REQUIRE(d_b && d_lower && d_fib && d_corner && d_out4 && d_next, "NULL pointer argument");
+        PBVI_REQUIRE(n_ub == 0 || (d_idx && d_val && d_count && d_dot && d_ub_values), "NULL pointer argument: support lists are required when n_ub > 0");
+    }
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    if (K == 0) return PBVI_OK;
+    const int A = m->A, O = m->O, S = m->S;
+    const size_t nZ = (size_t)K * m->nZ;
+    PBVI_REQUIRE(nZ <= (size_t)INT32_MAX, "too many successors in one call: pass fewer trials");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    m->last_launches = 0;
+    PBVI_TAKE(succ, double, nZ * S);
+    PBVI_TAKE(mass, double, nZ);
+    PBVI_TAKE(fibSucc, double, nZ);
+    PBVI_TAKE(sawSucc, double, nZ);
+    PBVI_TAKE(rb, double, (size_t)K * A);
+    PBVI_TAKE(q, double, (size_t)K);
+    PBVI_TAKE(bestA, int32_t, (size_t)K);
+    PBVI_TAKE(bestO, int32_t, (size_t)K);
+    PBVI_TAKE(rows, double, (size_t)K * O * S);
+    PBVI_TAKE(lower, double, (size_t)K * O);
+    // Q and a* exactly as pbvi_upper_backup computes them (same launches on the same inputs)
+    PBVI_TRY(belief_successors_impl(m, d_b, K, 1, succ, mass, st));
+    PBVI_TRY(few_rows_max_impl(m, succ, (int)nZ, d_fib, k, fibSucc, st));
+    PBVI_TRY(sawtooth_lists_impl(m, d_corner, d_idx, d_val, d_count, d_dot, d_ub_values, n_ub, succ, (int)nZ, mass, sawSucc, st));
+    reward_dots_kernel<<<ceil_div(K * A, 8), 256, 0, st>>>(d_b, K, S, m->rbarNzPtr, m->rbarNzIdx, m->rbarNzVal, A, rb);
+    upper_q_kernel<<<ceil_div(K, 128), 128, 0, st>>>(mass, fibSucc, sawSucc, rb, nullptr, nullptr, K, A, O, gamma, q, nullptr, bestA);
+    // L_o = max_n X_n . b^{a* o} for the O successors of a* only
+    gap_gather_kernel<<<K * O, 256, 0, st>>>(succ, mass, bestA, O, m->nZ, S, rows);
+    m->last_launches += 3;
+    PBVI_TRY(max_values_impl(m, rows, K * O, d_lower, N, lower, nullptr, st));
+    gap_choose_kernel<<<ceil_div(K, 128), 128, 0, st>>>(mass, fibSucc, sawSucc, lower, bestA, q, K, A, O, theta, d_uniform, d_out4, bestO,
+                                                        d_U, d_L);
+    gap_next_kernel<<<K, 256, 0, st>>>(succ, d_b, bestA, bestO, O, m->nZ, S, d_next);
+    m->last_launches += 2;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}

@@ -47,6 +47,35 @@ def reachable_subgraph(actions, successors, roots) -> tuple:
     return keep, act[keep], renumber[succ[keep]]
 
 
+def backup_tuples(dev, beliefs: torch.Tensor, rows: torch.Tensor, gamma: float) -> np.ndarray:
+    """The backup tuple t_b = (a*_b, v*[b, a*_b, 0..O-1]) of every belief against the node rows (`backup_select`): int64 [nB, 1 + O].
+    Read as a controller node, t_b plays a*_b and moves to node v*[b, a*_b, o] on o (an impossible observation scores zero everywhere,
+    so it leads to node 0)."""
+    vstar, _, astar = dev.backup_select(beliefs, rows, gamma, want_value=False)
+    idx = torch.arange(beliefs.shape[0], device=astar.device)
+    return torch.cat([astar[:, None], vstar[idx, astar.long()]], dim=1).cpu().numpy().astype(np.int64)
+
+
+def node_index(actions, successors) -> dict:
+    """(action, successor_0, ..., successor_{O-1}) -> node, the first node with a given tuple winning."""
+    node_of = {}
+    for n in range(len(actions) - 1, -1, -1):
+        node_of[(int(actions[n]), *successors[n].tolist())] = n
+    return node_of
+
+
+def match_tuples(node_of: dict, tuples: np.ndarray) -> tuple:
+    """Splits backup tuples [n, 1 + O] into the nodes that already play one (a set) and the distinct other tuples in order of first
+    occurrence (int64 [m, 1 + O])."""
+    in_use, new = set(), {}
+    for t in map(tuple, tuples.tolist()):
+        if t in node_of:
+            in_use.add(node_of[t])
+        elif t not in new:
+            new[t] = len(new)
+    return in_use, np.asarray(list(new), dtype=np.int64).reshape(-1, tuples.shape[1])
+
+
 class PolicyGraph:
     """
     A finite-state controller over `model`: `actions` [N] and `successors` [N, O] (node indices) as host int64 arrays; after `evaluate` (or
@@ -268,21 +297,11 @@ class PolicyGraph:
             W, N = pg.rows, len(pg)
             sec = {}
             t0 = time.perf_counter()
-            vstar, _, astar = dev.backup_select(B, W, gamma, want_value=False)
-            idx = torch.arange(B.shape[0], device=astar.device)
-            tuples = torch.cat([astar[:, None], vstar[idx, astar.long()]], dim=1).cpu().numpy().astype(np.int64)   # [nB, 1 + O]
+            tuples = backup_tuples(dev, B, W, gamma)
             sec['select'] = time.perf_counter() - t0
             t0 = time.perf_counter()
-            node_of = {}
-            for n in range(N - 1, -1, -1):                                 # the first node with a given tuple wins
-                node_of[(int(pg.actions[n]), *pg.successors[n].tolist())] = n
-            in_use, new = set(), {}
-            for t in map(tuple, tuples.tolist()):
-                if t in node_of:
-                    in_use.add(node_of[t])
-                elif t not in new:
-                    new[t] = len(new)
-            new_t = np.asarray(list(new), dtype=np.int64).reshape(-1, 1 + m.observation_count)
+            node_of = node_index(pg.actions, pg.successors)
+            in_use, new_t = match_tuples(node_of, tuples)
             Y = dev.backup_assemble(W, gamma, new_t[:, 0], new_t[:, 1:]) if len(new_t) else None
             torch.cuda.synchronize(dev.device)
             sec['assemble'] = time.perf_counter() - t0
