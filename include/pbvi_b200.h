@@ -248,6 +248,12 @@ PBVI_API int pbvi_prune_dominated(pbvi_model* m, const double* d_alphas, int nV,
 PBVI_API int pbvi_first_dominating_row(pbvi_model* m, const double* d_new, int n_new, const double* d_old, int n_old, int32_t* d_first,
                                        void* stream);
 
+/* pbvi_dominating_row: pointwise dominance within one row set (PolicyGraph.prune_dominated; same tiling and merge as
+ * pbvi_first_dominating_row).  d_witness[i] = the smallest j != i with d_rows[j][s] >= d_rows[i][s] at every state s and, when j > i,
+ * d_rows[j][s] > d_rows[i][s] at some state; -1 when there is none.  Of equal rows only the first has no witness, so witness chains
+ * cannot cycle; a row with a NaN is never a witness and never has one.  Enqueues on `stream`, does not synchronise. */
+PBVI_API int pbvi_dominating_row(pbvi_model* m, const double* d_rows, int n, int32_t* d_witness, void* stream);
+
 /* ---- LP-domination prune (ValueFunction.prune level 3; the reference's intended Lark / White filter, src/mdp.py:834-906, whose
  * branch fails on the undefined `pruned_alpha_set` at :872) ----------------------------------------------------------------------
  * d_keep[i] = 0 iff a convex combination of the other rows exceeds alpha_i by more than tol = 1e-9*max(1, max|alpha|) at every
@@ -273,6 +279,16 @@ PBVI_API int pbvi_support_lists(pbvi_model* m, const double* d_rows, int n, cons
 PBVI_API int pbvi_sawtooth_lists(pbvi_model* m, const double* d_corner, const int32_t* d_idx, const double* d_val, const int32_t* d_count,
                                  const double* d_dot, const double* d_ub_values, int n_ub, const double* d_queries, int n_q, double* d_out,
                                  void* stream);
+/* pbvi_sawtooth_witness: sawtooth dominance among the stored pairs themselves (UpperBound.prune).  With
+ * s_j(b) = v0(b) + (ub_value_j - dot_j) * min_{s in supp b_j} b[s] / b_j[s] the term pbvi_sawtooth_lists computes for pair j at the query b
+ * (bitwise the same term, v0(b_i) = d_dot[i]), for every stored belief b_i:
+ *   d_self[i] = s_i(b_i);   d_min[i] = min_{j != i} s_j(b_i) (+inf when n_ub = 1);
+ *   d_arg[i]  = the first j != i attaining d_min[i], or -1 when no such term lies below v0(b_i).
+ * The queries are read from the support lists (d_corner: the corner values the lists were built with).  Scratch: min(n_ub, 4 * SMs)
+ * rows of S doubles from the handle's arena; no n_ub x n_ub matrix.  Enqueues on `stream`, does not synchronise. */
+PBVI_API int pbvi_sawtooth_witness(pbvi_model* m, const double* d_corner, const int32_t* d_idx, const double* d_val, const int32_t* d_count,
+                                   const double* d_dot, const double* d_ub_values, int n_ub, double* d_min, int32_t* d_arg, double* d_self,
+                                   void* stream);
 
 /* ---- one level of HSVI's exploration (PBVI_Solver.expand_hsvi, src/pomdp.py:1803-1855) in one call, one synchronisation ---------------
  * For the belief d_b: all A*O successors (d_succ [A][O][S], NaN rows for impossible observations) and masses P(o|b,a) (d_mass [A][O]; both

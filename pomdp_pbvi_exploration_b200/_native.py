@@ -55,11 +55,13 @@ SIGNATURES = {
     'pbvi_upper_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_dominated': [_P, _P, c_int, _P, _P],
     'pbvi_first_dominating_row': [_P, _P, c_int, _P, c_int, _P, _P],
+    'pbvi_dominating_row': [_P, _P, c_int, _P, _P],
     'pbvi_prune_lp': [_P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_lp_stats': [_P, _P],
     'pbvi_sawtooth': [_P, _P, _P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_support_lists': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth_lists': [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int, _P, _P],
+    'pbvi_sawtooth_witness': [_P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
     'pbvi_hsvi_level': [_P, _P, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_double, c_int, _P, _P, _P, _P, _P],
     'pbvi_gap_trial_step': [_P, _P, c_int, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, c_int, c_double, _P, _P, _P, _P, _P, _P],
     'pbvi_min_l2_distance': [_P, _P, c_int, _P, c_int, _P, _P],
@@ -249,6 +251,14 @@ class DeviceModel:
         first = torch.empty((X.shape[0],), dtype=torch.int32, device=self.device)
         self._call(self._lib.pbvi_first_dominating_row(self._h, _ptr(Y), Y.shape[0], _ptr(X), X.shape[0], _ptr(first), self._stream))
         return first
+
+    def dominating_row(self, rows) -> torch.Tensor:
+        """For every row, the smallest other row that is >= it at every state and, when it comes later, > it somewhere, or -1
+        (`pbvi_dominating_row`): int32 [n] CUDA tensor."""
+        X = self._beliefs(rows)
+        witness = torch.empty((X.shape[0],), dtype=torch.int32, device=self.device)
+        self._call(self._lib.pbvi_dominating_row(self._h, _ptr(X), X.shape[0], _ptr(witness), self._stream))
+        return witness
 
     def backup(self, beliefs, alphas, gamma: float):
         """select + assemble for every belief, no dedup: (alpha [nB,S], action [nB], v* [nB,A,O], value [nB,A])."""
@@ -588,6 +598,17 @@ class DeviceModel:
         self._call(self._lib.pbvi_sawtooth_lists(self._h, _ptr(corner), _ptr(idx), _ptr(val), _ptr(count), _ptr(dot), _ptr(ub_values), int(n_ub),
                                                  _ptr(q), q.shape[0], _ptr(out), self._stream))
         return out
+
+    def sawtooth_witness(self, corner, idx, val, count, dot, ub_values, n_ub: int) -> tuple:
+        """Sawtooth dominance among the n_ub stored pairs of the support lists (`pbvi_sawtooth_witness`): returns (min [n_ub] f64 =
+        min_{j != i} s_j(b_i), arg [n_ub] int32 = its first j or -1 when no term lies below v0(b_i), self [n_ub] f64 = s_i(b_i))."""
+        n_ub = int(n_ub)
+        mn = torch.empty((n_ub,), dtype=torch.float64, device=self.device)
+        arg = torch.empty((n_ub,), dtype=torch.int32, device=self.device)
+        own = torch.empty((n_ub,), dtype=torch.float64, device=self.device)
+        self._call(self._lib.pbvi_sawtooth_witness(self._h, _ptr(corner), _ptr(idx), _ptr(val), _ptr(count), _ptr(dot), _ptr(ub_values), n_ub,
+                                                   _ptr(mn), _ptr(arg), _ptr(own), self._stream))
+        return mn, arg, own
 
     def hsvi_level(self, b: torch.Tensor, alphas: torch.Tensor, gamma: float, corner, idx, val, count, dot, ub_values, n_ub: int,
                    stored_keys, stored_vals, n_stored: int, conv_term: float, may_continue: bool, next_out: torch.Tensor | None = None,

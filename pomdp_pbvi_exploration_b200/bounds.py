@@ -36,6 +36,31 @@ def certificate_contraction(model: Model, gamma: float, what: str) -> float:
     return gamma_c
 
 
+def resolve_witnesses(witness) -> np.ndarray:
+    """
+    Where every entry of a dominance prune ends up: witness [n] names, per entry, an entry that may replace it (-1: none).  Returns
+    target [n]: target[i] = i for a kept entry, else the kept entry at the end of i's witness chain.  Chains are followed in index order;
+    a cycle (which the witness rules exclude in exact arithmetic, but rounding may close) keeps its lowest index.
+    """
+    w = np.asarray(witness, dtype=np.int64).reshape(-1)
+    target = np.full(w.shape[0], -1, dtype=np.int64)
+    for i in range(w.shape[0]):
+        path, on_path, j = [], {}, i
+        while target[j] < 0 and w[j] >= 0 and j not in on_path:
+            on_path[j] = len(path)
+            path.append(j)
+            j = int(w[j])
+        if target[j] >= 0:
+            end = int(target[j])
+        elif w[j] < 0:
+            end = j
+        else:
+            end = min(path[on_path[j]:])
+        target[end] = end
+        target[path] = end
+    return target
+
+
 def belief_rows(model: Model, beliefs) -> torch.Tensor:
     """A BeliefSet, a Belief, or an array / tensor of one or more rows as a contiguous CUDA float64 [n,S] tensor; non-finite rows raise
     ValueError."""
@@ -205,6 +230,70 @@ class UpperBound:
         rows = self._rows_of(b)[:1]
         lower = float(self.model.device.max_values(rows, value_function.alpha_vector_array)[0][0])
         return lower, float(self.evaluate(rows)[0])
+
+    # ---- pruning ----------------------------------------------------------------------------------------------------------
+    def prune(self, keep_beliefs=None) -> int:
+        """
+        Drops the stored pairs whose sawtooth term lies above another pair's everywhere; returns how many were dropped.
+
+        With v0(b) = b . corner and s_j(b) = v0(b) + (v_j - b_j . corner) * min_{s in supp b_j} b[s] / b_j[s] (the term of pair j):
+        if s_j(b_i) <= s_i(b_i) = v_i, then s_i(b) >= s_j(b) at every b.  For every s, b[s] >= m_i(b) * b_i[s] and
+        b_i[s] >= m_j(b_i) * b_j[s], so m_j(b) >= m_i(b) * m_j(b_i); and v_j - b_j . corner < 0 for every stored pair, since a pair is
+        stored only below min(F, sawtooth) <= v0 and F does not change.  `pbvi_sawtooth_witness` gives min_{j != i} s_j(b_i), its first
+        j and s_i(b_i); pair i is removable when that j exists and the minimum is <= s_i(b_i), and its witness chain (`resolve_witnesses`)
+        ends at a kept pair.  Soundness does not rest on this: dropping pairs only drops terms from a minimum of upper bounds, and every
+        kept term is computed as before, so the bound never falls, bitwise.  In exact arithmetic it does not rise either; under rounding
+        it can rise by a few ulps of |v_j - b_j . corner|.  So that upper(b0) and upper(b) for b in `keep_beliefs` stay bitwise the same,
+        the first pair that attains the sawtooth minimum at each of them is never dropped (the minimum of independently computed terms
+        does not depend on their order).  The kept pairs are compacted in order on the device and the row-key index is rebuilt: a later
+        `improve` behaves as if the dropped pairs had never been stored.
+        """
+        n = self._n
+        if n == 0:
+            return 0
+        m = self.model
+        idx, val, count, dot, vals, _ = self._lists()
+        mn, arg, own = m.device.sawtooth_witness(self.corner_values, idx, val, count, dot, vals, n)
+        witness = torch.where((arg >= 0) & (mn <= own), arg, torch.full_like(arg, -1)).cpu().numpy().astype(np.int64)
+        keep_rows = self._rows_of(m.start_probabilities)[:1]
+        if keep_beliefs is not None:
+            keep_rows = torch.cat([keep_rows, self._rows_of(keep_beliefs)])
+        for b in keep_rows:
+            p = self._first_attaining_pair(b[None, :])
+            if p >= 0:
+                witness[p] = -1
+        target = resolve_witnesses(witness)
+        keep = np.flatnonzero(target == np.arange(n))
+        if len(keep) == n:
+            return 0
+        k = torch.as_tensor(keep, dtype=torch.int64, device=self._F.device)
+        for t in (self._rows, self._vals, self._idx, self._val, self._count, self._dot):
+            t[:len(keep)] = t[k]
+        renumber = np.full(n, -1, dtype=np.int64)
+        renumber[keep] = np.arange(len(keep))
+        self._index = {key: int(renumber[pos]) for key, pos in self._index.items() if renumber[pos] >= 0}
+        self._n = len(keep)
+        return n - len(keep)
+
+    def _first_attaining_pair(self, b: torch.Tensor) -> int:
+        """The first stored pair whose term equals sawtooth(b), or -1 when v0(b) attains it: a bisection over prefixes of the store
+        (the sawtooth over pairs [0, p) is non-increasing in p and made of the same terms, so the comparison is exact)."""
+        dev = self.model.device
+        idx, val, count, dot, vals, n = self._lists()
+
+        def saw(p):
+            return float(dev.sawtooth_lists(self.corner_values, idx, val, count, dot, vals, p, b)[0])
+        full = saw(n)
+        if not full < saw(0):
+            return -1
+        lo, hi = 1, n
+        while lo < hi:
+            mid = (lo + hi) // 2
+            if saw(mid) == full:
+                hi = mid
+            else:
+                lo = mid + 1
+        return lo - 1
 
     # ---- point-based backups ----------------------------------------------------------------------------------------------
     def _chunk(self, n_left: int) -> int:

@@ -129,6 +129,81 @@ __global__ void __launch_bounds__(256) sawtooth_lists_kernel(const int32_t* __re
     }
 }
 
+// Sawtooth dominance among the stored pairs (pbvi_sawtooth_witness): the queries are the stored beliefs b_i themselves.  A block takes one
+// query at a time and scatters b_i's support list into its own zeroed dense row (global scratch, zeroed again afterwards), so that
+// q[s] / b_j[s] reads exactly what sawtooth_lists_kernel reads from the dense query.  v0 = dot[i]: support_lists_kernel sums b_i . corner
+// in the reduction shape of sawtooth_v0_terms_kernel, so it is bitwise the v0 of that query.  Warp per stored pair j: a list longer than
+// b_i's has a state outside supp b_i (ratio 0, m = 0 without a walk); otherwise the warp walks b_j's list 32 entries at a time and stops
+// at the first zero ratio, as sawtooth_lists_kernel does.  Each warp keeps its smallest term (first j on ties, j ascending), the block
+// merges the eight warps; no n_ub x n_ub matrix is formed.
+constexpr int WIT_BLOCKS_PER_SM = 4;
+
+__global__ void __launch_bounds__(256) sawtooth_witness_kernel(const int32_t* __restrict__ idx, const double* __restrict__ val,
+                                                               const int32_t* __restrict__ count, const double* __restrict__ dot,
+                                                               const double* __restrict__ ubV, int nUb, int S, double* __restrict__ dense,
+                                                               double* __restrict__ dMin, int32_t* __restrict__ dArg, double* __restrict__ dSelf) {
+    __shared__ double s_term[8];
+    __shared__ int s_arg[8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double* q = dense + (size_t)blockIdx.x * S;
+    for (int i = blockIdx.x; i < nUb; i += gridDim.x) {
+        const int ci = count[i];
+        const int32_t* li = idx + (size_t)i * S;
+        const double* lvi = val + (size_t)i * S;
+        for (int k = threadIdx.x; k < ci; k += 256) q[li[k]] = lvi[k];
+        __syncthreads();
+        const double v0 = dot[i];
+        double best = INFINITY;
+        int arg = -1;
+        for (int j = warp; j < nUb; j += 8) {
+            const int cj = count[j];
+            double m = 0.0;
+            if (cj <= ci) {
+                const int32_t* lj = idx + (size_t)j * S;
+                const double* lvj = val + (size_t)j * S;
+                double r = INFINITY;
+                for (int k0 = 0; k0 < cj; k0 += 32) {
+                    const int k = k0 + lane;
+                    if (k < cj) r = fmin(r, q[lj[k]] / lvj[k]);
+                    if (__any_sync(0xffffffffu, r == 0.0)) {
+                        r = 0.0;
+                        break;
+                    }
+                }
+#pragma unroll
+                for (int off = 16; off > 0; off >>= 1) r = fmin(r, __shfl_xor_sync(0xffffffffu, r, off));
+                m = r;
+            }
+            const double scale = ubV[j] - dot[j];
+            const double t = v0 + scale * m;
+            if (j == i) {
+                if (lane == 0) dSelf[i] = t;
+            } else if (t < best) {
+                best = t;
+                arg = j;
+            }
+        }
+        if (lane == 0) {
+            s_term[warp] = best;
+            s_arg[warp] = arg;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double t = s_term[0];
+            int a = s_arg[0];
+            for (int w = 1; w < 8; w++)
+                if (s_arg[w] >= 0 && (s_term[w] < t || (s_term[w] == t && (a < 0 || s_arg[w] < a)))) {
+                    t = s_term[w];
+                    a = s_arg[w];
+                }
+            dMin[i] = t;
+            dArg[i] = (t < v0) ? a : -1;
+        }
+        for (int k = threadIdx.x; k < ci; k += 256) q[li[k]] = 0.0;
+        __syncthreads();
+    }
+}
+
 // v0[q] = queries[q] . corner (same reduction shape as sawtooth_v0_kernel); also terms[q][nUb] = v0[q]
 __global__ void __launch_bounds__(256) sawtooth_v0_terms_kernel(const double* __restrict__ corner, const double* __restrict__ queries, int S, int nUb,
                                                                 double* __restrict__ v0, double* __restrict__ terms) {
@@ -408,6 +483,26 @@ extern "C" int pbvi_sawtooth_lists(pbvi_model* m, const double* d_corner, const 
     PBVI_TRY(enter_call(m, (cudaStream_t)stream));
     m->last_launches = 0;
     return sawtooth_lists_impl(m, d_corner, d_idx, d_val, d_count, d_dot, d_ub_values, n_ub, d_queries, n_q, nullptr, d_out, (cudaStream_t)stream);
+}
+
+extern "C" int pbvi_sawtooth_witness(pbvi_model* m, const double* d_corner, const int32_t* d_idx, const double* d_val, const int32_t* d_count,
+                                     const double* d_dot, const double* d_ub_values, int n_ub, double* d_min, int32_t* d_arg, double* d_self,
+                                     void* stream) {
+    PBVI_REQUIRE(n_ub >= 0, "n_ub must be non-negative");
+    PBVI_REQUIRE(n_ub == 0 || (d_corner && d_idx && d_val && d_count && d_dot && d_ub_values && d_min && d_arg && d_self), "NULL pointer argument");
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    m->last_launches = 0;
+    if (n_ub == 0) return PBVI_OK;
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    const int blocks = std::min(n_ub, m->sm_count * WIT_BLOCKS_PER_SM);
+    PBVI_TAKE(dense, double, (size_t)blocks * m->S);
+    PBVI_CUDA(cudaMemsetAsync(dense, 0, (size_t)blocks * m->S * sizeof(double), st));
+    sawtooth_witness_kernel<<<blocks, 256, 0, st>>>(d_idx, d_val, d_count, d_dot, d_ub_values, n_ub, m->S, dense, d_min, d_arg, d_self);
+    m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
 }
 
 extern "C" int pbvi_hsvi_level(pbvi_model* m, const double* d_b, const double* d_alphas, int nV, double gamma, const double* d_corner,

@@ -358,8 +358,11 @@ __global__ void __launch_bounds__(256) prune_dominated_kernel(const double* __re
 // violating state and the block stops when none is left.  first[] starts at -1 (all ones) and the tiles meet through an unsigned
 // atomicMin, so the result does not depend on the order of the blocks; a pair whose j is not below the best j already found for its i is
 // dropped at the start.
+// kSelf (pbvi_dominating_row: Y and X are the same rows): the pair j = i is excluded, and a pair with j > i also has to be strictly greater
+// at some state ("above" collects that bit per pair), so that of two equal rows only the later one has a witness.
 constexpr int DOM_T = 32, DOM_KS = 32;
 
+template <bool kSelf>
 __global__ void __launch_bounds__(256) first_dominating_row_kernel(const double* __restrict__ Y, int nNew, const double* __restrict__ X, int nOld,
                                                                    int S, int32_t* first) {
     __shared__ double xs[DOM_KS][DOM_T + 1], ys[DOM_KS][DOM_T + 1];
@@ -367,11 +370,11 @@ __global__ void __launch_bounds__(256) first_dominating_row_kernel(const double*
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int i = i0 + lane;
     const unsigned best = (i < nOld) ? *(volatile unsigned*)(first + i) : 0u;
-    unsigned alive = 0;
+    unsigned alive = 0, above = 0;
 #pragma unroll
     for (int q = 0; q < 4; q++) {
         const int j = j0 + warp + 8 * q;
-        if (i < nOld && j < nNew && (unsigned)j < best) alive |= 1u << q;
+        if (i < nOld && j < nNew && (unsigned)j < best && (!kSelf || j != i)) alive |= 1u << q;
     }
     for (int s0 = 0; s0 < S; s0 += DOM_KS) {
         if (!__syncthreads_or(alive != 0)) return;                     // also: the tiles of the previous chunk have been read
@@ -386,9 +389,17 @@ __global__ void __launch_bounds__(256) first_dominating_row_kernel(const double*
         for (int c = 0; c < ks && alive; c++) {
             const double x = xs[c][lane];
 #pragma unroll
-            for (int q = 0; q < 4; q++)
-                if (!(ys[c][warp + 8 * q] >= x)) alive &= ~(1u << q);
+            for (int q = 0; q < 4; q++) {
+                const double y = ys[c][warp + 8 * q];
+                if (!(y >= x)) alive &= ~(1u << q);
+                if (kSelf && y > x) above |= 1u << q;
+            }
         }
+    }
+    if (kSelf) {
+#pragma unroll
+        for (int q = 0; q < 4; q++)
+            if (j0 + warp + 8 * q > i && !(above & (1u << q))) alive &= ~(1u << q);
     }
     // the lowest surviving j of this thread, then of the block per i: the atomic keeps the lowest over all tiles
 #pragma unroll
@@ -833,7 +844,24 @@ extern "C" int pbvi_first_dominating_row(pbvi_model* m, const double* d_new, int
     PBVI_CUDA(cudaMemsetAsync(d_first, 0xFF, (size_t)n_old * sizeof(int32_t), st));
     m->last_launches = 0;
     if (n_new == 0) return PBVI_OK;
-    first_dominating_row_kernel<<<dim3(ceil_div(n_old, DOM_T), ceil_div(n_new, DOM_T)), 256, 0, st>>>(d_new, n_new, d_old, n_old, m->S, d_first);
+    first_dominating_row_kernel<false><<<dim3(ceil_div(n_old, DOM_T), ceil_div(n_new, DOM_T)), 256, 0, st>>>(d_new, n_new, d_old, n_old, m->S,
+                                                                                                             d_first);
+    m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_dominating_row(pbvi_model* m, const double* d_rows, int n, int32_t* d_witness, void* stream) {
+    PBVI_REQUIRE(n >= 0, "n must be non-negative");
+    PBVI_REQUIRE(n == 0 || (d_rows && d_witness), "NULL pointer argument");
+    PBVI_REQUIRE(n <= 65535 * DOM_T, "n above 65535 * 32 (grid.y)");
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    m->last_launches = 0;
+    if (n == 0) return PBVI_OK;
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_CUDA(cudaMemsetAsync(d_witness, 0xFF, (size_t)n * sizeof(int32_t), st));
+    first_dominating_row_kernel<true><<<dim3(ceil_div(n, DOM_T), ceil_div(n, DOM_T)), 256, 0, st>>>(d_rows, n, d_rows, n, m->S, d_witness);
     m->last_launches = 1;
     PBVI_CUDA(cudaGetLastError());
     return PBVI_OK;

@@ -18,7 +18,7 @@ import torch
 
 from .bounds import FIB_Solver, UpperBound, belief_rows, certificate_contraction
 from .model import Model, log
-from .policy_graph import PolicyGraph, backup_tuples, match_tuples, node_index, reachable_subgraph
+from .policy_graph import PolicyGraph, backup_tuples, match_tuples, node_index, reachable_subgraph, redirect_dominated
 
 
 class GapSolverHistory:
@@ -29,7 +29,8 @@ class GapSolverHistory:
       shift          the certificate shift of the last `evaluate`
       rounds         one dict per round: round, seconds (wall time since the start), upper_b0, lower_b0 (max_n X_n . b0 of the
                      uncertified rows), nodes, stored_pairs, depths (per trial: depth of its last belief), phase_seconds {descent, lower,
-                     upper, certify} and, in the rounds that certified, certified_lower / certified_upper
+                     upper, certify} and, in the rounds that certified, certified_lower / certified_upper; with prune_growth also
+                     pruned_nodes, pruned_pairs (nodes and stored_pairs are the counts after the prune) and phase_seconds['prune']
       seconds        wall time of the whole solve
       uncertified    the append-only controller with its rows X before the last certificate (X <= T_pi X)
     """
@@ -87,6 +88,22 @@ class _AppendOnlyGraph:
         self.n += k
         return k
 
+    def prune(self) -> int:
+        """Drops the nodes whose row X_i another row dominates at every state and redirects their edges (`redirect_dominated`); returns
+        how many were dropped.  Each predecessor then sees a successor row at least as large and no other entry changes, so
+        X <= T_pi X still holds, and max_n X_n . b is bitwise unchanged (see `PolicyGraph.prune_dominated`).  node_of is rebuilt; two
+        nodes that now carry the same tuple both stay (both rows satisfy the invariant), and the tuple maps to the lower one."""
+        witness = self.model.device.dominating_row(self.rows).cpu().numpy()
+        keep, act, succ = redirect_dominated(self.actions, self.successors, witness)
+        if len(keep) == self.n:
+            return 0
+        removed = self.n - len(keep)
+        self._X[:len(keep)] = self._X[torch.as_tensor(keep, device=self._X.device)]
+        self.actions, self.successors = list(act), list(succ)
+        self.node_of = node_index(self.actions, self.successors)
+        self.n = len(keep)
+        return removed
+
     def certify(self, b0: torch.Tensor, eps: float) -> tuple:
         """(certified PolicyGraph pruned to what b0's best node reaches, its value at b0, the certificate shift)."""
         act, succ = np.asarray(self.actions), np.stack(self.successors)
@@ -127,17 +144,26 @@ class GapSolver:
          `UpperBound.improve`.
       3. When upper(b0) - max_n X_n . b0 <= target_gap the controller is certified (`PolicyGraph.evaluate` from X, then
          `reachable_subgraph`); the solve ends if the certified gap is within the target.
+      With `prune_growth` = f > 1, after step 2: when the node count has reached f times its count after the last prune (at the start:
+         the starting controller), dominated nodes are dropped (`_AppendOnlyGraph.prune`); the stored pairs are pruned on the same rule
+         (`UpperBound.prune`, b0 protected).  Neither prune changes upper(b0) or max_n X_n . b0 by a bit, and both keep the
+         certificates.  With None (the default) nothing is pruned and a solve is the solve without pruning.
     `max_rounds` and `time_limit` (seconds, checked before each round) also end a solve; the returned graph is certified either way.
-    Upper(b0) never rises (stored upper values only decrease) and the uncertified lower(b0) never falls (nodes are only appended).
+    Upper(b0) never rises (stored upper values only decrease, and a prune keeps the pair that attains it) and the uncertified
+    lower(b0) never falls (nodes are only appended, and a prune only drops nodes that another node dominates).
     The solve is deterministic for a given seed; with trials = 1 the seed is not used.
     """
 
-    def __init__(self, gamma: float, target_gap: float, trials: int = 8, max_depth: int = 200, seed: int = 0):
+    def __init__(self, gamma: float, target_gap: float, trials: int = 8, max_depth: int = 200, seed: int = 0,
+                 prune_growth: float | None = None):
         if not target_gap > 0.0:
             raise ValueError('target_gap must be positive')
         if trials < 1 or max_depth < 1:
             raise ValueError('trials and max_depth must be at least 1')
+        if prune_growth is not None and not float(prune_growth) > 1.0:
+            raise ValueError('prune_growth must be None or a factor above 1')
         self.gamma, self.target_gap, self.trials, self.max_depth, self.seed = float(gamma), float(target_gap), int(trials), int(max_depth), seed
+        self.prune_growth = None if prune_growth is None else float(prune_growth)
 
     def solve(self, model: Model, max_rounds: int = 100, time_limit: float | None = None, lower: PolicyGraph | None = None,
               upper: UpperBound | None = None, eps: float = 1e-6, print_progress: bool = False) -> tuple:
@@ -165,6 +191,7 @@ class GapSolver:
         rng = np.random.default_rng(self.seed)
         history = GapSolverHistory(gamma, target, K, self.max_depth, self.seed)
         certified, cert_at = None, -1                  # the last certified graph and the node count it was made from
+        nodes_at_prune, pairs_at_prune = graph.n, len(upper)
 
         def sync_time():
             torch.cuda.synchronize(dev.device)
@@ -217,7 +244,21 @@ class GapSolver:
                 sec['upper'] += t2 - t1
             up_b0 = float(upper.evaluate(b0)[0])
             lo_b0 = float(dev.max_values(b0, graph.rows)[0][0])
+            if self.prune_growth is not None:
+                t0 = time.perf_counter()
+                pruned_nodes = pruned_pairs = 0
+                if graph.n >= self.prune_growth * max(nodes_at_prune, 1):
+                    pruned_nodes = graph.prune()
+                    nodes_at_prune = graph.n
+                    if pruned_nodes:
+                        cert_at = -1                  # the last certificate was made from rows that are gone
+                if len(upper) >= self.prune_growth * max(pairs_at_prune, 1):
+                    pruned_pairs = upper.prune()
+                    pairs_at_prune = len(upper)
+                sec['prune'] = sync_time() - t0
             rec = dict(round=rnd, upper_b0=up_b0, lower_b0=lo_b0, nodes=graph.n, stored_pairs=len(upper), depths=depths.tolist())
+            if self.prune_growth is not None:
+                rec.update(pruned_nodes=pruned_nodes, pruned_pairs=pruned_pairs)
             # ---- 3. certificate ----
             if up_b0 - lo_b0 <= target:
                 t0 = time.perf_counter()

@@ -19,7 +19,7 @@ import time
 import numpy as np
 import torch
 
-from .bounds import belief_rows, certificate_contraction
+from .bounds import belief_rows, certificate_contraction, resolve_witnesses
 from .model import Model, log
 from .solver import MDPSolverHistory
 from .value_function import ValueFunction
@@ -45,6 +45,21 @@ def reachable_subgraph(actions, successors, roots) -> tuple:
     renumber = np.full(act.shape[0], -1, dtype=np.int64)
     renumber[keep] = np.arange(len(keep))
     return keep, act[keep], renumber[succ[keep]]
+
+
+def redirect_dominated(actions, successors, witness) -> tuple:
+    """
+    Drops the nodes that have a witness (`pbvi_dominating_row`: a row >= theirs at every state) and sends every edge that pointed to a
+    dropped node to the kept node at the end of its witness chain (`resolve_witnesses`), node-0 and impossible-observation edges
+    included: returns (kept node indices ascending, their actions, their successors renumbered to positions in the kept list).
+    """
+    act = np.asarray(actions, dtype=np.int64).reshape(-1)
+    succ = np.asarray(successors, dtype=np.int64)
+    target = resolve_witnesses(witness)
+    keep = np.flatnonzero(target == np.arange(act.shape[0]))
+    renumber = np.full(act.shape[0], -1, dtype=np.int64)
+    renumber[keep] = np.arange(len(keep))
+    return keep, act[keep], renumber[target[succ[keep]]]
 
 
 def backup_tuples(dev, beliefs: torch.Tensor, rows: torch.Tensor, gamma: float) -> np.ndarray:
@@ -339,6 +354,25 @@ class PolicyGraph:
                          shift=hist.shift, seconds=sec)
             all_stats.append(stats)
         return pg, all_stats
+
+    def prune_dominated(self) -> 'PolicyGraph':
+        """
+        The graph without its pointwise-dominated nodes: a new PolicyGraph with the kept rows and `gamma`; this graph is not changed.
+
+        Node i is dropped when some node j has W_j >= W_i at every state (`pbvi_dominating_row`: the smallest such j != i, and when j > i
+        it must also be larger somewhere, so equal rows keep their first copy and witness chains cannot cycle; a row with a NaN is never a
+        witness and never has one), and every edge to i goes to the kept node at the end of its witness chain (`redirect_dominated`).
+        The RTO weights are non-negative, so every predecessor p sees a successor row that is at least as large:
+        (T_new W)_p >= (T_old W)_p >= W_p, and no other row or entry changes.  The certificate W <= T_pi W therefore still holds and the
+        kept rows need no re-evaluation.  max_n W_n . b is unchanged at every belief, bitwise in FP64: `max_values` sums every row in the
+        same order with b >= 0, and rounded products, sums and FMAs are monotone in each argument, so the computed value of W_j is >= that
+        of W_i.
+        """
+        W = self._require_rows()
+        keep, act, succ = redirect_dominated(self.actions, self.successors, self.model.device.dominating_row(W).cpu().numpy())
+        pg = PolicyGraph(self.model, act, succ, rows=W[torch.as_tensor(keep, device=W.device)])
+        pg.gamma = self.gamma
+        return pg
 
     def _require_rows(self) -> torch.Tensor:
         if self.rows is None:
