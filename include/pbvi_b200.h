@@ -104,6 +104,22 @@ PBVI_API int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n, 
                                       const int32_t* d_succ, double tol, int max_sweeps, double* d_out, double* d_changes,
                                       int* h_sweeps, void* stream);
 
+/* pbvi_controller_outcomes: exact outcomes of a controller whose runs stop at end states (Simulation.run_action's rule: a run stops
+ * after a step that lands in an end state or plays an end action; that step's reward counts).  With c(s,a,r) = 0 when d_end_state[reach[s,a,r]]
+ * or d_end_action[a] is non-zero and 1 otherwise, `steps` = H sweeps from zero rows of
+ *   d_success[i][s] = sum_o sum_r RTO[s,a_i,o,r] * (c ? P(succ_i[o], reach) : 1)              P(T <= k) of a run started in (node i, s)
+ *   d_steps[i][s]   = 1 + sum_o sum_r RTO[s,a_i,o,r] * (c ? M(succ_i[o], reach) : 0)          E[min(T, k)]
+ *   d_return[i][s]  = Rbar[s,a_i] + ((G_0 + G_1) + ...),  G_o = gamma * sum_r RTO * (c ? G(succ_i[o], reach) : 0)   sum_t gamma^t r_t
+ * in pbvi_controller_sweep's order (with nothing ending, d_return after k steps is bitwise k pbvi_controller_sweep calls from zero
+ * rows), in one persistent cooperative launch.  d_end_state [S] and d_end_action [A] are uint8 flags; indices are clamped into range.
+ * For q query pairs (belief d_queries[j] [S], start node d_query_nodes[j]) d_series [steps][q][3] receives b_j . {P, M, G}_k(node_j)
+ * after every sweep k = 1..H (a fixed-shape reduction: bitwise repeatable); with q = 0 or steps = 0 the query pointers may be NULL.
+ * steps = 0 gives zero rows.  Synchronises `stream` once, at the end. */
+PBVI_API int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, const uint8_t* d_end_state,
+                                      const uint8_t* d_end_action, double gamma, int steps, const double* d_queries,
+                                      const int32_t* d_query_nodes, int q, double* d_success, double* d_steps, double* d_return,
+                                      double* d_series, void* stream);
+
 /* pbvi_backup: select + assemble for every belief (no dedup): d_out_alpha [nB][S], d_out_action [nB];
  * d_out_vstar [nB][A][O] and d_out_value [nB][A] may be NULL. */
 PBVI_API int pbvi_backup(pbvi_model* m, const double* d_beliefs, int nB, const double* d_alphas, int nV, double gamma,

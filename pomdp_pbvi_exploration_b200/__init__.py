@@ -20,7 +20,7 @@ _LAZY = {
     'RewardSet': 'simulation',
     'load_POMDP_file': 'pomdp_file', 'save_POMDP_file': 'pomdp_file', 'parse_POMDP': 'pomdp_file',
     'DeviceModel': '_native', 'ShardedBackup': 'parallel', 'ShardedSolveState': 'parallel', 'NativeComm': 'parallel',
-    'FIB_Solver': 'bounds', 'UpperBound': 'bounds', 'PolicyGraph': 'policy_graph',
+    'FIB_Solver': 'bounds', 'UpperBound': 'bounds', 'PolicyGraph': 'policy_graph', 'ControllerOutcomes': 'policy_graph',
     'GapSolver': 'gap_solver', 'GapSolverHistory': 'gap_solver',
 }
 

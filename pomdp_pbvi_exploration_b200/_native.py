@@ -31,6 +31,7 @@ SIGNATURES = {
     'pbvi_backup_assemble': [_P, _P, c_int, c_double, _P, _P, c_int, _P, _P, _P],
     'pbvi_controller_sweep': [_P, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_controller_evaluate': [_P, _P, c_int, c_double, _P, _P, c_double, c_int, _P, _P, POINTER(c_int), _P],
+    'pbvi_controller_outcomes': [_P, c_int, _P, _P, _P, _P, c_double, c_int, _P, _P, c_int, _P, _P, _P, _P, _P],
     'pbvi_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_backup_host': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P],
     'pbvi_backup_host_unique': [_P, _P, c_int, _P, c_int, c_double, _P, c_int, _P, POINTER(c_int), _P],
@@ -243,6 +244,26 @@ class DeviceModel:
         self._call(self._lib.pbvi_controller_evaluate(self._h, _ptr(W), n, float(gamma), _ptr(act), _ptr(sc), float(tol), int(max_sweeps),
                                                       _ptr(out), _ptr(changes), byref(k), self._stream))
         return out, changes[:k.value], k.value
+
+    def controller_outcomes(self, actions, succ, end_state, end_action, gamma: float, steps: int, queries, query_nodes):
+        """`steps` sweeps of the outcome recursions of a controller whose runs stop at end states (`pbvi_controller_outcomes`, one
+        persistent launch): returns (success, steps, return) rows [n,S] and the series [steps, q, 3] of b_j . {P, M, G}_k(query_nodes[j])
+        after every sweep, CUDA float64.  `end_state` [S] / `end_action` [A] are flags (non-zero: ends).  Synchronises."""
+        act, sc = _i32(actions, self.device), _i32(succ, self.device)
+        n = act.shape[0]
+        assert sc.shape == (n, self.O)
+        es = torch.as_tensor(np.asarray(end_state) != 0, device=self.device).to(torch.uint8).contiguous()
+        ea = torch.as_tensor(np.asarray(end_action) != 0, device=self.device).to(torch.uint8).contiguous()
+        assert es.shape == (self.S,) and ea.shape == (self.A,)
+        b = self._beliefs(queries)
+        qn = _i32(query_nodes, self.device).reshape(-1)
+        q = b.shape[0]
+        assert qn.shape == (q,)
+        P, M, G = (torch.empty((n, self.S), dtype=torch.float64, device=self.device) for _ in range(3))
+        series = torch.empty((int(steps), q, 3), dtype=torch.float64, device=self.device)
+        self._call(self._lib.pbvi_controller_outcomes(self._h, n, _ptr(act), _ptr(sc), _ptr(es), _ptr(ea), float(gamma), int(steps), _ptr(b),
+                                                      _ptr(qn), q, _ptr(P), _ptr(M), _ptr(G), _ptr(series), self._stream))
+        return P, M, G, series
 
     def first_dominating_row(self, new_rows, old_rows) -> torch.Tensor:
         """For every row of `old_rows`, the first row of `new_rows` that is >= it at every state, or -1 (`pbvi_first_dominating_row`):

@@ -19,6 +19,9 @@
 //   controller_sweep_kernel   the same rows for the nodes of a finite-state controller against its own rows, plus a fused residual
 // pbvi_controller_evaluate:
 //   controller_evaluate_kernel   persistent cooperative launch: the sweeps of controller_sweep_kernel until the change test stops them
+// pbvi_controller_outcomes:
+//   controller_outcomes_kernel   persistent cooperative launch: H sweeps of the success / step / return recursions of a controller that
+//                                stops at end states, plus b . row of query pairs after every sweep
 #include <algorithm>
 #include <thread>
 
@@ -612,6 +615,124 @@ __global__ void __launch_bounds__(CTRL_THREADS) controller_evaluate_kernel(const
         const size_t total = (size_t)n * S;
         for (size_t e = (size_t)blockIdx.x * CTRL_THREADS + threadIdx.x; e < total; e += (size_t)gridDim.x * CTRL_THREADS) bufA[e] = __ldcg(bufB + e);
     }
+}
+
+// ---- H sweeps of the outcome recursions of a controller that stops at end states (pbvi_controller_outcomes), one cooperative launch.
+//      With c = 0 when reach[s,a,r] is an end state or a is an end action (1 otherwise), sweep k + 1 computes from the rows of step k
+//          P(n,s) = sum_o sum_r RTO * (c ? P_k(succ_o, s') : 1)
+//          M(n,s) = 1 + sum_o sum_r RTO * (c ? M_k(succ_o, s') : 0)
+//          G(n,s) = Rbar[s,a] + sum_o gamma * sum_r RTO * (c ? G_k(succ_o, s') : 0)
+//      in alpha_a_entry's order (r inside, then o, one rounding per operation, the same zero-RTO skip), so G is bitwise the
+//      controller sweep when nothing ends.  Step 0 is the zero rows: sweep 0 gathers nothing.  The reach / RTO reads and the flag
+//      lookups are shared by the three recurrences.  Blocks stride over the (node, 256-state) items as controller_evaluate_kernel does;
+//      the rows of step k live in out* when H - k is even and in tmp* otherwise, so step H lands in out*, and one grid barrier
+//      separates the sweeps.  Query pair j (belief row j, node qnode[j]) gets b_j . {P, M, G}_k(qnode[j]) in series[k-1][j][0..2]:
+//      block j % gridDim reduces it at the start of sweep k + 1 (the rows of step k are complete after the barrier and are overwritten
+//      only after the next one) or after the loop for k = H.  The dot product has a fixed shape -- thread t sums states t, t + 256, ...
+//      in order, skipping b = 0, then block_sum_256's tree -- so it does not depend on the grid size and a call is bitwise repeatable.
+__device__ __forceinline__ void outcome_queries(const double* __restrict__ queries, const int32_t* __restrict__ qnode, int q, int n, int S,
+                                                const double* P, const double* M, const double* G, double* __restrict__ series, double* sh) {
+    for (int j = blockIdx.x; j < q; j += gridDim.x) {
+        const int i = min(max(qnode[j], 0), n - 1);
+        const double* b = queries + (size_t)j * S;
+        const size_t row = (size_t)i * S;
+        double p = 0.0, m = 0.0, g = 0.0;
+        for (int s = threadIdx.x; s < S; s += CTRL_THREADS) {
+            const double bv = b[s];
+            if (bv != 0.0) {
+                p = __dadd_rn(p, __dmul_rn(bv, __ldcg(P + row + s)));
+                m = __dadd_rn(m, __dmul_rn(bv, __ldcg(M + row + s)));
+                g = __dadd_rn(g, __dmul_rn(bv, __ldcg(G + row + s)));
+            }
+        }
+        __syncthreads();                                               // sh of the previous use has been read
+        p = block_sum_256(p, sh);
+        __syncthreads();
+        m = block_sum_256(m, sh);
+        __syncthreads();
+        g = block_sum_256(g, sh);
+        if (threadIdx.x == 0) {
+            series[3 * (size_t)j] = p;
+            series[3 * (size_t)j + 1] = m;
+            series[3 * (size_t)j + 2] = g;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(CTRL_THREADS) controller_outcomes_kernel(int n, const int32_t* __restrict__ actions, const int32_t* __restrict__ succ,
+                                                                           const uint8_t* __restrict__ endState, const uint8_t* __restrict__ endAction,
+                                                                           const int32_t* __restrict__ reachK, const double* __restrict__ rtoK,
+                                                                           const double* __restrict__ rbarT, double gamma, int S, int R, int O, int A,
+                                                                           int sBlocks, bool skipZero, int H, double* outP, double* outM, double* outG,
+                                                                           double* tmpP, double* tmpM, double* tmpG, const double* __restrict__ queries,
+                                                                           const int32_t* __restrict__ qnode, int q, double* __restrict__ series) {
+    extern __shared__ int s_vsel[];
+    __shared__ double sh[CTRL_THREADS / 32];
+    cg::grid_group grid = cg::this_grid();
+    const int items = n * sBlocks;
+    for (int k = 0; k < H; k++) {
+        // rows written earlier in this launch are read with ld.global.cg, never through the read-only data cache
+        const bool srcOut = ((H - k) & 1) == 0;                        // rows of step k; step 0 (zero rows) is never read
+        const double* sP = srcOut ? outP : tmpP;
+        const double* sM = srcOut ? outM : tmpM;
+        const double* sG = srcOut ? outG : tmpG;
+        double* dP = srcOut ? tmpP : outP;
+        double* dM = srcOut ? tmpM : outM;
+        double* dG = srcOut ? tmpG : outG;
+        if (k > 0) outcome_queries(queries, qnode, q, n, S, sP, sM, sG, series + (size_t)(k - 1) * q * 3, sh);
+        for (int it = blockIdx.x; it < items; it += gridDim.x) {
+            const int i = it / sBlocks, s = (it % sBlocks) * CTRL_THREADS + threadIdx.x;
+            const int a = min(max(actions[i], 0), A - 1);
+            __syncthreads();                                           // s_vsel of the previous item has been used
+            for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), n - 1);
+            __syncthreads();
+            if (s >= S) continue;
+            const int32_t* reach = reachK + (size_t)a * S * R;
+            const double* rtoA = rtoK + (size_t)a * O * S * R;
+            const double rb = rbarT[(size_t)a * S + s];
+            const bool skip = skipZero && !(rb == 0.0 && signbit(rb));
+            const bool endA = endAction[a] != 0;
+            double totP = 0.0, totM = 0.0, totG = 0.0;
+            for (int o = 0; o < O; o++) {
+                const size_t rowBase = (size_t)s_vsel[o] * S;
+                const double* rto = rtoA + (size_t)o * S * R;
+                double inP = 0.0, inM = 0.0, inG = 0.0;
+                for (int r = 0; r < R; r++) {
+                    const size_t kk = (size_t)s * R + r;
+                    const double w = rto[kk];
+                    double pp = 0.0, pm = 0.0, pg = 0.0;
+                    if (!(skip && w == 0.0)) {
+                        const int sp = reach[kk];
+                        const bool cont = !endA && endState[sp] == 0;
+                        double xp = 1.0, xm = 0.0, xg = 0.0;
+                        if (cont && k > 0) {
+                            xp = __ldcg(sP + rowBase + sp);
+                            xm = __ldcg(sM + rowBase + sp);
+                            xg = __ldcg(sG + rowBase + sp);
+                        } else if (cont) {
+                            xp = 0.0;
+                        }
+                        pp = __dmul_rn(w, xp);
+                        pm = __dmul_rn(w, xm);
+                        pg = __dmul_rn(w, xg);
+                    }
+                    inP = (r == 0) ? pp : __dadd_rn(inP, pp);
+                    inM = (r == 0) ? pm : __dadd_rn(inM, pm);
+                    inG = (r == 0) ? pg : __dadd_rn(inG, pg);
+                }
+                const double termG = __dmul_rn(gamma, inG);
+                totP = (o == 0) ? inP : __dadd_rn(totP, inP);
+                totM = (o == 0) ? inM : __dadd_rn(totM, inM);
+                totG = (o == 0) ? termG : __dadd_rn(totG, termG);
+            }
+            const size_t e = (size_t)i * S + s;
+            dP[e] = totP;
+            dM[e] = __dadd_rn(1.0, totM);
+            dG[e] = __dadd_rn(rb, totG);
+        }
+        grid.sync();
+    }
+    if (H > 0) outcome_queries(queries, qnode, q, n, S, outP, outM, outG, series + (size_t)(H - 1) * q * 3, sh);
 }
 
 // ---- order[] = tuple indices grouped by action, every group padded with -1 to a multiple of G (so that a block of the grouped
@@ -1211,6 +1332,54 @@ extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n
     PBVI_CUDA(cudaMemcpyAsync(&sweeps, d_sweeps, sizeof(int), cudaMemcpyDeviceToHost, st));
     PBVI_CUDA(cudaStreamSynchronize(st));
     *h_sweeps = sweeps;
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, const uint8_t* d_end_state,
+                                        const uint8_t* d_end_action, double gamma, int steps, const double* d_queries,
+                                        const int32_t* d_query_nodes, int q, double* d_success, double* d_steps, double* d_return,
+                                        double* d_series, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_REQUIRE(d_actions && d_succ && d_end_state && d_end_action && d_success && d_steps && d_return, "NULL pointer argument");
+    PBVI_REQUIRE(n >= 1, "need n >= 1 controller nodes");
+    PBVI_REQUIRE(steps >= 0, "need steps >= 0");
+    PBVI_REQUIRE(q >= 0, "need q >= 0 query pairs");
+    PBVI_REQUIRE(q == 0 || steps == 0 || (d_queries && d_query_nodes && d_series), "NULL pointer argument");   // steps = 0 reads no query
+    const int sBlocks = ceil_div(m->S, CTRL_THREADS);
+    PBVI_REQUIRE((long long)n * sBlocks <= 0x7fffffffLL, "too many controller nodes in one call");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    m->last_launches = 0;
+    const size_t rowBytes = (size_t)n * m->S * sizeof(double);
+    if (steps == 0) {                                                  // zero rows, no series
+        PBVI_CUDA(cudaMemsetAsync(d_success, 0, rowBytes, st));
+        PBVI_CUDA(cudaMemsetAsync(d_steps, 0, rowBytes, st));
+        PBVI_CUDA(cudaMemsetAsync(d_return, 0, rowBytes, st));
+        PBVI_CUDA(cudaStreamSynchronize(st));
+        return PBVI_OK;
+    }
+    const size_t smem = (size_t)m->O * sizeof(int);
+    int perSM = 0;
+    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, controller_outcomes_kernel, CTRL_THREADS, smem));
+    if (perSM < 1) {
+        set_error("pbvi_controller_outcomes: the kernel cannot be resident with %zu bytes of shared memory", smem);
+        return PBVI_ERR_UNSUPPORTED;
+    }
+    // every block must be resident for the grid barrier; more blocks than items (or query pairs) would only add blocks to each barrier
+    const int nBlocks = (int)std::min<long long>((long long)perSM * m->sm_count, std::max<long long>((long long)n * sBlocks, q));
+    PBVI_TAKE(tmpP, double, (size_t)n * m->S);
+    PBVI_TAKE(tmpM, double, (size_t)n * m->S);
+    PBVI_TAKE(tmpG, double, (size_t)n * m->S);
+    const bool skipZero = fabs(gamma) <= 1.79769313486231570e308;   // as pbvi_controller_sweep
+    int S = m->S, R = m->R, O = m->O, A = m->A;
+    void* args[] = {(void*)&n, (void*)&d_actions, (void*)&d_succ, (void*)&d_end_state, (void*)&d_end_action, (void*)&m->reachK,
+                    (void*)&m->rtoK, (void*)&m->rbarT, (void*)&gamma, (void*)&S, (void*)&R, (void*)&O, (void*)&A, (void*)&sBlocks,
+                    (void*)&skipZero, (void*)&steps, (void*)&d_success, (void*)&d_steps, (void*)&d_return, (void*)&tmpP, (void*)&tmpM,
+                    (void*)&tmpG, (void*)&d_queries, (void*)&d_query_nodes, (void*)&q, (void*)&d_series};
+    PBVI_CUDA(cudaLaunchCooperativeKernel((const void*)controller_outcomes_kernel, dim3(nBlocks), dim3(CTRL_THREADS), args, smem, st));
+    m->last_launches++;
+    PBVI_CUDA(cudaStreamSynchronize(st));
     return PBVI_OK;
 }
 

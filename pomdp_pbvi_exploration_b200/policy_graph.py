@@ -6,7 +6,8 @@ Finite-state controllers (policy graphs) extracted from a value function, and th
                   and max_n V_n . b is the value of a policy that can be executed, hence a lower bound on V*(b) at every belief and for
                   every model, whatever the signs of its rewards.  `evaluate` iterates that fixed point on the device (one
                   persistent `pbvi_controller_evaluate` launch) and certifies the returned rows with a residual shift; `improve`
-                  raises that bound by point-based policy iteration on the controller.
+                  raises that bound by point-based policy iteration on the controller.  `outcomes` gives the exact success probability,
+                  expected step count and return of runs that stop at end states, for every start (node, state) at once.
 
 The file formats of `save` / `load` are pomdp-solve's: `.pg` ("id action succ_0 ... succ_{O-1}" per node) and `.alpha` (an action line, a
 values line and a blank line per node).
@@ -89,6 +90,25 @@ def match_tuples(node_of: dict, tuples: np.ndarray) -> tuple:
         elif t not in new:
             new[t] = len(new)
     return in_use, np.asarray(list(new), dtype=np.int64).reshape(-1, tuples.shape[1])
+
+
+class ControllerOutcomes:
+    """
+    What `PolicyGraph.outcomes` returns for q query pairs (belief b_j, start node n_j) and horizon H:
+        start_nodes                                    int64 [q]
+        success, steps, discounted_return              float64 [q]: P(T <= H), E[min(T, H)] and E[sum_{t < min(T, H)} gamma^t r_t] at b_j
+        success_curve, steps_curve, return_curve       float64 [q, H] (NumPy): the same after k = 1..H steps (column k - 1)
+        success_rows, steps_rows, return_rows          CUDA float64 [N, S]: the values at H of a run started in (node, true state)
+    """
+
+    def __init__(self, start_nodes, series: np.ndarray, rows: tuple, gamma: float, max_steps: int):
+        self.start_nodes = np.asarray(start_nodes, dtype=np.int64)
+        self.gamma, self.max_steps = gamma, max_steps
+        curves = np.ascontiguousarray(np.transpose(series, (1, 2, 0)))                       # [q, 3, H]
+        self.success_curve, self.steps_curve, self.return_curve = curves[:, 0], curves[:, 1], curves[:, 2]
+        last = curves[:, :, -1] if max_steps > 0 else np.zeros((len(self.start_nodes), 3))
+        self.success, self.steps, self.discounted_return = last[:, 0].copy(), last[:, 1].copy(), last[:, 2].copy()
+        self.success_rows, self.steps_rows, self.return_rows = rows
 
 
 class PolicyGraph:
@@ -427,6 +447,55 @@ class PolicyGraph:
             node = self.successors[node, o]
             disc *= self.gamma
         return ret
+
+    def outcomes(self, max_steps: int, beliefs=None, start_nodes=None, gamma=None) -> ControllerOutcomes:
+        """
+        Exact outcomes of the controller's runs under the reference's termination rule (`Simulation.run_action`): a run starts in a state
+        s and a node n, each step plays a = a_n, collects Rbar[s, a], draws (o, r) from RTO[s, a, :, :] and moves to reach[s, a, r] and
+        sigma(n, o).  It stops after a step that lands in one of the model's `end_states` or plays one of its `end_actions`; that step's
+        reward counts, nothing after it does, and a run that starts in an end state still takes its first step.  With T the stopping step
+        and H = `max_steps`, returns (`ControllerOutcomes`) P(T <= H), E[min(T, H)] and the discounted return
+        G = E[sum_{t < min(T, H)} gamma^t r_t] at each query pair, the same after every k <= H, and the rows over every (node, state).
+        No sampling: `pbvi_controller_outcomes` runs the H steps of the three recursions over (node, state) in one persistent launch.
+
+        G starts its discount at 1 (gamma^0 on the first reward); the average discounted reward the reference's simulations print starts
+        it at gamma, so it is gamma * G.  With gamma = 1 and a finite H, G is the reference's average total reward.
+
+        Query pairs: the rows of `beliefs` (default: b0) with `start_nodes` (default: the best node at each belief, as `simulate` starts).
+        `gamma` defaults to the gamma of the last `evaluate` and may be anywhere in (0, 1].  Raises ValueError when there is no gamma, gamma
+        is outside (0, 1], max_steps < 0, the graph has no rows and no `start_nodes` are given, or an RTO row does not sum to 1 within
+        1e-9 (as `simulate`); non-finite beliefs are rejected by `belief_rows`.
+        """
+        gamma = self.gamma if gamma is None else gamma
+        if gamma is None:
+            raise ValueError('outcomes needs a gamma: pass one or call evaluate(gamma) first')
+        gamma = float(gamma)
+        if not 0.0 < gamma <= 1.0:
+            raise ValueError('gamma must lie in (0, 1]')
+        if int(max_steps) != max_steps or max_steps < 0:
+            raise ValueError('max_steps must be an integer >= 0')
+        max_steps = int(max_steps)
+        m = self.model
+        rto = np.asarray(m.reachable_transitional_observation_table, dtype=np.float64)
+        if not np.all(np.abs(rto.sum(axis=(2, 3)) - 1.0) <= 1e-9):
+            raise ValueError('outcomes needs RTO rows that sum to 1 (a model with leaking mass has no run distribution)')
+        if start_nodes is None and self.rows is None:
+            raise ValueError('the graph has no rows to choose start nodes by: pass start_nodes or call evaluate(gamma) first')
+        B = belief_rows(m, m.start_probabilities if beliefs is None else beliefs)
+        if start_nodes is None:
+            nodes = self.value(B)[1].cpu().numpy().astype(np.int64)
+        else:
+            nodes = np.asarray(start_nodes, dtype=np.int64).reshape(-1)
+            if nodes.shape != (B.shape[0],):
+                raise ValueError(f'start_nodes must have one node per belief row ({B.shape[0]}), got {nodes.shape[0]}')
+            if nodes.size and (nodes.min() < 0 or nodes.max() >= len(self)):
+                raise ValueError(f'start nodes must lie in [0, {len(self)})')
+        end_state = np.zeros(m.state_count, dtype=np.uint8)
+        end_state[np.asarray(m.end_states, dtype=np.int64)] = 1
+        end_action = np.zeros(m.action_count, dtype=np.uint8)
+        end_action[np.asarray(m.end_actions, dtype=np.int64)] = 1
+        P, M, G, series = m.device.controller_outcomes(self.actions, self.successors, end_state, end_action, gamma, max_steps, B, nodes)
+        return ControllerOutcomes(nodes, series.cpu().numpy(), (P, M, G), gamma, max_steps)
 
     # ---- persistence (pomdp-solve formats) --------------------------------------------------------------------------------
     def save(self, path: str, name: str) -> None:
