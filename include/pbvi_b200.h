@@ -120,6 +120,29 @@ PBVI_API int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_act
                                       const int32_t* d_query_nodes, int q, double* d_success, double* d_steps, double* d_return,
                                       double* d_series, void* stream);
 
+/* Controllers with stochastic successor edges (PolicyGraph with mixtures).  A mixture m is a convex combination of node rows, given as a
+ * CSR table: members d_mix_nodes[k] in [0, n) with weights d_mix_weights[k] for k in [d_mix_offsets[m], d_mix_offsets[m + 1]),
+ * d_mix_offsets [n_mix + 1] non-decreasing from 0 (the caller's contract; member indices are clamped into range).  A successor entry
+ * v in [n, n + n_mix) of d_succ means "mixture v - n"; entries are clamped into [0, n + n_mix).  Each sweep runs in two phases of the
+ * same persistent launch, separated by a grid barrier:
+ *   1. mixture rows  Z_m[s] = mu_0 * X[node_0][s], then Z_m[s] = Z_m[s] + mu_k * X[node_k][s] for the further members in stored order
+ *                    (one rounding per operation, no FMA), X the rows the sweep reads;
+ *   2. the node sweep of the call without mixtures, gathering successor rows from [X; Z].
+ * pbvi_controller_evaluate_mixed: pbvi_controller_evaluate of such a controller (change values over the n node rows).
+ * pbvi_controller_outcomes_mixed: pbvi_controller_outcomes of such a controller, one mixture phase for each of P, M and G (from sweep 1
+ * on: sweep 0 reads no rows).
+ * With n_mix = 0 the mixture pointers may be NULL and both calls are bitwise the calls without mixtures.  Scratch: n_mix (evaluate) or
+ * 3 * n_mix (outcomes) rows of S doubles from the handle's arena.  Both synchronise `stream` once, at the end. */
+PBVI_API int pbvi_controller_evaluate_mixed(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions,
+                                            const int32_t* d_succ, int n_mix, const int32_t* d_mix_offsets, const int32_t* d_mix_nodes,
+                                            const double* d_mix_weights, double tol, int max_sweeps, double* d_out, double* d_changes,
+                                            int* h_sweeps, void* stream);
+PBVI_API int pbvi_controller_outcomes_mixed(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, int n_mix,
+                                            const int32_t* d_mix_offsets, const int32_t* d_mix_nodes, const double* d_mix_weights,
+                                            const uint8_t* d_end_state, const uint8_t* d_end_action, double gamma, int steps,
+                                            const double* d_queries, const int32_t* d_query_nodes, int q, double* d_success,
+                                            double* d_steps, double* d_return, double* d_series, void* stream);
+
 /* pbvi_backup: select + assemble for every belief (no dedup): d_out_alpha [nB][S], d_out_action [nB];
  * d_out_vstar [nB][A][O] and d_out_value [nB][A] may be NULL. */
 PBVI_API int pbvi_backup(pbvi_model* m, const double* d_beliefs, int nB, const double* d_alphas, int nV, double gamma,
@@ -278,6 +301,12 @@ PBVI_API int pbvi_dominating_row(pbvi_model* m, const double* d_rows, int n, int
  * kept undecided}.  Rows must be pairwise distinct.  A row with a non-finite entry is kept (counted with the corners, bound NaN) and
  * never used as a competitor.  Synchronises `stream`. */
 PBVI_API int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts, void* stream);
+/* pbvi_prune_lp_certificates: pbvi_prune_lp (bitwise the same d_keep, d_bound, h_counts and instrumentation) that also returns the
+ * certificate of every pruned row i: d_cert_idx [nV][64] int32 receives its competitor set J (-1 padded) and d_cert_w [nV][64] the
+ * weights lambda >= 0 (summing to 1 up to rounding; 0 padded) of the verified bound u = max_s (alpha_i - sum_q lambda_q alpha_J[q])[s]
+ * < -tol.  Rows that are kept get -1 / 0 throughout.  Synchronises `stream`. */
+PBVI_API int pbvi_prune_lp_certificates(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts,
+                                        int32_t* d_cert_idx, double* d_cert_w, void* stream);
 /* instrumentation of the last pbvi_prune_lp call: h_out4 = {largest competitor set |J| reached, restricted LPs solved, simplex pivots,
  * rows sent to the LP stage} */
 PBVI_API int pbvi_prune_lp_stats(const pbvi_model* m, int64_t* h_out4);

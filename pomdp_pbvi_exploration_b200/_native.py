@@ -32,6 +32,8 @@ SIGNATURES = {
     'pbvi_controller_sweep': [_P, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_controller_evaluate': [_P, _P, c_int, c_double, _P, _P, c_double, c_int, _P, _P, POINTER(c_int), _P],
     'pbvi_controller_outcomes': [_P, c_int, _P, _P, _P, _P, c_double, c_int, _P, _P, c_int, _P, _P, _P, _P, _P],
+    'pbvi_controller_evaluate_mixed': [_P, _P, c_int, c_double, _P, _P, c_int, _P, _P, _P, c_double, c_int, _P, _P, POINTER(c_int), _P],
+    'pbvi_controller_outcomes_mixed': [_P, c_int, _P, _P, c_int, _P, _P, _P, _P, _P, c_double, c_int, _P, _P, c_int, _P, _P, _P, _P, _P],
     'pbvi_backup': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P],
     'pbvi_backup_host': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P],
     'pbvi_backup_host_unique': [_P, _P, c_int, _P, c_int, c_double, _P, c_int, _P, POINTER(c_int), _P],
@@ -58,6 +60,7 @@ SIGNATURES = {
     'pbvi_first_dominating_row': [_P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_dominating_row': [_P, _P, c_int, _P, _P],
     'pbvi_prune_lp': [_P, _P, c_int, _P, _P, _P, _P],
+    'pbvi_prune_lp_certificates': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_prune_lp_stats': [_P, _P],
     'pbvi_sawtooth': [_P, _P, _P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_support_lists': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
@@ -264,6 +267,50 @@ class DeviceModel:
         self._call(self._lib.pbvi_controller_outcomes(self._h, n, _ptr(act), _ptr(sc), _ptr(es), _ptr(ea), float(gamma), int(steps), _ptr(b),
                                                       _ptr(qn), q, _ptr(P), _ptr(M), _ptr(G), _ptr(series), self._stream))
         return P, M, G, series
+
+    def _mixtures(self, mixtures):
+        off, nodes, w = mixtures
+        off, nodes, w = _i32(off, self.device).reshape(-1), _i32(nodes, self.device).reshape(-1), _f64(w, self.device).reshape(-1)
+        assert off.shape[0] >= 1 and nodes.shape == w.shape
+        return off.shape[0] - 1, off, nodes, w
+
+    def controller_evaluate_mixed(self, rows, gamma: float, actions, succ, mixtures, tol: float, max_sweeps: int):
+        """`controller_evaluate` of a controller with mixtures (`pbvi_controller_evaluate_mixed`): `mixtures` = (offsets [M+1], member
+        nodes [nnz], weights [nnz]); a successor entry v >= n means mixture v - n.  Returns (last iterate [n,S], per-sweep max |out - in|
+        over the n node rows [k] CUDA float64, k).  Synchronises."""
+        W = self._beliefs(rows)
+        act, sc = _i32(actions, self.device), _i32(succ, self.device)
+        n = W.shape[0]
+        assert act.shape == (n,) and sc.shape == (n, self.O)
+        M, off, nodes, w = self._mixtures(mixtures)
+        out = torch.empty((n, self.S), dtype=torch.float64, device=self.device)
+        changes = torch.empty((max(int(max_sweeps), 1),), dtype=torch.float64, device=self.device)
+        k = c_int(0)
+        self._call(self._lib.pbvi_controller_evaluate_mixed(self._h, _ptr(W), n, float(gamma), _ptr(act), _ptr(sc), M, _ptr(off), _ptr(nodes),
+                                                            _ptr(w), float(tol), int(max_sweeps), _ptr(out), _ptr(changes), byref(k),
+                                                            self._stream))
+        return out, changes[:k.value], k.value
+
+    def controller_outcomes_mixed(self, actions, succ, mixtures, end_state, end_action, gamma: float, steps: int, queries, query_nodes):
+        """`controller_outcomes` of a controller with mixtures (`pbvi_controller_outcomes_mixed`; `mixtures` as for
+        `controller_evaluate_mixed`).  Synchronises."""
+        act, sc = _i32(actions, self.device), _i32(succ, self.device)
+        n = act.shape[0]
+        assert sc.shape == (n, self.O)
+        M, off, nodes, w = self._mixtures(mixtures)
+        es = torch.as_tensor(np.asarray(end_state) != 0, device=self.device).to(torch.uint8).contiguous()
+        ea = torch.as_tensor(np.asarray(end_action) != 0, device=self.device).to(torch.uint8).contiguous()
+        assert es.shape == (self.S,) and ea.shape == (self.A,)
+        b = self._beliefs(queries)
+        qn = _i32(query_nodes, self.device).reshape(-1)
+        q = b.shape[0]
+        assert qn.shape == (q,)
+        P, Mr, G = (torch.empty((n, self.S), dtype=torch.float64, device=self.device) for _ in range(3))
+        series = torch.empty((int(steps), q, 3), dtype=torch.float64, device=self.device)
+        self._call(self._lib.pbvi_controller_outcomes_mixed(self._h, n, _ptr(act), _ptr(sc), M, _ptr(off), _ptr(nodes), _ptr(w), _ptr(es),
+                                                            _ptr(ea), float(gamma), int(steps), _ptr(b), _ptr(qn), q, _ptr(P), _ptr(Mr), _ptr(G),
+                                                            _ptr(series), self._stream))
+        return P, Mr, G, series
 
     def first_dominating_row(self, new_rows, old_rows) -> torch.Tensor:
         """For every row of `old_rows`, the first row of `new_rows` that is >= it at every state, or -1 (`pbvi_first_dominating_row`):
@@ -589,6 +636,21 @@ class DeviceModel:
         counts = np.zeros(4, dtype=np.int32)
         self._call(self._lib.pbvi_prune_lp(self._h, _ptr(al), n, _ptr(keep), _ptr(bound), counts.ctypes.data, self._stream))
         return keep, bound, counts.astype(np.int64)
+
+    def prune_lp_certificates(self, alphas):
+        """`prune_lp` that also returns the certificate of every pruned row (`pbvi_prune_lp_certificates`): (keep, bound, counts, idx
+        [n, 64] int32, weights [n, 64] float64), idx / weights the competitor set J (-1 padded) and the lambda of the verified bound u
+        (0 padded); -1 / 0 throughout for a kept row.  Synchronises."""
+        al = self._beliefs(alphas)
+        n = al.shape[0]
+        keep = torch.empty((n,), dtype=torch.int32, device=self.device)
+        bound = torch.empty((n,), dtype=torch.float64, device=self.device)
+        idx = torch.empty((n, 64), dtype=torch.int32, device=self.device)
+        w = torch.empty((n, 64), dtype=torch.float64, device=self.device)
+        counts = np.zeros(4, dtype=np.int32)
+        self._call(self._lib.pbvi_prune_lp_certificates(self._h, _ptr(al), n, _ptr(keep), _ptr(bound), counts.ctypes.data, _ptr(idx), _ptr(w),
+                                                        self._stream))
+        return keep, bound, counts.astype(np.int64), idx, w
 
     def prune_lp_stats(self) -> dict:
         """Work of the last `prune_lp` call: largest competitor set, restricted LPs, simplex pivots, rows that reached the LP stage."""

@@ -22,6 +22,9 @@
 // pbvi_controller_outcomes:
 //   controller_outcomes_kernel   persistent cooperative launch: H sweeps of the success / step / return recursions of a controller that
 //                                stops at end states, plus b . row of query pairs after every sweep
+// pbvi_controller_evaluate_mixed / pbvi_controller_outcomes_mixed:
+//   the same two kernels with kMix: every sweep first forms the mixture rows (convex combinations of node rows that a successor entry
+//   >= n stands for), then, after a grid barrier, runs the node sweep against [W; Z]
 #include <algorithm>
 #include <thread>
 
@@ -266,15 +269,17 @@ __device__ __forceinline__ double block_sum_256(double v, double* sh) {
 // the olfactory model) are never issued.
 // Coherent: the alpha rows were written earlier in the same launch (controller_evaluate_kernel), so they are gathered with ld.global.cg
 // instead of through the read-only data cache, which is not kept coherent with writes during a launch.
-template <bool Coherent = false>
+// Mixed: a selection v >= nRows names row v - nRows of `mixRows` (the mixture rows of controller_evaluate_kernel<true>).
+template <bool Coherent = false, bool Mixed = false>
 __device__ __forceinline__ double alpha_a_entry(const double* __restrict__ alphas, int S, int R, int O, const int* vsel,
                                                 const int32_t* __restrict__ reach, const double* __restrict__ rtoA,
-                                                const double* __restrict__ rbarA, double gamma, int s, bool skipZero) {
+                                                const double* __restrict__ rbarA, double gamma, int s, bool skipZero,
+                                                const double* mixRows = nullptr, int nRows = 0) {
     const double rb = rbarA[s];
     const bool skip = skipZero && !(rb == 0.0 && signbit(rb));
     double tot = 0.0;
     for (int o = 0; o < O; o++) {
-        const double* arow = alphas + (size_t)vsel[o] * S;
+        const double* arow = (Mixed && vsel[o] >= nRows) ? mixRows + (size_t)(vsel[o] - nRows) * S : alphas + (size_t)vsel[o] * S;
         const double* rto = rtoA + (size_t)o * S * R;
         double inner = 0.0;
         for (int r = 0; r < R; r++) {
@@ -562,33 +567,61 @@ __device__ __forceinline__ double ctrl_reduce_max(double v, bool nan, double* sh
     return n ? NAN : v;
 }
 
+// Mixture m of a controller with mixtures: member nodes mixNodes[mixOff[m] .. mixOff[m + 1]) with weights mixW, in stored order.
+// z = mu_0 * x_0, then z = z + mu_k * x_k: one rounding per operation, no FMA, so that NumPy restates it bitwise.  Member indices are
+// clamped into [0, n); the rows x were written earlier in the same launch (ld.global.cg).
+__device__ __forceinline__ double mixture_entry(const double* rows, int n, int S, int s, int lo, int hi, const int32_t* __restrict__ mixNodes,
+                                                const double* __restrict__ mixW) {
+    double z = 0.0;
+    for (int k = lo; k < hi; k++) {
+        const double t = __dmul_rn(mixW[k], __ldcg(rows + (size_t)min(max(mixNodes[k], 0), n - 1) * S + s));
+        z = (k == lo) ? t : __dadd_rn(z, t);
+    }
+    return z;
+}
+
+// kMix (pbvi_controller_evaluate_mixed): each sweep first writes the nMix mixture rows of its source rows into Z [nMix][S] (items
+// (mixture, 256 states) strided over the grid), then passes a grid barrier, and only then runs the node sweep, in which a successor
+// entry v in [n, n + nMix) reads row v - n of Z.  Z is rewritten only in the next sweep, after the barrier that ends this one.  The
+// change values are over the n node rows as without mixtures; with kMix = false the kernel is the one without mixtures.
+template <bool kMix>
 __global__ void __launch_bounds__(CTRL_THREADS) controller_evaluate_kernel(const double* __restrict__ in0, int n, const int32_t* __restrict__ actions,
                                                                            const int32_t* __restrict__ succ, const int32_t* __restrict__ reachK,
                                                                            const double* __restrict__ rtoK, const double* __restrict__ rbarT,
                                                                            double gamma, int S, int R, int O, int A, int sBlocks, bool skipZero,
                                                                            double tol, int maxSweeps, double* bufA, double* bufB, double* part,
-                                                                           double* __restrict__ changes, int* __restrict__ sweepsOut) {
+                                                                           double* __restrict__ changes, int* __restrict__ sweepsOut, int nMix,
+                                                                           const int32_t* __restrict__ mixOff, const int32_t* __restrict__ mixNodes,
+                                                                           const double* __restrict__ mixW, double* Z) {
     extern __shared__ int s_vsel[];
     __shared__ double sh[CTRL_THREADS / 32];
     __shared__ int shn[CTRL_THREADS / 32];
     cg::grid_group grid = cg::this_grid();
     const int items = n * sBlocks;
+    const int nSel = kMix ? n + nMix : n;                              // successor entries are clamped into [0, nSel)
     int k = 0;
     for (;; k++) {
         // rows written earlier in this launch are read with ld.global.cg, never through the read-only data cache
         const double* src = (k == 0) ? in0 : ((k & 1) ? bufA : bufB);
         double* dst = (k & 1) ? bufB : bufA;
+        if (kMix) {
+            for (int it = blockIdx.x; it < nMix * sBlocks; it += gridDim.x) {
+                const int mx = it / sBlocks, s = (it % sBlocks) * CTRL_THREADS + threadIdx.x;
+                if (s < S) Z[(size_t)mx * S + s] = mixture_entry(src, n, S, s, mixOff[mx], mixOff[mx + 1], mixNodes, mixW);
+            }
+            grid.sync();
+        }
         double amax = 0.0;
         bool nan = false;
         for (int it = blockIdx.x; it < items; it += gridDim.x) {
             const int i = it / sBlocks, s = (it % sBlocks) * CTRL_THREADS + threadIdx.x;
             const int a = min(max(actions[i], 0), A - 1);
             __syncthreads();                                           // s_vsel of the previous item has been used
-            for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), n - 1);
+            for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), nSel - 1);
             __syncthreads();
             if (s < S) {
-                const double v = alpha_a_entry<true>(src, S, R, O, s_vsel, reachK + (size_t)a * S * R, rtoK + (size_t)a * O * S * R,
-                                                     rbarT + (size_t)a * S, gamma, s, skipZero);
+                const double v = alpha_a_entry<true, kMix>(src, S, R, O, s_vsel, reachK + (size_t)a * S * R, rtoK + (size_t)a * O * S * R,
+                                                           rbarT + (size_t)a * S, gamma, s, skipZero, Z, n);
                 dst[(size_t)i * S + s] = v;
                 const double d = __dadd_rn(v, -__ldcg(src + (size_t)i * S + s));
                 nan |= d != d;
@@ -659,17 +692,25 @@ __device__ __forceinline__ void outcome_queries(const double* __restrict__ queri
     }
 }
 
+// kMix (pbvi_controller_outcomes_mixed): sweep k > 0 first writes the mixture rows of P, M and G of step k into ZP / ZM / ZG [nMix][S]
+// (mixture_entry, one pass for the three), passes a grid barrier, and then runs as without mixtures, a successor entry v in
+// [n, n + nMix) reading row v - n of the Z rows.  Sweep 0 gathers nothing and forms no mixture rows.
+template <bool kMix>
 __global__ void __launch_bounds__(CTRL_THREADS) controller_outcomes_kernel(int n, const int32_t* __restrict__ actions, const int32_t* __restrict__ succ,
                                                                            const uint8_t* __restrict__ endState, const uint8_t* __restrict__ endAction,
                                                                            const int32_t* __restrict__ reachK, const double* __restrict__ rtoK,
                                                                            const double* __restrict__ rbarT, double gamma, int S, int R, int O, int A,
                                                                            int sBlocks, bool skipZero, int H, double* outP, double* outM, double* outG,
                                                                            double* tmpP, double* tmpM, double* tmpG, const double* __restrict__ queries,
-                                                                           const int32_t* __restrict__ qnode, int q, double* __restrict__ series) {
+                                                                           const int32_t* __restrict__ qnode, int q, double* __restrict__ series,
+                                                                           int nMix, const int32_t* __restrict__ mixOff,
+                                                                           const int32_t* __restrict__ mixNodes, const double* __restrict__ mixW,
+                                                                           double* ZP, double* ZM, double* ZG) {
     extern __shared__ int s_vsel[];
     __shared__ double sh[CTRL_THREADS / 32];
     cg::grid_group grid = cg::this_grid();
     const int items = n * sBlocks;
+    const int nSel = kMix ? n + nMix : n;                              // successor entries are clamped into [0, nSel)
     for (int k = 0; k < H; k++) {
         // rows written earlier in this launch are read with ld.global.cg, never through the read-only data cache
         const bool srcOut = ((H - k) & 1) == 0;                        // rows of step k; step 0 (zero rows) is never read
@@ -679,12 +720,24 @@ __global__ void __launch_bounds__(CTRL_THREADS) controller_outcomes_kernel(int n
         double* dP = srcOut ? tmpP : outP;
         double* dM = srcOut ? tmpM : outM;
         double* dG = srcOut ? tmpG : outG;
+        if (kMix && k > 0) {
+            for (int it = blockIdx.x; it < nMix * sBlocks; it += gridDim.x) {
+                const int mx = it / sBlocks, s = (it % sBlocks) * CTRL_THREADS + threadIdx.x;
+                if (s >= S) continue;
+                const int lo = mixOff[mx], hi = mixOff[mx + 1];
+                const size_t e = (size_t)mx * S + s;
+                ZP[e] = mixture_entry(sP, n, S, s, lo, hi, mixNodes, mixW);
+                ZM[e] = mixture_entry(sM, n, S, s, lo, hi, mixNodes, mixW);
+                ZG[e] = mixture_entry(sG, n, S, s, lo, hi, mixNodes, mixW);
+            }
+            grid.sync();
+        }
         if (k > 0) outcome_queries(queries, qnode, q, n, S, sP, sM, sG, series + (size_t)(k - 1) * q * 3, sh);
         for (int it = blockIdx.x; it < items; it += gridDim.x) {
             const int i = it / sBlocks, s = (it % sBlocks) * CTRL_THREADS + threadIdx.x;
             const int a = min(max(actions[i], 0), A - 1);
             __syncthreads();                                           // s_vsel of the previous item has been used
-            for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), n - 1);
+            for (int o = threadIdx.x; o < O; o += CTRL_THREADS) s_vsel[o] = min(max(succ[(size_t)i * O + o], 0), nSel - 1);
             __syncthreads();
             if (s >= S) continue;
             const int32_t* reach = reachK + (size_t)a * S * R;
@@ -694,7 +747,11 @@ __global__ void __launch_bounds__(CTRL_THREADS) controller_outcomes_kernel(int n
             const bool endA = endAction[a] != 0;
             double totP = 0.0, totM = 0.0, totG = 0.0;
             for (int o = 0; o < O; o++) {
-                const size_t rowBase = (size_t)s_vsel[o] * S;
+                const bool fromZ = kMix && s_vsel[o] >= n;
+                const size_t rowBase = (size_t)(fromZ ? s_vsel[o] - n : s_vsel[o]) * S;
+                const double* gP = fromZ ? ZP : sP;
+                const double* gM = fromZ ? ZM : sM;
+                const double* gG = fromZ ? ZG : sG;
                 const double* rto = rtoA + (size_t)o * S * R;
                 double inP = 0.0, inM = 0.0, inG = 0.0;
                 for (int r = 0; r < R; r++) {
@@ -706,9 +763,9 @@ __global__ void __launch_bounds__(CTRL_THREADS) controller_outcomes_kernel(int n
                         const bool cont = !endA && endState[sp] == 0;
                         double xp = 1.0, xm = 0.0, xg = 0.0;
                         if (cont && k > 0) {
-                            xp = __ldcg(sP + rowBase + sp);
-                            xm = __ldcg(sM + rowBase + sp);
-                            xg = __ldcg(sG + rowBase + sp);
+                            xp = __ldcg(gP + rowBase + sp);
+                            xm = __ldcg(gM + rowBase + sp);
+                            xg = __ldcg(gG + rowBase + sp);
                         } else if (cont) {
                             xp = 0.0;
                         }
@@ -1295,8 +1352,18 @@ extern "C" int pbvi_controller_sweep(pbvi_model* m, const double* d_in, int n, d
     return PBVI_OK;
 }
 
-extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions, const int32_t* d_succ,
-                                        double tol, int max_sweeps, double* d_out, double* d_changes, int* h_sweeps, void* stream) {
+// the mixture table of a controller with mixtures (pbvi_controller_*_mixed): n_mix = 0 is a controller without them
+static int check_mixtures(int n_mix, const int32_t* d_mix_offsets, const int32_t* d_mix_nodes, const double* d_mix_weights, int S) {
+    PBVI_REQUIRE(n_mix >= 0, "need n_mix >= 0 mixtures");
+    PBVI_REQUIRE(n_mix == 0 || (d_mix_offsets && d_mix_nodes && d_mix_weights), "NULL pointer argument");
+    PBVI_REQUIRE((long long)n_mix * ceil_div(S, CTRL_THREADS) <= 0x7fffffffLL, "too many mixtures in one call");
+    return PBVI_OK;
+}
+
+template <bool kMix>
+static int controller_evaluate_impl(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions, const int32_t* d_succ,
+                                    int n_mix, const int32_t* d_mix_offsets, const int32_t* d_mix_nodes, const double* d_mix_weights,
+                                    double tol, int max_sweeps, double* d_out, double* d_changes, int* h_sweeps, void* stream) {
     PBVI_REQUIRE(d_in && d_actions && d_succ && d_out && h_sweeps, "NULL pointer argument");
     PBVI_REQUIRE(n >= 1, "need n >= 1 controller nodes");
     PBVI_REQUIRE(max_sweeps >= 1, "need max_sweeps >= 1");
@@ -1311,7 +1378,7 @@ extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n
     m->last_launches = 0;
     const size_t smem = (size_t)m->O * sizeof(int);
     int perSM = 0;
-    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, controller_evaluate_kernel, CTRL_THREADS, smem));
+    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, controller_evaluate_kernel<kMix>, CTRL_THREADS, smem));
     if (perSM < 1) {
         set_error("pbvi_controller_evaluate: the kernel cannot be resident with %zu bytes of shared memory", smem);
         return PBVI_ERR_UNSUPPORTED;
@@ -1321,12 +1388,18 @@ extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n
     PBVI_TAKE(bufB, double, (size_t)n * m->S);
     PBVI_TAKE(part, double, (size_t)2 * nBlocks);
     PBVI_TAKE(d_sweeps, int, 1);
+    double* Z = nullptr;
+    if (kMix) {
+        PBVI_TAKE(zrows, double, (size_t)n_mix * m->S);
+        Z = zrows;
+    }
     const bool skipZero = fabs(gamma) <= 1.79769313486231570e308;   // as pbvi_controller_sweep
     int S = m->S, R = m->R, O = m->O, A = m->A;
     void* args[] = {(void*)&d_in, (void*)&n, (void*)&d_actions, (void*)&d_succ, (void*)&m->reachK, (void*)&m->rtoK, (void*)&m->rbarT,
                     (void*)&gamma, (void*)&S, (void*)&R, (void*)&O, (void*)&A, (void*)&sBlocks, (void*)&skipZero, (void*)&tol,
-                    (void*)&max_sweeps, (void*)&d_out, (void*)&bufB, (void*)&part, (void*)&d_changes, (void*)&d_sweeps};
-    PBVI_CUDA(cudaLaunchCooperativeKernel((const void*)controller_evaluate_kernel, dim3(nBlocks), dim3(CTRL_THREADS), args, smem, st));
+                    (void*)&max_sweeps, (void*)&d_out, (void*)&bufB, (void*)&part, (void*)&d_changes, (void*)&d_sweeps, (void*)&n_mix,
+                    (void*)&d_mix_offsets, (void*)&d_mix_nodes, (void*)&d_mix_weights, (void*)&Z};
+    PBVI_CUDA(cudaLaunchCooperativeKernel((const void*)controller_evaluate_kernel<kMix>, dim3(nBlocks), dim3(CTRL_THREADS), args, smem, st));
     m->last_launches++;
     int sweeps = 0;
     PBVI_CUDA(cudaMemcpyAsync(&sweeps, d_sweeps, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -1335,10 +1408,31 @@ extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n
     return PBVI_OK;
 }
 
-extern "C" int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, const uint8_t* d_end_state,
-                                        const uint8_t* d_end_action, double gamma, int steps, const double* d_queries,
-                                        const int32_t* d_query_nodes, int q, double* d_success, double* d_steps, double* d_return,
-                                        double* d_series, void* stream) {
+extern "C" int pbvi_controller_evaluate(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions, const int32_t* d_succ,
+                                        double tol, int max_sweeps, double* d_out, double* d_changes, int* h_sweeps, void* stream) {
+    return controller_evaluate_impl<false>(m, d_in, n, gamma, d_actions, d_succ, 0, nullptr, nullptr, nullptr, tol, max_sweeps, d_out,
+                                           d_changes, h_sweeps, stream);
+}
+
+extern "C" int pbvi_controller_evaluate_mixed(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions,
+                                              const int32_t* d_succ, int n_mix, const int32_t* d_mix_offsets, const int32_t* d_mix_nodes,
+                                              const double* d_mix_weights, double tol, int max_sweeps, double* d_out, double* d_changes,
+                                              int* h_sweeps, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_TRY(check_mixtures(n_mix, d_mix_offsets, d_mix_nodes, d_mix_weights, m->S));
+    if (n_mix == 0)
+        return controller_evaluate_impl<false>(m, d_in, n, gamma, d_actions, d_succ, 0, nullptr, nullptr, nullptr, tol, max_sweeps, d_out,
+                                               d_changes, h_sweeps, stream);
+    return controller_evaluate_impl<true>(m, d_in, n, gamma, d_actions, d_succ, n_mix, d_mix_offsets, d_mix_nodes, d_mix_weights, tol,
+                                          max_sweeps, d_out, d_changes, h_sweeps, stream);
+}
+
+template <bool kMix>
+static int controller_outcomes_impl(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, int n_mix,
+                                    const int32_t* d_mix_offsets, const int32_t* d_mix_nodes, const double* d_mix_weights,
+                                    const uint8_t* d_end_state, const uint8_t* d_end_action, double gamma, int steps, const double* d_queries,
+                                    const int32_t* d_query_nodes, int q, double* d_success, double* d_steps, double* d_return,
+                                    double* d_series, void* stream) {
     PBVI_REQUIRE(m != nullptr, "model handle is NULL");
     PBVI_REQUIRE(d_actions && d_succ && d_end_state && d_end_action && d_success && d_steps && d_return, "NULL pointer argument");
     PBVI_REQUIRE(n >= 1, "need n >= 1 controller nodes");
@@ -1361,7 +1455,7 @@ extern "C" int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_a
     }
     const size_t smem = (size_t)m->O * sizeof(int);
     int perSM = 0;
-    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, controller_outcomes_kernel, CTRL_THREADS, smem));
+    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, controller_outcomes_kernel<kMix>, CTRL_THREADS, smem));
     if (perSM < 1) {
         set_error("pbvi_controller_outcomes: the kernel cannot be resident with %zu bytes of shared memory", smem);
         return PBVI_ERR_UNSUPPORTED;
@@ -1371,16 +1465,47 @@ extern "C" int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_a
     PBVI_TAKE(tmpP, double, (size_t)n * m->S);
     PBVI_TAKE(tmpM, double, (size_t)n * m->S);
     PBVI_TAKE(tmpG, double, (size_t)n * m->S);
+    double *ZP = nullptr, *ZM = nullptr, *ZG = nullptr;
+    if (kMix) {
+        PBVI_TAKE(zrows, double, (size_t)3 * n_mix * m->S);
+        ZP = zrows;
+        ZM = zrows + (size_t)n_mix * m->S;
+        ZG = zrows + (size_t)2 * n_mix * m->S;
+    }
     const bool skipZero = fabs(gamma) <= 1.79769313486231570e308;   // as pbvi_controller_sweep
     int S = m->S, R = m->R, O = m->O, A = m->A;
     void* args[] = {(void*)&n, (void*)&d_actions, (void*)&d_succ, (void*)&d_end_state, (void*)&d_end_action, (void*)&m->reachK,
                     (void*)&m->rtoK, (void*)&m->rbarT, (void*)&gamma, (void*)&S, (void*)&R, (void*)&O, (void*)&A, (void*)&sBlocks,
                     (void*)&skipZero, (void*)&steps, (void*)&d_success, (void*)&d_steps, (void*)&d_return, (void*)&tmpP, (void*)&tmpM,
-                    (void*)&tmpG, (void*)&d_queries, (void*)&d_query_nodes, (void*)&q, (void*)&d_series};
-    PBVI_CUDA(cudaLaunchCooperativeKernel((const void*)controller_outcomes_kernel, dim3(nBlocks), dim3(CTRL_THREADS), args, smem, st));
+                    (void*)&tmpG, (void*)&d_queries, (void*)&d_query_nodes, (void*)&q, (void*)&d_series, (void*)&n_mix,
+                    (void*)&d_mix_offsets, (void*)&d_mix_nodes, (void*)&d_mix_weights, (void*)&ZP, (void*)&ZM, (void*)&ZG};
+    PBVI_CUDA(cudaLaunchCooperativeKernel((const void*)controller_outcomes_kernel<kMix>, dim3(nBlocks), dim3(CTRL_THREADS), args, smem, st));
     m->last_launches++;
     PBVI_CUDA(cudaStreamSynchronize(st));
     return PBVI_OK;
+}
+
+extern "C" int pbvi_controller_outcomes(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, const uint8_t* d_end_state,
+                                        const uint8_t* d_end_action, double gamma, int steps, const double* d_queries,
+                                        const int32_t* d_query_nodes, int q, double* d_success, double* d_steps, double* d_return,
+                                        double* d_series, void* stream) {
+    return controller_outcomes_impl<false>(m, n, d_actions, d_succ, 0, nullptr, nullptr, nullptr, d_end_state, d_end_action, gamma, steps,
+                                           d_queries, d_query_nodes, q, d_success, d_steps, d_return, d_series, stream);
+}
+
+extern "C" int pbvi_controller_outcomes_mixed(pbvi_model* m, int n, const int32_t* d_actions, const int32_t* d_succ, int n_mix,
+                                              const int32_t* d_mix_offsets, const int32_t* d_mix_nodes, const double* d_mix_weights,
+                                              const uint8_t* d_end_state, const uint8_t* d_end_action, double gamma, int steps,
+                                              const double* d_queries, const int32_t* d_query_nodes, int q, double* d_success,
+                                              double* d_steps, double* d_return, double* d_series, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_TRY(check_mixtures(n_mix, d_mix_offsets, d_mix_nodes, d_mix_weights, m->S));
+    if (n_mix == 0)
+        return controller_outcomes_impl<false>(m, n, d_actions, d_succ, 0, nullptr, nullptr, nullptr, d_end_state, d_end_action, gamma, steps,
+                                               d_queries, d_query_nodes, q, d_success, d_steps, d_return, d_series, stream);
+    return controller_outcomes_impl<true>(m, n, d_actions, d_succ, n_mix, d_mix_offsets, d_mix_nodes, d_mix_weights, d_end_state,
+                                          d_end_action, gamma, steps, d_queries, d_query_nodes, q, d_success, d_steps, d_return, d_series,
+                                          stream);
 }
 
 extern "C" int pbvi_backup(pbvi_model* m, const double* d_beliefs, int nB, const double* d_alphas, int nV, double gamma,

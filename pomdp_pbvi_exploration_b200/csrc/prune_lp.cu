@@ -159,11 +159,21 @@ __global__ void __launch_bounds__(PL_THREADS) prune_lp_corner_kernel(const doubl
 // Variables: b_s -> id s, t_q -> id S + q, delta -> id S + J_MAX.  delta is basic from the start (at the position of the tightest
 // competitor of the seed corner) and, being free, never leaves.  Duals y = row pos(delta) of the basis inverse; at the optimum
 // lambda_q = -y_q >= 0 sums to 1 and max_s sum_q lambda_q d_q[s] = delta_J.
+// kCert (pbvi_prune_lp_certificates): a pruned row also leaves its certificate, the competitor set J in certIdx[i][0..k) and the weights
+// lambda behind the verified bound u in certW[i][0..k) (the rest of the row is left as the caller initialised it).  Nothing else changes.
+// The two outputs come as the parameter pack `cert` = (certIdx, certW), empty without kCert: the kernel of pbvi_prune_lp keeps its
+// exact parameter list, and with it its code.
+__device__ __forceinline__ void write_certificate(int32_t* certIdx, double* certW, int i, int q, int j, double lambda) {
+    certIdx[(size_t)i * J_MAX + q] = j;
+    certW[(size_t)i * J_MAX + q] = lambda;
+}
+
+template <bool kCert, typename... Cert>
 __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* __restrict__ A, int n, int S, const int32_t* __restrict__ finite,
                                                               const double* __restrict__ tauP, const int32_t* __restrict__ cornerS,
                                                               const int32_t* __restrict__ cornerJ, int32_t* __restrict__ keep,
                                                               double* __restrict__ bound, int* __restrict__ queue, int* __restrict__ counts,
-                                                              unsigned long long* __restrict__ stats) {
+                                                              unsigned long long* __restrict__ stats, Cert... cert) {
     __shared__ double Binv[M_MAX][M_MAX];
     __shared__ double xB[M_MAX], wv[M_MAX], col[M_MAX], prow[M_MAX], lam[J_MAX], suppB[M_MAX];
     __shared__ int basis[M_MAX], J[J_MAX], suppS[M_MAX];
@@ -354,6 +364,9 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
             k++;
             __syncthreads();
         }
+        if constexpr (kCert) {
+            if (verdict == 0 && tid < k) write_certificate(cert..., i, tid, J[tid], lam[tid]);   // J and lambda of the LP that gave u
+        }
         if (tid == 0) {
             keep[i] = verdict == 0 ? 0 : 1;
             bound[i] = bnd;
@@ -370,7 +383,9 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
 
 using namespace pbvi;
 
-extern "C" int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts, void* stream) {
+template <bool kCert>
+static int prune_lp_impl(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts,
+                         int32_t* d_cert_idx, double* d_cert_w, void* stream) {
     PBVI_REQUIRE(nV >= 0, "nV must be non-negative");
     PBVI_REQUIRE(m != nullptr, "model handle is NULL");
     if (h_counts) std::fill(h_counts, h_counts + 4, 0);
@@ -378,6 +393,7 @@ extern "C" int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int3
     std::fill(m->prune_lp_stats, m->prune_lp_stats + 4, 0ll);
     if (nV == 0) return PBVI_OK;
     PBVI_REQUIRE(d_alphas && d_keep, "NULL pointer argument");
+    PBVI_REQUIRE(!kCert || (d_cert_idx && d_cert_w), "NULL pointer argument");
     PBVI_CUDA(cudaSetDevice(m->device));
     cudaStream_t st = (cudaStream_t)stream;
     PBVI_TRY(enter_call(m, st));
@@ -400,14 +416,26 @@ extern "C" int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int3
     }
     PBVI_CUDA(cudaMemsetAsync(counters, 0, 8 * sizeof(int), st));
     PBVI_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), st));
+    if (kCert) {
+        PBVI_CUDA(cudaMemsetAsync(d_cert_idx, 0xff, (size_t)n * J_MAX * sizeof(int32_t), st));   // -1
+        PBVI_CUDA(cudaMemsetAsync(d_cert_w, 0, (size_t)n * J_MAX * sizeof(double), st));
+    }
     prune_lp_row_stats_kernel<<<n, PL_THREADS, 0, st>>>(d_alphas, S, finite, rowMax);
     prune_lp_tau_kernel<<<1, PL_THREADS, 0, st>>>(rowMax, n, tau);
     prune_lp_columns_kernel<<<ceil_div(S, PL_THREADS), PL_THREADS, 0, st>>>(d_alphas, n, S, finite, v1, i1, v2, i2);
     prune_lp_corner_kernel<<<n, PL_THREADS, 0, st>>>(d_alphas, S, finite, tau, v1, i1, v2, i2, cornerS, cornerJ, d_keep, bound, counters + 1);
     int perSM = 1;
-    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, prune_lp_kernel, PL_THREADS, 0));
-    const int grid = std::max(1, std::min(n, m->sm_count * std::max(perSM, 1)));
-    prune_lp_kernel<<<grid, PL_THREADS, 0, st>>>(d_alphas, n, S, finite, tau, cornerS, cornerJ, d_keep, bound, counters, counters + 1, stats);
+    if constexpr (kCert) {
+        PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, prune_lp_kernel<true, int32_t*, double*>, PL_THREADS, 0));
+        const int grid = std::max(1, std::min(n, m->sm_count * std::max(perSM, 1)));
+        prune_lp_kernel<true><<<grid, PL_THREADS, 0, st>>>(d_alphas, n, S, finite, tau, cornerS, cornerJ, d_keep, bound, counters, counters + 1,
+                                                           stats, d_cert_idx, d_cert_w);
+    } else {
+        PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, prune_lp_kernel<false>, PL_THREADS, 0));
+        const int grid = std::max(1, std::min(n, m->sm_count * std::max(perSM, 1)));
+        prune_lp_kernel<false><<<grid, PL_THREADS, 0, st>>>(d_alphas, n, S, finite, tau, cornerS, cornerJ, d_keep, bound, counters, counters + 1,
+                                                            stats);
+    }
     m->last_launches = 5;
     PBVI_CUDA(cudaGetLastError());
     int32_t c[8];
@@ -418,6 +446,15 @@ extern "C" int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int3
     if (h_counts) std::copy(c + 1, c + 5, h_counts);
     for (int k = 0; k < 4; k++) m->prune_lp_stats[k] = (long long)sv[k];
     return PBVI_OK;
+}
+
+extern "C" int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts, void* stream) {
+    return prune_lp_impl<false>(m, d_alphas, nV, d_keep, d_bound, h_counts, nullptr, nullptr, stream);
+}
+
+extern "C" int pbvi_prune_lp_certificates(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts,
+                                          int32_t* d_cert_idx, double* d_cert_w, void* stream) {
+    return prune_lp_impl<true>(m, d_alphas, nV, d_keep, d_bound, h_counts, d_cert_idx, d_cert_w, stream);
 }
 
 extern "C" int pbvi_prune_lp_stats(const pbvi_model* m, int64_t* h_out4) {

@@ -183,6 +183,8 @@ class GapSolver:
             lower.evaluate(gamma, eps)
         elif lower.rows is None or lower.gamma != gamma:
             raise ValueError('lower must be a PolicyGraph evaluated with the solver gamma')
+        elif lower.mixtures is not None:
+            raise ValueError('lower must be a PolicyGraph without mixtures: the solver keys its nodes by deterministic tuples')
         if upper is None:
             upper = UpperBound(model, FIB_Solver(gamma=gamma, eps=1e-6).solve(model, print_progress=False)[0], gamma)
         elif upper.gamma != gamma:

@@ -9,8 +9,13 @@ Finite-state controllers (policy graphs) extracted from a value function, and th
                   raises that bound by point-based policy iteration on the controller.  `outcomes` gives the exact success probability,
                   expected step count and return of runs that stop at end states, for every start (node, state) at once.
 
+A graph may also have stochastic successor edges: a mixture is a convex combination of nodes, and a successor entry N + m means "move
+to member k of mixture m with probability mu_k" (value-wise: the mixture row sum_k mu_k W_{node_k}).  `prune_lp` creates them when it
+drops a node that a convex combination of other nodes dominates.
+
 The file formats of `save` / `load` are pomdp-solve's: `.pg` ("id action succ_0 ... succ_{O-1}" per node) and `.alpha` (an action line, a
-values line and a blank line per node).
+values line and a blank line per node), plus `.mix` ("mixture_id k node_1 weight_1 ... node_k weight_k" per mixture) for a graph with
+mixtures.
 """
 from __future__ import annotations
 
@@ -61,6 +66,147 @@ def redirect_dominated(actions, successors, witness) -> tuple:
     renumber = np.full(act.shape[0], -1, dtype=np.int64)
     renumber[keep] = np.arange(len(keep))
     return keep, act[keep], renumber[target[succ[keep]]]
+
+
+def check_mixtures(mixtures, N: int):
+    """
+    The validated mixture table of a graph with N nodes: (offsets int64 [M+1], nodes int64 [nnz], weights float64 [nnz]) with offsets
+    rising strictly from 0 to nnz (no empty mixture), members in [0, N), finite weights >= 0 summing to 1 within 1e-12 per mixture.
+    None, or a table with M = 0, gives None.  Raises ValueError otherwise.
+    """
+    if mixtures is None:
+        return None
+    if len(mixtures) != 3:
+        raise ValueError('mixtures must be a tuple (offsets [M+1], nodes [nnz], weights [nnz])')
+    off, nodes, w = (np.asarray(x).reshape(-1) for x in mixtures)
+    if off.size == 0 or not np.issubdtype(off.dtype, np.integer) or (nodes.size and not np.issubdtype(nodes.dtype, np.integer)):
+        raise ValueError('mixture offsets and nodes must be integer arrays, with at least one offset')
+    off, nodes, w = off.astype(np.int64), nodes.astype(np.int64), w.astype(np.float64)
+    if off.size == 1 and off[0] == 0 and nodes.size == 0 and w.size == 0:
+        return None
+    if off[0] != 0 or off[-1] != nodes.size or w.size != nodes.size or np.any(np.diff(off) <= 0):
+        raise ValueError('mixture offsets must rise strictly from 0 to the number of members, with one weight per member')
+    if nodes.min() < 0 or nodes.max() >= N:
+        raise ValueError(f'mixture members must be nodes in [0, {N})')
+    if not np.all(np.isfinite(w)) or w.min() < 0.0:
+        raise ValueError('mixture weights must be finite and >= 0')
+    sums = np.add.reduceat(w, off[:-1])
+    if np.max(np.abs(sums - 1.0)) > 1e-12:
+        raise ValueError('the weights of every mixture must sum to 1 (within 1e-12)')
+    return off, nodes, w
+
+
+def resolve_certificates(pruned, cert_idx, cert_w, drop: float = 1e-13, max_rounds: int = 100) -> dict:
+    """
+    The LP certificates of `pbvi_prune_lp_certificates` resolved onto kept nodes: pruned bool [n]; cert_idx [n, J] (-1 padded) and
+    cert_w [n, J] the competitor sets and weights lambda of the pruned rows.  Returns {i: (nodes int64 ascending, weights float64)} for every
+    pruned i whose resolution is non-empty: the weights on kept nodes of W_i's dominating combination, after substituting each pruned
+    member j by its own combination (depth first, memoised; members that close a cycle are substituted again, in rounds, with the current
+    resolutions).  Every certificate has a strict margin (its combination exceeds its row by more than tau everywhere), so no closed set of
+    pruned rows keeps its weight among itself and the pruned mass decays geometrically.  What is left after `max_rounds`, and any weight
+    below `drop`, is dropped and the rest renormalised: the result is a candidate, which `PolicyGraph.prune_lp` verifies on the device.
+    """
+    pruned = np.asarray(pruned, dtype=bool).reshape(-1)
+    cert_idx, cert_w = np.asarray(cert_idx, dtype=np.int64), np.asarray(cert_w, dtype=np.float64)
+    state = np.zeros(pruned.shape[0], dtype=np.int8)          # 0 new, 1 in progress, 2 resolved (possibly with cycle members left)
+    res = {}
+
+    def combine(nodes, weights):
+        u, inv = np.unique(nodes, return_inverse=True)
+        return u, np.bincount(inv, weights=weights, minlength=len(u))
+
+    def substitute(nodes, weights, skip_in_progress):
+        parts_n, parts_w = [nodes[~pruned[nodes]]], [weights[~pruned[nodes]]]
+        for j, mu in zip(nodes[pruned[nodes]].tolist(), weights[pruned[nodes]].tolist()):
+            if skip_in_progress and state[j] == 1:
+                parts_n.append(np.asarray([j]))
+                parts_w.append(np.asarray([mu]))
+            else:
+                rn, rw = res[j]
+                parts_n.append(rn)
+                parts_w.append(mu * rw)
+        return combine(np.concatenate(parts_n), np.concatenate(parts_w))
+
+    def visit(i):
+        stack = [i]
+        state[i] = 1
+        while stack:
+            top = stack[-1]
+            sel = cert_idx[top] >= 0
+            nxt = [j for j in cert_idx[top][sel].tolist() if pruned[j] and state[j] == 0]
+            if nxt:
+                state[nxt[0]] = 1
+                stack.append(nxt[0])
+                continue
+            res[top] = substitute(cert_idx[top][sel], cert_w[top][sel], True)
+            state[top] = 2
+            stack.pop()
+
+    for i in np.flatnonzero(pruned).tolist():
+        if state[i] == 0:
+            visit(i)
+    for _ in range(max_rounds):
+        left = [i for i, (nodes, weights) in res.items() if np.any(pruned[nodes])]
+        if not left or all(float(np.sum(res[i][1][pruned[res[i][0]]])) <= drop for i in left):
+            break
+        for i in left:
+            res[i] = substitute(*res[i], False)
+    out = {}
+    for i, (nodes, weights) in res.items():
+        ok = ~pruned[nodes] & (weights > drop)
+        if np.any(ok):
+            out[i] = (nodes[ok], weights[ok] / np.sum(weights[ok]))
+    return out
+
+
+def mixture_rows(W: torch.Tensor, mixtures) -> torch.Tensor:
+    """Z [M, S]: the mixture rows over node rows W in the arithmetic of the mixture phase of `pbvi_controller_evaluate_mixed`:
+    z = mu_0 * W_0, then z = z + mu_k * W_k for the further members in stored order.  Each FP64 elementwise multiply and add rounds once
+    (no FMA), as the kernel's __dmul_rn / __dadd_rn."""
+    off, nodes, w = mixtures
+    d = W.device
+    lengths = np.diff(off)
+    Z = torch.empty((len(lengths), W.shape[1]), dtype=torch.float64, device=d)
+    for p in range(int(lengths.max()) if len(lengths) else 0):
+        sel = np.flatnonzero(lengths > p)
+        k = off[sel] + p
+        t = W[torch.as_tensor(nodes[k], device=d)] * torch.as_tensor(w[k], dtype=torch.float64, device=d)[:, None]
+        rows = torch.as_tensor(sel, device=d)
+        Z[rows] = t if p == 0 else Z[rows] + t
+    return Z
+
+
+def compact_graph(actions, successors, redirect, mixtures=None, member_target=None) -> tuple:
+    """
+    A graph after dropping nodes.  redirect [N] sends the edges into each node to the node itself (it is kept), to another kept node, or
+    to a mixture entry N + m of `mixtures` (which may hold more mixtures than the graph referenced so far); mixture members go to
+    member_target [N] (default: redirect), which must name kept nodes.  Returns (kept node indices ascending, their actions, their
+    successors, the mixtures that some kept edge references or None), nodes renumbered to positions in the kept list and the mixtures
+    kept in their old order.
+    """
+    act = np.asarray(actions, dtype=np.int64).reshape(-1)
+    succ = np.asarray(successors, dtype=np.int64)
+    redirect = np.asarray(redirect, dtype=np.int64).reshape(-1)
+    N = act.shape[0]
+    keep = np.flatnonzero(redirect == np.arange(N))
+    K = len(keep)
+    renumber = np.full(N, -1, dtype=np.int64)
+    renumber[keep] = np.arange(K)
+    s = succ[keep]
+    s = np.where(s < N, redirect[np.minimum(s, N - 1)], s)
+    if mixtures is None:
+        return keep, act[keep], renumber[s], None
+    off, nodes, w = mixtures
+    used = np.unique(s[s >= N]) - N
+    mix_renumber = np.full(len(off) - 1, -1, dtype=np.int64)
+    mix_renumber[used] = np.arange(len(used))
+    target = redirect if member_target is None else np.asarray(member_target, dtype=np.int64).reshape(-1)
+    sel = np.concatenate([np.arange(off[m], off[m + 1]) for m in used]) if len(used) else np.zeros(0, dtype=np.int64)
+    out = np.where(s < N, renumber[np.minimum(s, N - 1)], K + mix_renumber[np.maximum(s - N, 0)])
+    if not len(used):
+        return keep, act[keep], out, None
+    table = (np.concatenate([[0], np.cumsum(np.diff(off)[used])]), renumber[target[nodes[sel]]], w[sel])
+    return keep, act[keep], out, table
 
 
 def backup_tuples(dev, beliefs: torch.Tensor, rows: torch.Tensor, gamma: float) -> np.ndarray:
@@ -116,9 +262,13 @@ class PolicyGraph:
     A finite-state controller over `model`: `actions` [N] and `successors` [N, O] (node indices) as host int64 arrays; after `evaluate` (or
     `load` of a saved graph with rows) `rows` [N, S] is a CUDA float64 tensor of node values.  `source_rows` [N] holds, for an extracted
     graph, the row of the value function each node came from (None otherwise).
+
+    `mixtures` (optional): stochastic successor edges as a CSR table (offsets [M+1], nodes [nnz], weights [nnz]) -- mixture m moves to
+    node nodes[k] with probability weights[k] for k in [offsets[m], offsets[m+1]) (members in [0, N), FP64 weights >= 0 summing to 1
+    within 1e-12) -- and a successor entry N + m means "mixture m".  Stored as host int64 / int64 / float64 arrays, or None.
     """
 
-    def __init__(self, model: Model, actions, successors, rows=None, source_rows=None):
+    def __init__(self, model: Model, actions, successors, rows=None, source_rows=None, mixtures=None):
         self.model = model
         A, O, S = model.action_count, model.observation_count, model.state_count
         act = np.asarray(actions).astype(np.int64).reshape(-1)
@@ -130,8 +280,10 @@ class PolicyGraph:
             raise ValueError(f'successors must be [{N}, {O}], got {tuple(succ.shape)}')
         if act.min() < 0 or act.max() >= A:
             raise ValueError(f'node actions must lie in [0, {A})')
-        if succ.min() < 0 or succ.max() >= N:
-            raise ValueError(f'successor nodes must lie in [0, {N})')
+        self.mixtures = check_mixtures(mixtures, N)
+        M = 0 if self.mixtures is None else len(self.mixtures[0]) - 1
+        if succ.min() < 0 or succ.max() >= N + M:
+            raise ValueError(f'successor entries must lie in [0, {N + M}) ({N} nodes, {M} mixtures)')
         self.actions, self.successors = act, succ
         self.source_rows = None if source_rows is None else np.asarray(source_rows).astype(np.int64).reshape(-1)
         self.rows = None
@@ -144,6 +296,7 @@ class PolicyGraph:
         self.witnesses = None          # [N, S] of an extracted graph: the belief at which each node's row was chosen
         self._value_function = None
         self.gamma = None              # discount of the last `evaluate`
+        self.prune_stats = None        # of a graph that `prune_lp` returned
 
     def __len__(self) -> int:
         return int(self.actions.shape[0])
@@ -232,7 +385,8 @@ class PolicyGraph:
 
         Iterates W <- T_pi W (`pbvi_controller_evaluate`: every sweep in one persistent launch, synchronised once) from the source rows
         (the Rbar rows of the node actions for a graph without them; the start `improve` sets) until max |T_pi W - W| <
-        eps * gamma / (1 - gamma) or `max_sweeps` sweeps.  Certificate, the
+        eps * gamma / (1 - gamma) or `max_sweeps` sweeps.  A graph with mixtures runs `pbvi_controller_evaluate_mixed`, whose sweeps
+        read a mixture successor as the mixture row sum_k mu_k W_{node_k}; the certificate is the same.  Certificate, the
         mirror image of FIB_Solver's: with e = max(W - T_pi W) and gamma' = gamma * max(1, max_{s,a} sum_{o,r} RTO) the returned rows are
         W - max(e, 0) / (1 - gamma').  A constant shift c >= 0 passes through T_pi as at most gamma' * c, so they satisfy W <= T_pi W; they
         are re-checked with one more sweep, and while rounding leaves a positive residual e' the rows are lowered again by
@@ -258,7 +412,10 @@ class PolicyGraph:
         if max_sweeps >= 1:
             # the whole iteration is one persistent launch; the sweeps are not timed one by one, so each gets an even share of the wall time
             start = time.perf_counter()
-            W, changes, k = dev.controller_evaluate(W, gamma, act, succ, tol, max_sweeps)
+            if self.mixtures is None:
+                W, changes, k = dev.controller_evaluate(W, gamma, act, succ, tol, max_sweeps)
+            else:
+                W, changes, k = dev.controller_evaluate_mixed(W, gamma, act, succ, self.mixtures, tol, max_sweeps)
             changes = changes.cpu().numpy().tolist()
             per_sweep = (time.perf_counter() - start) / k
             for c in changes:
@@ -266,7 +423,7 @@ class PolicyGraph:
             change = changes[-1]
             if change != change:
                 raise ValueError('the controller iterates are not finite')
-        residual = float(dev.controller_sweep(W, gamma, act, succ, want_stats=True)[1][1])
+        residual = self._residual(W, gamma, act, succ)
         if residual != residual:
             raise ValueError('the controller iterates are not finite')
         shift = max(residual, 0.0) / (1.0 - gamma_c)
@@ -277,7 +434,7 @@ class PolicyGraph:
         m = self.model
         ulps = (m.observation_count * m.reachable_state_count + 2) * 2.0 ** -52
         for _ in range(3):
-            left = float(dev.controller_sweep(W, gamma, act, succ, want_stats=True)[1][1])
+            left = self._residual(W, gamma, act, succ)
             if not left > 0.0:
                 break
             extra = (left + ulps * float(torch.max(torch.abs(W)))) / (1.0 - gamma_c)
@@ -290,6 +447,16 @@ class PolicyGraph:
         if print_progress:
             log(f'PolicyGraph: {len(self)} nodes, {history.sweeps} sweeps, residual max(W - TW) = {residual:.3e}, certificate shift {shift:.3e}')
         return self.rows, history
+
+    def _residual(self, W, gamma, act, succ) -> float:
+        """max(W - T_pi W) over every entry (NaN wins) from one sweep: `pbvi_controller_sweep`'s stats, or for a graph with mixtures one
+        sweep of `pbvi_controller_evaluate_mixed` (W - out rounds as -(out - W), so it is the same quantity)."""
+        dev = self.model.device
+        if self.mixtures is None:
+            return float(dev.controller_sweep(W, gamma, act, succ, want_stats=True)[1][1])
+        out = dev.controller_evaluate_mixed(W, gamma, act, succ, self.mixtures, float('inf'), 1)[0]
+        d = W - out
+        return float('nan') if bool(torch.isnan(d).any()) else float(d.max())
 
     # ---- improvement -------------------------------------------------------------------------------------------------------
     def improve(self, beliefs, iterations: int = 1, eps: float = 1e-6) -> tuple:
@@ -317,11 +484,13 @@ class PolicyGraph:
         by their shift, and that is what a caller sees at most as a fall.  Pruning keeps the argmax nodes of B and everything they reach.
 
         Stats per iteration: nodes_before, nodes_after, appended, overwritten, pruned, sweeps, value_b0 (certified), shift and
-        seconds {select, assemble, dominance, evaluate, prune}.
+        seconds {select, assemble, dominance, evaluate, prune}.  A graph with mixtures raises ValueError.
         """
         self._require_rows()
         if self.gamma is None:
             raise ValueError('improve needs the gamma of evaluate: call evaluate(gamma) first')
+        if self.mixtures is not None:
+            raise ValueError('improve needs a graph without mixtures: it keys nodes by deterministic (action, successors) tuples')
         m, gamma = self.model, self.gamma
         dev = m.device
         B = belief_rows(m, m.start_probabilities)
@@ -386,12 +555,78 @@ class PolicyGraph:
         (T_new W)_p >= (T_old W)_p >= W_p, and no other row or entry changes.  The certificate W <= T_pi W therefore still holds and the
         kept rows need no re-evaluation.  max_n W_n . b is unchanged at every belief, bitwise in FP64: `max_values` sums every row in the
         same order with b >= 0, and rounded products, sums and FMAs are monotone in each argument, so the computed value of W_j is >= that
-        of W_i.
+        of W_i.  In a graph with mixtures the members of every mixture go along the witness chains too (a mixture row can only rise,
+        entry by entry), and only the mixtures that some kept edge references are kept.
         """
         W = self._require_rows()
-        keep, act, succ = redirect_dominated(self.actions, self.successors, self.model.device.dominating_row(W).cpu().numpy())
-        pg = PolicyGraph(self.model, act, succ, rows=W[torch.as_tensor(keep, device=W.device)])
+        witness = self.model.device.dominating_row(W).cpu().numpy()
+        if self.mixtures is None:
+            keep, act, succ = redirect_dominated(self.actions, self.successors, witness)
+            mix = None
+        else:
+            keep, act, succ, mix = compact_graph(self.actions, self.successors, resolve_witnesses(witness), self.mixtures)
+        pg = PolicyGraph(self.model, act, succ, rows=W[torch.as_tensor(keep, device=W.device)], mixtures=mix)
         pg.gamma = self.gamma
+        return pg
+
+    def prune_lp(self) -> 'PolicyGraph':
+        """
+        The graph without the nodes that a convex combination of other nodes dominates: a new PolicyGraph with mixtures, the kept rows,
+        `gamma` and `prune_stats`; this graph is not changed.  Needs rows (an evaluated graph) and a graph without mixtures.
+
+          1. `prune_dominated()`: `pbvi_prune_lp` needs pairwise distinct rows, and pointwise pruning leaves no two equal rows.
+          2. `pbvi_prune_lp_certificates` on the rows: node i is pruned when a convex combination lambda of other rows exceeds W_i by more
+             than tau = 1e-9 * max(1, max |W|) at every state (verified in FP64), and lambda comes back with it.
+          3. `resolve_certificates`: lambda's weight on pruned nodes is substituted by their own combinations until it is negligible; small
+             weights are dropped and the rest renormalised: a mixture of kept nodes per pruned node.
+          4. Each mixture is verified on the device: Z_i = `mixture_rows` (the arithmetic of the mixture phase of the sweeps) must satisfy
+             Z_i[s] - W_i[s] > tau / 2 at every state.  A node that fails is kept with its own edges; the others stay valid, because each
+             mixture is verified on its own and names kept nodes only.
+          5. Every edge into a pruned node goes to its mixture (successor entry N' + m); only mixtures that some edge references are stored.
+
+        Why nothing needs re-evaluation: the RTO weights are non-negative and the computed Z_i >= W_i entry by entry, and rounded products
+        and sums are monotone in each argument, so every predecessor p sees (T' W)_p >= (T W)_p >= W_p in the sweep's own arithmetic: the
+        certificate W <= T_pi W survives.  The value is bitwise unchanged: tau / 2 is far above the rounding of a dot product (even at
+        S = 22 021, FP64 rounding of b . W is below 1e-11 relative), and Z_i is a convex combination of kept rows, so some kept row beats
+        W_i . b at every belief b and a pruned row never attains max_n W_n . b; that maximum, over the same kept rows in the same order, is
+        bitwise the same at every belief, with the same best node.  An `evaluate` afterwards starts from rows that satisfy X <= T_pi' X,
+        so its certified value can only rise, up to its own shift.
+
+        `prune_stats`: nodes, after_dominated, nodes_after, mixtures, nnz, lp_counts (kept at a corner, kept by an LP witness, pruned, kept
+        undecided), lp_stats (`prune_lp_stats`), failed (pruned by the LP but not verified) and seconds.
+        """
+        t0 = time.perf_counter()
+        self._require_rows()
+        if self.mixtures is not None:
+            raise ValueError('prune_lp needs a graph without mixtures')
+        dev = self.model.device
+        pd = self.prune_dominated()
+        W = pd.rows
+        N = len(pd)
+        keep, _, counts, cidx, cw = dev.prune_lp_certificates(W)
+        lp_stats = dev.prune_lp_stats()
+        pruned = keep.cpu().numpy() == 0
+        res = resolve_certificates(pruned, cidx.cpu().numpy(), cw.cpu().numpy())
+        cand = sorted(res)
+        ok = np.zeros(0, dtype=bool)
+        if cand:
+            off = np.concatenate([[0], np.cumsum([len(res[i][0]) for i in cand])]).astype(np.int64)
+            table = (off, np.concatenate([res[i][0] for i in cand]), np.concatenate([res[i][1] for i in cand]))
+            tau = 1e-9 * max(1.0, float(torch.max(torch.abs(W))))
+            Z = mixture_rows(W, table)
+            ok = ((Z - W[torch.as_tensor(cand, device=W.device)]) > tau / 2).all(dim=1).cpu().numpy()
+        redirect = np.arange(N, dtype=np.int64)
+        good = [i for i, v in zip(cand, ok.tolist()) if v]
+        if good:
+            redirect[good] = N + np.flatnonzero(ok)
+            kept, act, succ, mix = compact_graph(pd.actions, pd.successors, redirect, table, np.arange(N))
+        else:
+            kept, act, succ, mix = np.arange(N), pd.actions, pd.successors, None
+        pg = PolicyGraph(self.model, act, succ, rows=W[torch.as_tensor(kept, device=W.device)], mixtures=mix)
+        pg.gamma = self.gamma
+        pg.prune_stats = dict(nodes=len(self), after_dominated=N, nodes_after=len(pg), mixtures=0 if mix is None else len(mix[0]) - 1,
+                              nnz=0 if mix is None else len(mix[1]), lp_counts=counts.tolist(), lp_stats=lp_stats,
+                              failed=int(pruned.sum()) - len(good), seconds=time.perf_counter() - t0)
         return pg
 
     def _require_rows(self) -> torch.Tensor:
@@ -417,6 +652,8 @@ class PolicyGraph:
         drawn from the belief (default b0), and every agent starts in the best node for it.  Each step collects Rbar[s, a_node], draws
         (o, r) jointly from RTO[s, a_node, :, :], then moves s <- reach[s, a, r] and node <- sigma(node, o).  A validation tool, not a
         hot path: NumPy, vectorised over agents.  Raises ValueError when an RTO row does not sum to 1 (within 1e-9).
+        In a graph with mixtures every step draws one more uniform per agent (after the observation's), and an agent whose edge leads to
+        mixture m moves to the first member k whose cumulative weight exceeds it; a graph without mixtures draws nothing more.
         """
         self._require_rows()
         if self.gamma is None:
@@ -435,6 +672,12 @@ class PolicyGraph:
         s = rng.choice(S, size=n, p=p / p.sum())
         node = np.full(n, node0, dtype=np.int64)
         cdf = np.cumsum(rto.reshape(S, A, O * R), axis=2)
+        N = len(self)
+        if self.mixtures is not None:
+            off, members, w = self.mixtures
+            mix_of = np.repeat(np.arange(len(off) - 1), np.diff(off))
+            # member k of mixture m covers cumulative weights up to m + sum_{k' <= k} w_k' (within the mixture): one sorted key array
+            key = mix_of + np.concatenate([np.cumsum(w[off[m]:off[m + 1]]) for m in range(len(off) - 1)])
         ret = np.zeros(n)
         disc = 1.0
         for _ in range(max_steps):
@@ -445,6 +688,12 @@ class PolicyGraph:
             o, r = k // R, k % R
             s = reach[s, a, r]
             node = self.successors[node, o]
+            if self.mixtures is not None:
+                u2 = rng.random(n)
+                mx = np.flatnonzero(node >= N)
+                m = node[mx] - N
+                k = np.searchsorted(key, m + u2[mx], side='right')
+                node[mx] = members[np.clip(k, off[m], off[m + 1] - 1)]
             disc *= self.gamma
         return ret
 
@@ -456,7 +705,8 @@ class PolicyGraph:
         reward counts, nothing after it does, and a run that starts in an end state still takes its first step.  With T the stopping step
         and H = `max_steps`, returns (`ControllerOutcomes`) P(T <= H), E[min(T, H)] and the discounted return
         G = E[sum_{t < min(T, H)} gamma^t r_t] at each query pair, the same after every k <= H, and the rows over every (node, state).
-        No sampling: `pbvi_controller_outcomes` runs the H steps of the three recursions over (node, state) in one persistent launch.
+        No sampling: `pbvi_controller_outcomes` runs the H steps of the three recursions over (node, state) in one persistent launch
+        (`pbvi_controller_outcomes_mixed` for a graph with mixtures: a mixture successor contributes the mixture of its members' rows).
 
         G starts its discount at 1 (gamma^0 on the first reward); the average discounted reward the reference's simulations print starts
         it at gamma, so it is gamma * G.  With gamma = 1 and a finite H, G is the reference's average total reward.
@@ -494,12 +744,17 @@ class PolicyGraph:
         end_state[np.asarray(m.end_states, dtype=np.int64)] = 1
         end_action = np.zeros(m.action_count, dtype=np.uint8)
         end_action[np.asarray(m.end_actions, dtype=np.int64)] = 1
-        P, M, G, series = m.device.controller_outcomes(self.actions, self.successors, end_state, end_action, gamma, max_steps, B, nodes)
+        if self.mixtures is None:
+            P, M, G, series = m.device.controller_outcomes(self.actions, self.successors, end_state, end_action, gamma, max_steps, B, nodes)
+        else:
+            P, M, G, series = m.device.controller_outcomes_mixed(self.actions, self.successors, self.mixtures, end_state, end_action, gamma,
+                                                                 max_steps, B, nodes)
         return ControllerOutcomes(nodes, series.cpu().numpy(), (P, M, G), gamma, max_steps)
 
     # ---- persistence (pomdp-solve formats) --------------------------------------------------------------------------------
     def save(self, path: str, name: str) -> None:
-        """Writes `<path>/<name>.pg` and, when the graph has rows, `<path>/<name>.alpha` (values as %.17g: a round trip is bitwise)."""
+        """Writes `<path>/<name>.pg`, when the graph has rows `<path>/<name>.alpha`, and when it has mixtures `<path>/<name>.mix`
+        ("mixture_id k node_1 weight_1 ... node_k weight_k" per mixture).  Values and weights as %.17g: a round trip is bitwise."""
         os.makedirs(path, exist_ok=True)
         with open(os.path.join(path, name + '.pg'), 'w') as f:
             for i in range(len(self)):
@@ -509,10 +764,16 @@ class PolicyGraph:
             with open(os.path.join(path, name + '.alpha'), 'w') as f:
                 for i in range(len(self)):
                     f.write(f'{int(self.actions[i])}\n' + ' '.join('%.17g' % x for x in rows[i]) + '\n\n')
+        if self.mixtures is not None:
+            off, members, w = self.mixtures
+            with open(os.path.join(path, name + '.mix'), 'w') as f:
+                for m in range(len(off) - 1):
+                    pairs = ' '.join(f'{int(members[k])} {w[k]:.17g}' for k in range(off[m], off[m + 1]))
+                    f.write(f'{m} {off[m + 1] - off[m]} {pairs}\n')
 
     @classmethod
     def load(cls, path: str, name: str, model: Model) -> 'PolicyGraph':
-        """Reads what `save` wrote (the `.alpha` file is optional); node ids must be 0..N-1 in order."""
+        """Reads what `save` wrote (the `.alpha` and `.mix` files are optional); node ids must be 0..N-1 and mixture ids 0..M-1 in order."""
         with open(os.path.join(path, name + '.pg')) as f:
             lines = [ln.split() for ln in f if ln.strip()]
         table = np.asarray([[int(x) for x in ln] for ln in lines], dtype=np.int64)
@@ -526,4 +787,17 @@ class PolicyGraph:
             if len(lines) != 2 * len(table) or any(int(lines[2 * i][0]) != table[i, 1] for i in range(len(table))):
                 raise ValueError(f'{name}.alpha does not match {name}.pg')
             rows = np.asarray([[float(x) for x in lines[2 * i + 1]] for i in range(len(table))], dtype=np.float64)
-        return cls(model, table[:, 1], table[:, 2:], rows=rows)
+        mixtures = None
+        mix = os.path.join(path, name + '.mix')
+        if os.path.isfile(mix):
+            with open(mix) as f:
+                lines = [ln.split() for ln in f if ln.strip()]
+            off, members, weights = [0], [], []
+            for m, ln in enumerate(lines):
+                if int(ln[0]) != m or len(ln) != 2 + 2 * int(ln[1]):
+                    raise ValueError(f'{name}.mix: expected lines "mixture_id k node_1 weight_1 .. node_k weight_k" with ids 0..M-1')
+                members += [int(x) for x in ln[2::2]]
+                weights += [float(x) for x in ln[3::2]]
+                off.append(len(members))
+            mixtures = (np.asarray(off, dtype=np.int64), np.asarray(members, dtype=np.int64), np.asarray(weights, dtype=np.float64))
+        return cls(model, table[:, 1], table[:, 2:], rows=rows, mixtures=mixtures)
