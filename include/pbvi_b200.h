@@ -310,6 +310,21 @@ PBVI_API int pbvi_prune_lp_certificates(pbvi_model* m, const double* d_alphas, i
 /* instrumentation of the last pbvi_prune_lp call: h_out4 = {largest competitor set |J| reached, restricted LPs solved, simplex pivots,
  * rows sent to the LP stage} */
 PBVI_API int pbvi_prune_lp_stats(const pbvi_model* m, int64_t* h_out4);
+/* pbvi_bpi_lp: one round of the restricted master LPs of bounded policy iteration (PolicyGraph.bounded_improve), a block per entry.
+ * Entry i improves node row W_i = d_pool[i] over the columns d_pool[d_cols[i][0 .. d_ncols[i])] (pool rows; d_cols[i][0] = the node's
+ * own one-sweep row, which is also at pool row n + i; at most 64 columns):  delta_J = max_{b in simplex} min_q b . (W_i - C_q).
+ * Only entries with d_status[i] == -1 run.  With d_price[i] >= 0 (the pool row of the backup at the last tangent belief d_bstar[i]),
+ * m* = b* . (W_i - C_price) goes to d_mstar[i] and decides first: m* > -tau -> status 1 (not improvable), m* >= d_delta[i] - tau or the
+ * column already listed -> 2 (the last LP is optimal), 64 columns -> 3 (budget); otherwise the column is appended.  Then the LP is
+ * solved cold from the seed corner d_corner[i] (the code of pbvi_prune_lp): d_delta[i] = delta_J, d_u[i] = the verified bound
+ * max_s (W_i - sum_q lambda_q C_q)[s], d_lambda[i][64] (0 padded), the dense tangent belief d_bstar[i][S], status stays -1; a pivot
+ * budget (3) or numerical trouble (4) leaves them as they were.  tau > 0 scales the simplex as in pbvi_prune_lp (scl = 1e9 tau).
+ * The caller guarantees 1 <= d_ncols[i] <= 64, listed columns and d_price[i] in [0, nP) and d_corner[i] in [0, S) for active entries
+ * (DeviceModel.bpi_lp checks them).  h_stats4 (nullable) = {largest column count, LPs solved, simplex pivots, entries run}.
+ * Synchronises `stream`. */
+PBVI_API int pbvi_bpi_lp(pbvi_model* m, const double* d_pool, int nP, int n, double tau, const int32_t* d_corner, const int32_t* d_price,
+                         int32_t* d_cols, int32_t* d_ncols, double* d_bstar, double* d_delta, double* d_u, double* d_lambda, double* d_mstar,
+                         int32_t* d_status, int64_t* h_stats4, void* stream);
 
 /* ---- HSVI sawtooth upper bound (BeliefValueMapping.evaluate, src/pomdp.py:887-895) -----------------
  * d_out[q] = min(v0_q, min_i v0_q + (ub_value_i - ub_belief_i . corner) * min_{s: ub_belief_i[s] > 0} query_q[s]/ub_belief_i[s]) */

@@ -62,6 +62,7 @@ SIGNATURES = {
     'pbvi_prune_lp': [_P, _P, c_int, _P, _P, _P, _P],
     'pbvi_prune_lp_certificates': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_prune_lp_stats': [_P, _P],
+    'pbvi_bpi_lp': [_P, _P, c_int, c_int, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth': [_P, _P, _P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_support_lists': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth_lists': [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int, _P, _P],
@@ -657,6 +658,32 @@ class DeviceModel:
         out = np.zeros(4, dtype=np.int64)
         _check(self._lib.pbvi_prune_lp_stats(self._h, out.ctypes.data))
         return dict(max_competitors=int(out[0]), lps=int(out[1]), pivots=int(out[2]), lp_rows=int(out[3]))
+
+    def bpi_lp(self, pool, n: int, tau: float, corner, price, cols, ncols, bstar, delta, u, lam, mstar, status) -> dict:
+        """One round of the restricted master LPs of bounded policy iteration (`pbvi_bpi_lp`) on n entries, updating the state tensors in
+        place: pool [P, S] float64 (rows 0..n-1 the node rows, rows n..2n-1 their own one-sweep rows, then priced columns), corner / price /
+        ncols / status int32 [n], cols int32 [n, 64], bstar float64 [n, S], delta / u / mstar float64 [n], lam float64 [n, 64], all CUDA and
+        contiguous.  Returns {max_columns, lps, pivots, entries}.  Synchronises."""
+        S = self.S
+        for t, shape, dt in ((pool, (pool.shape[0], S), torch.float64), (corner, (n,), torch.int32), (price, (n,), torch.int32),
+                             (cols, (n, 64), torch.int32), (ncols, (n,), torch.int32), (bstar, (n, S), torch.float64),
+                             (delta, (n,), torch.float64), (u, (n,), torch.float64), (lam, (n, 64), torch.float64),
+                             (mstar, (n,), torch.float64), (status, (n,), torch.int32)):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dt and tuple(t.shape) == shape and t.is_contiguous()):
+                raise ValueError(f'bpi_lp: expected a contiguous CUDA {dt} tensor of shape {shape}')
+        act = status == -1
+        if bool(act.any()):
+            k = ncols[act]
+            listed = torch.arange(64, device=self.device)[None, :] < ncols[act][:, None].long()
+            c, p, s0 = cols[act][listed], price[act], corner[act]
+            if (int(k.min()) < 1 or int(k.max()) > 64 or int(c.min()) < 0 or int(c.max()) >= pool.shape[0] or int(p.max()) >= pool.shape[0]
+                    or int(s0.min()) < 0 or int(s0.max()) >= S):
+                raise ValueError('bpi_lp: active entries need 1..64 columns, column and price rows below the pool size and corners in [0, S)')
+        out = np.zeros(4, dtype=np.int64)
+        self._call(self._lib.pbvi_bpi_lp(self._h, _ptr(pool), pool.shape[0], int(n), float(tau), _ptr(corner), _ptr(price), _ptr(cols),
+                                         _ptr(ncols), _ptr(bstar), _ptr(delta), _ptr(u), _ptr(lam), _ptr(mstar), _ptr(status),
+                                         out.ctypes.data, self._stream))
+        return dict(max_columns=int(out[0]), lps=int(out[1]), pivots=int(out[2]), entries=int(out[3]))
 
     def sawtooth(self, corner, ub_beliefs, ub_values, queries) -> torch.Tensor:
         c, q = _f64(corner, self.device), self._beliefs(queries)

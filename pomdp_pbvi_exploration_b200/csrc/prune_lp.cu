@@ -24,6 +24,8 @@
 // out rows to blocks and count outcomes, neither reaches a value.
 #include <algorithm>
 #include <climits>
+#include <cmath>
+#include <type_traits>
 
 #include "pbvi_common.cuh"
 
@@ -168,6 +170,42 @@ __device__ __forceinline__ void write_certificate(int32_t* certIdx, double* cert
     certW[(size_t)i * J_MAX + q] = lambda;
 }
 
+// Bounded policy iteration (pbvi_bpi_lp) is the instantiation whose pack is one BpiArgs: the restricted master LP of node n over columns
+// of a pool, with A = the pool and row i of the pool = W_n of entry i, so the LP code above reads a_i and the columns exactly as it reads
+// rows and competitors.  Per launch and entry (keep[i] = -1: active), the column priced at the last tangent belief is checked and
+// appended, then one LP is solved from the seed corner; the verified lower bound over all rows is not computed (the pricing is).
+struct BpiArgs {
+    const int32_t* price;       // [n] pool row of the column priced at bstar (the backup at bstar), -1 on the first launch
+    int32_t* cols;              // [n, J_MAX] column lists (pool rows; cols[i][0] = the node's own one-sweep row)
+    int32_t* ncols;             // [n] their lengths
+    double* bstar;              // [n, S] tangent belief of the last LP (dense)
+    double* u;                  // [n] verified bound max_s (W_n - sum_q lambda_q C_q)[s] of the last LP
+    double* lambda;             // [n, J_MAX] its weights (0 beyond ncols)
+    double* mstar;              // [n] b* . (W_n - C_price) of the last check
+};
+
+template <typename... T>
+constexpr bool kIsBpi = (false || ... || std::is_same<T, BpiArgs>::value);
+
+__device__ __forceinline__ const BpiArgs& bpi_args(const BpiArgs& a) { return a; }
+
+// sum of v over the block in a fixed order (warp shuffles, then the warps in order); every thread receives the result
+__device__ double block_sum(double v, double* sv) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
+    if ((threadIdx.x & 31) == 0) sv[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = sv[0];
+        for (int k = 1; k < PL_THREADS / 32; k++) t += sv[k];
+        sv[PL_THREADS / 32] = t;
+    }
+    __syncthreads();
+    const double t = sv[PL_THREADS / 32];
+    __syncthreads();
+    return t;
+}
+
 template <bool kCert, typename... Cert>
 __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* __restrict__ A, int n, int S, const int32_t* __restrict__ finite,
                                                               const double* __restrict__ tauP, const int32_t* __restrict__ cornerS,
@@ -193,11 +231,37 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
         if (keep[i] != -1) continue;
         const double* ai = A + (size_t)i * S;
         const int s0 = cornerS[i];
-        if (tid == 0) J[0] = cornerJ[i];
+        if constexpr (!kIsBpi<Cert...>) {
+            if (tid == 0) J[0] = cornerJ[i];
+        }
         int k = 1;
         int verdict = -1;                                   // 0 pruned, 1 kept by an LP witness, 3 undecided
         double bnd = 0.0;
         unsigned long long pivots = 0, rounds = 0;
+        if constexpr (kIsBpi<Cert...>) {
+            // the column priced at the last b*: m* = b* . (W_n - C_price) <= delta over every column <= delta_J
+            const BpiArgs& g = bpi_args(cert...);
+            k = g.ncols[i];
+            if (tid < k) J[tid] = g.cols[(size_t)i * J_MAX + tid];
+            const int p = g.price[i];
+            if (p >= 0) {
+                double v = 0.0;
+                for (int s = tid; s < S; s += PL_THREADS) v = fma(g.bstar[(size_t)i * S + s], ai[s] - A[(size_t)p * S + s], v);
+                const double mstar = block_sum(v, sv);
+                bool inJ = false;
+                for (int q = 0; q < k; q++) inJ |= J[q] == p;
+                // 1: not improvable by more than tau, 2: the last LP is optimal, 3: column budget
+                const int st = mstar > -tau ? 1 : (inJ || mstar >= bound[i] - tau) ? 2 : k == J_MAX ? 3 : -1;
+                if (tid == 0) g.mstar[i] = mstar;
+                if (st >= 0) {
+                    if (tid == 0) { keep[i] = st; atomicAdd(counts + st, 1); }
+                    continue;
+                }
+                if (tid == 0) { J[k] = p; g.cols[(size_t)i * J_MAX + k] = p; g.ncols[i] = k + 1; }
+                k++;
+            }
+            __syncthreads();
+        }
         while (verdict < 0) {
             rounds++;
             const int m = k + 1;
@@ -331,16 +395,20 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
             // ---- verified lower bound: m* = min over every finite j != i of b* . (alpha_i - alpha_j) ----
             double mv = -INFINITY;
             int mj = INT_MAX;
-            for (int j = tid; j < n; j += PL_THREADS) {
-                if (j == i || !finite[j]) continue;
-                const double* aj = A + (size_t)j * S;
-                double v = 0.0;
-                for (int p = 0; p < ns; p++) v = fma(suppB[p], ai[suppS[p]] - aj[suppS[p]], v);
-                arg_better(mv, mj, -v, j);
+            if constexpr (!kIsBpi<Cert...>) {
+                for (int j = tid; j < n; j += PL_THREADS) {
+                    if (j == i || !finite[j]) continue;
+                    const double* aj = A + (size_t)j * S;
+                    double v = 0.0;
+                    for (int p = 0; p < ns; p++) v = fma(suppB[p], ai[suppS[p]] - aj[suppS[p]], v);
+                    arg_better(mv, mj, -v, j);
+                }
+                block_argmax(mv, mj, sv, si);
             }
-            block_argmax(mv, mj, sv, si);
             const double mstar = -mv;
-            if (mstar > -tau) { verdict = 1; bnd = mstar; break; }
+            if constexpr (!kIsBpi<Cert...>) {
+                if (mstar > -tau) { verdict = 1; bnd = mstar; break; }
+            }
             // ---- verified upper bound: u = max_s (alpha_i - sum_q lambda_q alpha_J[q])[s] ----
             double uv = -INFINITY;
             int us = INT_MAX;
@@ -354,6 +422,7 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
                 uv = INFINITY; us = 0;
             }
             block_argmax(uv, us, sv, si);
+            if constexpr (kIsBpi<Cert...>) { verdict = 0; bnd = uv; break; }          // one LP per launch: the host prices at b*
             if (uv < -tau) { verdict = 0; bnd = uv; break; }
             // ---- cut: the row that beats alpha_i most at b* joins J ----
             bool inJ = false;
@@ -366,6 +435,28 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
         }
         if constexpr (kCert) {
             if (verdict == 0 && tid < k) write_certificate(cert..., i, tid, J[tid], lam[tid]);   // J and lambda of the LP that gave u
+        }
+        if constexpr (kIsBpi<Cert...>) {
+            // an LP that ran out of pivots (3) or into numerical trouble (4) leaves the previous LP's outputs as they were
+            const BpiArgs& g = bpi_args(cert...);
+            if (verdict == 0) {
+                double* b = g.bstar + (size_t)i * S;
+                for (int s = tid; s < S; s += PL_THREADS) b[s] = 0.0;
+                __syncthreads();
+                if (tid < shNSupp) b[suppS[tid]] = suppB[tid];
+                if (tid < J_MAX) g.lambda[(size_t)i * J_MAX + tid] = tid < k ? lam[tid] : 0.0;
+            }
+            if (tid == 0) {
+                const int st = verdict == 0 ? -1 : shStatus == 1 ? 3 : 4;
+                if (verdict == 0) { bound[i] = xB[shJstar] * scl; g.u[i] = bnd; }
+                keep[i] = st;
+                if (st >= 0) atomicAdd(counts + st, 1);
+                atomicMax(stats + 0, (unsigned long long)k);
+                atomicAdd(stats + 1, rounds);
+                atomicAdd(stats + 2, pivots);
+                atomicAdd(stats + 3, 1ull);
+            }
+            continue;
         }
         if (tid == 0) {
             keep[i] = verdict == 0 ? 0 : 1;
@@ -455,6 +546,43 @@ extern "C" int pbvi_prune_lp(pbvi_model* m, const double* d_alphas, int nV, int3
 extern "C" int pbvi_prune_lp_certificates(pbvi_model* m, const double* d_alphas, int nV, int32_t* d_keep, double* d_bound, int32_t* h_counts,
                                           int32_t* d_cert_idx, double* d_cert_w, void* stream) {
     return prune_lp_impl<true>(m, d_alphas, nV, d_keep, d_bound, h_counts, d_cert_idx, d_cert_w, stream);
+}
+
+extern "C" int pbvi_bpi_lp(pbvi_model* m, const double* d_pool, int nP, int n, double tau, const int32_t* d_corner, const int32_t* d_price,
+                           int32_t* d_cols, int32_t* d_ncols, double* d_bstar, double* d_delta, double* d_u, double* d_lambda, double* d_mstar,
+                           int32_t* d_status, int64_t* h_stats4, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_REQUIRE(n >= 0 && nP >= 2 * n, "need n >= 0 entries and a pool of at least 2n rows (the node rows, then the own columns)");
+    PBVI_REQUIRE(tau > 0.0 && std::isfinite(tau), "tau must be finite and > 0");
+    if (h_stats4) std::fill(h_stats4, h_stats4 + 4, 0ll);
+    m->last_launches = 0;
+    if (n == 0) return PBVI_OK;
+    PBVI_REQUIRE(d_pool && d_corner && d_price && d_cols && d_ncols && d_bstar && d_delta && d_u && d_lambda && d_mstar && d_status,
+                 "NULL pointer argument");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    PBVI_TAKE(tauD, double, 1);
+    PBVI_TAKE(counters, int, 8);                          // [0] entry queue, [1..4] status counts
+    PBVI_TAKE(stats, unsigned long long, 4);
+    PBVI_CUDA(cudaMemcpyAsync(tauD, &tau, sizeof(double), cudaMemcpyHostToDevice, st));
+    PBVI_CUDA(cudaMemsetAsync(counters, 0, 8 * sizeof(int), st));
+    PBVI_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), st));
+    const BpiArgs args{d_price, d_cols, d_ncols, d_bstar, d_u, d_lambda, d_mstar};
+    int perSM = 1;
+    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, prune_lp_kernel<false, BpiArgs>, PL_THREADS, 0));
+    const int grid = std::max(1, std::min(n, m->sm_count * std::max(perSM, 1)));
+    // finite and cornerJ are not read: no search over rows, and J comes from the entry's column list
+    prune_lp_kernel<false><<<grid, PL_THREADS, 0, st>>>(d_pool, n, m->S, nullptr, tauD, d_corner, nullptr, d_status, d_delta, counters,
+                                                        counters + 1, stats, args);
+    m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    unsigned long long sv[4];
+    PBVI_CUDA(cudaMemcpyAsync(sv, stats, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    PBVI_CUDA(cudaStreamSynchronize(st));
+    if (h_stats4)
+        for (int k = 0; k < 4; k++) h_stats4[k] = (long long)sv[k];
+    return PBVI_OK;
 }
 
 extern "C" int pbvi_prune_lp_stats(const pbvi_model* m, int64_t* h_out4) {

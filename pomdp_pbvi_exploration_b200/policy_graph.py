@@ -31,6 +31,24 @@ from .solver import MDPSolverHistory
 from .value_function import ValueFunction
 
 
+def reachable_nodes(successors, roots, mixtures=None) -> np.ndarray:
+    """bool [N]: the nodes a controller can reach from the nodes `roots`, through every edge (an impossible observation's included) and
+    every member of a mixture that an edge names (successor entry N + m)."""
+    succ = np.asarray(successors, dtype=np.int64)
+    N = succ.shape[0]
+    seen = np.zeros(N, dtype=bool)
+    stack = sorted({int(r) for r in np.asarray(roots).reshape(-1)})
+    seen[stack] = True
+    while stack:
+        for t in succ[stack.pop()].tolist():
+            targets = [t] if t < N else mixtures[1][mixtures[0][t - N]:mixtures[0][t - N + 1]].tolist()
+            for v in targets:
+                if not seen[v]:
+                    seen[v] = True
+                    stack.append(v)
+    return seen
+
+
 def reachable_subgraph(actions, successors, roots) -> tuple:
     """
     The part of a controller that can run from the nodes `roots`: returns (kept node indices ascending, their actions, their successors
@@ -39,15 +57,7 @@ def reachable_subgraph(actions, successors, roots) -> tuple:
     """
     act = np.asarray(actions, dtype=np.int64).reshape(-1)
     succ = np.asarray(successors, dtype=np.int64)
-    seen = np.zeros(act.shape[0], dtype=bool)
-    stack = sorted({int(r) for r in np.asarray(roots).reshape(-1)})
-    seen[stack] = True
-    while stack:
-        for t in succ[stack.pop()].tolist():
-            if not seen[t]:
-                seen[t] = True
-                stack.append(t)
-    keep = np.flatnonzero(seen)
+    keep = np.flatnonzero(reachable_nodes(succ, roots))
     renumber = np.full(act.shape[0], -1, dtype=np.int64)
     renumber[keep] = np.arange(len(keep))
     return keep, act[keep], renumber[succ[keep]]
@@ -236,6 +246,210 @@ def match_tuples(node_of: dict, tuples: np.ndarray) -> tuple:
         elif t not in new:
             new[t] = len(new)
     return in_use, np.asarray(list(new), dtype=np.int64).reshape(-1, tuples.shape[1])
+
+
+BPI_COLUMNS = 64                   # columns of one restricted master LP (J_MAX of pbvi_bpi_lp)
+BPI_POOL_BYTES = 2 << 30           # worst-case column pool of one batch of nodes
+BPI_POOL_ROWS = BPI_COLUMNS + 2    # per node: its row, its own row, 63 appended columns and the last one priced (checked, not appended)
+BPI_DROP = 1e-13                   # LP weights below this are dropped before the graph surgery
+
+
+def bpi_lps(dev, W: torch.Tensor, own: torch.Tensor, gamma: float, tau: float, batch: int | None = None) -> dict:
+    """
+    The restricted master LPs of bounded policy iteration for every node, by column generation: node n's LP is
+    max eps s.t. sum_t lambda_t Y_t >= W_n + eps, sum lambda = 1, lambda >= 0 over the columns generated so far, started from its own
+    one-sweep row own[n].  Each round runs `pbvi_bpi_lp` on the batch, then prices every still active node with one `backup_select` at its
+    tangent belief b* (the best tuple t* = argmax_t b* . Y_t), assembles the tuples that are new to the batch (`backup_assemble`, one row
+    per distinct tuple) into the pool and hands each node its t*.  Nodes go in batches of `batch` (default: the pool of a batch stays under
+    BPI_POOL_BYTES); an entry's results depend on its own rows and columns only, so they are bitwise the same for every batch split.
+
+    Returns status int64 [N] (1 not improvable, 2 optimal, 3 budget, 4 numerical), delta / u / mstar float64 [N] (delta_J of the last LP,
+    its verified bound max_s (W_n - sum lambda Y)[s], b* . (W_n - Y_{t*}) of the last check), lam float64 [N, 64], columns int64 [N, 64]
+    (-1 the node's own row, t >= 0 row t of `tuples`, -2 padding), tuples int64 [T, 1 + O] (action, successor nodes), bstar CUDA float64
+    [N, S], stats {rounds, max_columns, lps, pivots, pool_rows} and seconds {lp, select, assemble}.
+    """
+    N, S = W.shape
+    d = W.device
+    if batch is None:
+        batch = max(1, BPI_POOL_BYTES // (BPI_POOL_ROWS * S * 8))
+    out = dict(status=np.zeros(N, np.int64), delta=np.zeros(N), u=np.zeros(N), mstar=np.zeros(N), lam=np.zeros((N, BPI_COLUMNS)),
+               columns=np.full((N, BPI_COLUMNS), -2, np.int64), bstar=torch.zeros((N, S), dtype=torch.float64, device=d))
+    tuple_id = {}
+    stats = dict(rounds=0, max_columns=0, lps=0, pivots=0, pool_rows=0)
+    sec = dict(lp=0.0, select=0.0, assemble=0.0)
+    for lo in range(0, N, batch):
+        hi = min(N, lo + batch)
+        n = hi - lo
+        pool = torch.empty((BPI_POOL_ROWS * n, S), dtype=torch.float64, device=d)
+        pool[:n], pool[n:2 * n] = W[lo:hi], own[lo:hi]
+        P = 2 * n
+        row_tuple = {}                                     # tuple -> pool row
+        tuples_of_row = {}                                 # pool row -> tuple
+        i32 = dict(dtype=torch.int32, device=d)
+        f64 = dict(dtype=torch.float64, device=d)
+        corner = torch.argmax(W[lo:hi] - own[lo:hi], dim=1).to(torch.int32).contiguous()
+        price = torch.full((n,), -1, **i32)
+        cols = torch.full((n, BPI_COLUMNS), -1, **i32)
+        cols[:, 0] = torch.arange(n, 2 * n, **i32)
+        ncols = torch.ones((n,), **i32)
+        bstar = torch.zeros((n, S), **f64)
+        delta, u, mstar = (torch.full((n,), float('nan'), **f64) for _ in range(3))
+        lam = torch.zeros((n, BPI_COLUMNS), **f64)
+        status = torch.full((n,), -1, **i32)
+        while True:
+            t0 = time.perf_counter()
+            st = dev.bpi_lp(pool, n, tau, corner, price, cols, ncols, bstar, delta, u, lam, mstar, status)
+            sec['lp'] += time.perf_counter() - t0
+            stats['rounds'] += 1
+            stats['max_columns'] = max(stats['max_columns'], st['max_columns'])
+            stats['lps'] += st['lps']
+            stats['pivots'] += st['pivots']
+            active = np.flatnonzero(status.cpu().numpy() == -1)
+            if not len(active):
+                break
+            t0 = time.perf_counter()
+            tup = backup_tuples(dev, bstar[torch.as_tensor(active, device=d)], W, gamma)
+            sec['select'] += time.perf_counter() - t0
+            t0 = time.perf_counter()
+            rows, new = np.empty(len(active), np.int64), []
+            for k, t in enumerate(map(tuple, tup.tolist())):
+                if t not in row_tuple:
+                    row_tuple[t] = P + len(new)
+                    tuples_of_row[P + len(new)] = t
+                    new.append(t)
+                rows[k] = row_tuple[t]
+            if new:
+                assert P + len(new) <= pool.shape[0]           # every active node adds at most one column per round
+                nt = np.asarray(new, dtype=np.int64)
+                pool[P:P + len(new)] = dev.backup_assemble(W, gamma, nt[:, 0], nt[:, 1:])
+                P += len(new)
+            price[torch.as_tensor(active, device=d)] = torch.as_tensor(rows, **i32)
+            torch.cuda.synchronize(d)
+            sec['assemble'] += time.perf_counter() - t0
+        stats['pool_rows'] = max(stats['pool_rows'], P)
+        k = ncols.cpu().numpy()
+        c = cols.cpu().numpy()
+        for j in range(n):
+            for q in range(int(k[j])):
+                r = int(c[j, q])
+                if q == 0:
+                    out['columns'][lo + j, q] = -1
+                else:
+                    t = tuples_of_row[r]
+                    out['columns'][lo + j, q] = tuple_id.setdefault(t, len(tuple_id))
+        out['status'][lo:hi] = status.cpu().numpy()
+        out['delta'][lo:hi], out['u'][lo:hi], out['mstar'][lo:hi] = delta.cpu().numpy(), u.cpu().numpy(), mstar.cpu().numpy()
+        out['lam'][lo:hi] = lam.cpu().numpy()
+        out['bstar'][lo:hi] = bstar
+    out['tuples'] = np.asarray(list(tuple_id), dtype=np.int64).reshape(len(tuple_id), -1) if tuple_id else None
+    out['stats'], out['seconds'] = stats, sec
+    return out
+
+
+def successor_distribution(entry: int, N: int, mixtures) -> tuple:
+    """(members, weights) of a successor entry: node t is ([t], [1]), mixture entry N + m its members (a flattened mixture)."""
+    if entry < N:
+        return np.asarray([entry], np.int64), np.ones(1)
+    off, nodes, w = mixtures
+    m = entry - N
+    return nodes[off[m]:off[m + 1]], w[off[m]:off[m + 1]]
+
+
+def combine_members(nodes, weights) -> tuple:
+    """Duplicate members merged (ascending) and the weights renormalised to sum 1."""
+    u, inv = np.unique(np.asarray(nodes, np.int64), return_inverse=True)
+    w = np.bincount(inv, weights=np.asarray(weights, np.float64), minlength=len(u))
+    return u, w / w.sum()
+
+
+def bpi_split(columns, lam, N: int, mixtures, drop: float = BPI_DROP) -> list:
+    """
+    The nodes that replace an improved node: `columns` = [(action, successor entries [O])] of its LP solution, `lam` their weights.
+    Weights below `drop` are dropped and the rest renormalised; per action a (ascending) the node n_a plays a and on o moves to the
+    distribution {sigma_t(o) : a_t = a} with weights lambda_t / c_a (mixture entries flattened into their members, duplicates merged).
+    Returns [(a, c_a, [(members, weights) per o])], the c_a summing to 1.
+    """
+    lam = np.asarray(lam, np.float64)
+    keep = np.flatnonzero(lam >= drop)
+    lam = lam[keep] / lam[keep].sum()
+    cols = [columns[k] for k in keep]
+    acts = np.asarray([a for a, _ in cols], np.int64)
+    out = []
+    for a in np.unique(acts).tolist():
+        idx = np.flatnonzero(acts == a)
+        c = float(lam[idx].sum())
+        O = len(cols[idx[0]][1])
+        edges = []
+        for o in range(O):
+            parts = [successor_distribution(int(cols[k][1][o]), N, mixtures) for k in idx]
+            edges.append(combine_members(np.concatenate([p[0] for p in parts]),
+                                         np.concatenate([p[1] * (lam[k] / c) for p, k in zip(parts, idx)])))
+        out.append((a, c, edges))
+    return out
+
+
+def bpi_assemble(actions, successors, mixtures, splits: dict, redirect: bool) -> tuple:
+    """
+    A graph with the nodes of `splits` ({n: bpi_split(...)}) added.  redirect=False (the graph the start rows are swept on): every
+    split node is appended and no old edge changes.  redirect=True (the improved graph): n_{a_0} of the first action takes n's index and
+    the others are appended, and every edge or mixture member naming a split node n with more than one action goes to the mixture
+    {n_a : c_a} instead (members flattened).  Old mixtures keep their ids (members rewritten when they name such an n); further mixtures
+    are appended, one per distinct distribution.  Returns (actions, successors, mixtures or None, {(n, j): node index of n's j-th split}).
+    """
+    act = np.asarray(actions, np.int64)
+    succ = np.asarray(successors, np.int64)
+    N, O = succ.shape
+    pos, extra = {}, N
+    for n in sorted(splits):
+        for j in range(len(splits[n])):
+            if redirect and j == 0:
+                pos[(n, 0)] = n
+            else:
+                pos[(n, j)] = extra
+                extra += 1
+    N2 = extra
+    sub = {n: (np.asarray([pos[(n, j)] for j in range(len(sp))]), np.asarray([c for _, c, _ in sp]))
+           for n, sp in splits.items() if redirect and len(sp) > 1}
+
+    def substitute(nodes, weights):
+        if not any(int(t) in sub for t in nodes):
+            return nodes, weights
+        parts = [sub[int(t)] if int(t) in sub else (np.asarray([t]), np.ones(1)) for t in nodes]
+        return combine_members(np.concatenate([p[0] for p in parts]), np.concatenate([p[1] * w for p, w in zip(parts, weights)]))
+
+    table, index = [], {}
+    M = 0 if mixtures is None else len(mixtures[0]) - 1
+    for m in range(M):
+        table.append(substitute(*successor_distribution(N + m, N, mixtures)))
+
+    def intern(nodes, weights):
+        key = (tuple(nodes.tolist()), tuple(weights.tolist()))
+        if key not in index:
+            index[key] = len(table)
+            table.append((nodes, weights))
+        return index[key]
+
+    target = np.arange(N)
+    for n in sorted(sub):
+        target[n] = N2 + intern(*sub[n])
+    act2 = np.concatenate([act, np.zeros(N2 - N, np.int64)])
+    succ2 = np.zeros((N2, O), np.int64)
+    succ2[:N] = np.where(succ < N, target[np.minimum(succ, N - 1)], N2 + succ - N)
+    for n in sorted(splits):
+        for j, (a, _, edges) in enumerate(splits[n]):
+            k = pos[(n, j)]
+            act2[k] = a
+            for o, (nodes, weights) in enumerate(edges):
+                nodes, weights = substitute(nodes, weights)
+                succ2[k, o] = int(nodes[0]) if len(nodes) == 1 else N2 + intern(nodes, weights)
+    if not table:
+        return act2, succ2, None, pos
+    off = np.concatenate([[0], np.cumsum([len(t[0]) for t in table])]).astype(np.int64)
+    mix = (off, np.concatenate([t[0] for t in table]).astype(np.int64), np.concatenate([t[1] for t in table]).astype(np.float64))
+    return act2, succ2, mix, pos
+
+
+NO_MIXTURES = (np.zeros(1, np.int64), np.zeros(0, np.int64), np.zeros(0))
 
 
 class ControllerOutcomes:
@@ -543,6 +757,137 @@ class PolicyGraph:
                          shift=hist.shift, seconds=sec)
             all_stats.append(stats)
         return pg, all_stats
+
+    def bounded_improve(self, beliefs=None, iterations: int = 1, eps: float = 1e-6) -> tuple:
+        """
+        Bounded policy iteration (Poupart & Boutilier 2003) on the controller: returns (PolicyGraph, list of per-iteration stats dicts).
+        Needs an evaluated graph (`rows`, `gamma`); graphs with mixtures are accepted.  Each iteration, with W the certified node rows
+        (W <= T_pi W) and a tuple t = (a, sigma(0..O-1)) a node that plays a and moves to node sigma(o), with row Y_t = backup_assemble(W, t):
+
+          1. LP: for every node n, max eps s.t. sum_t lambda_t Y_t[s] >= W_n[s] + eps at every s, sum lambda = 1, lambda >= 0, over all
+             A * N^O tuples.  In belief space this is delta = max_{b in simplex} min_t b . (W_n - Y_t), eps = -delta: the restricted LP
+             of `pbvi_prune_lp` with columns Y_t as competitors, generated by `bpi_lps`.  J starts with n's own one-sweep row
+             (T_pi W)_n >= W_n (for a node with mixture edges the mixed sweep's row, not a deterministic tuple) and the seed corner
+             argmax_s (W_n - Y_own)[s].  Pricing: at the LP's tangent belief b* the best column over all tuples is the point-based backup
+             at b* (one `backup_select` row), and m* = b* . (W_n - Y_t*) <= delta <= delta_J.  The search stops when m* > -tau (n cannot
+             be improved by more than tau; b* is its tangent belief), when m* >= delta_J - tau (the LP is optimal), or at 64 columns or
+             the pivot budget (the last LP stands).  n is improved when the last LP's verified bound u = max_s (W_n - sum lambda Y_J)[s]
+             is < -tau, with tau = 1e-9 * max(1, max |W|, max |T_pi W|).
+          2. Surgery (`bpi_split`, `bpi_assemble`): weights below 1e-13 are dropped; per action a of the solution, c_a = the weight of
+             its columns and n_a plays a and on o moves to the mixture {sigma_t(o) : a_t = a} with weights lambda_t / c_a (the own
+             column contributes n's own successor entries, mixtures flattened).  X_{n_a} = one mixed sweep of these edges over the old
+             rows W (`controller_evaluate_mixed` on a graph with the n_a appended).  n_{a_0} takes n's index and the others are appended,
+             and edges into n (mixture members naming n too) go to the mixture {n_a : c_a} -- only if `mixture_rows` verifies
+             sum_a c_a X_{n_a} - W_n > tau / 2 at every state; otherwise n stays as it was.  With one action no mixture is needed.
+             The graph grows by at most (distinct actions of the solution - 1) nodes per improved node: that is the bound of BPI here.
+          3. `evaluate(gamma, eps)` from X (W on the old nodes, X_{n_a} on the new), with its certificate.
+          4. Only the nodes reachable from the argmax nodes of b0 and `beliefs`, through edges and mixture members, are kept
+             (`reachable_nodes`, `compact_graph`).
+
+        Why the bound does not fall: old nodes keep W, and an edge n -> mixture whose row is >= W_n + tau / 2 only raises (T' X)_p, by
+        non-negative RTO and monotone rounding.  Each n_a's edges name old rows, or improved nodes' mixtures that lie above them.  So
+        X <= T' X in exact arithmetic, the new controller's value is >= X, and at every belief max_n X_n . b >= the old value.  The
+        certificate of `evaluate` absorbs rounding, so what a caller can see is at most a fall by its shift.
+
+        Stats per iteration: nodes_before, nodes_after, improved, not_improvable, budget, numerical, failed (improvable but not
+        verified), unchanged (improvable, but the LP's solution is the node itself: its own action on its own edges, which only the start
+        row would change; such nodes are left as they are and do not count as improved), mixtures, nnz, lp_rounds, max_columns, pivots, pool_rows, value_b0 (certified), shift and seconds {lp, select, assemble,
+        build, evaluate, prune}.  An iteration that improves no node returns the graph unchanged and ends the loop.
+        """
+        self._require_rows()
+        if self.gamma is None:
+            raise ValueError('bounded_improve needs the gamma of evaluate: call evaluate(gamma) first')
+        m, gamma = self.model, self.gamma
+        dev = m.device
+        d = dev.device
+        B = belief_rows(m, m.start_probabilities)
+        if beliefs is not None:
+            B = torch.cat([B, belief_rows(m, beliefs)])
+        pg, all_stats = self, []
+        for _ in range(int(iterations)):
+            W, N = pg.rows, len(pg)
+            act = torch.as_tensor(pg.actions, dtype=torch.int32, device=d)
+            succ = torch.as_tensor(pg.successors, dtype=torch.int32, device=d).contiguous()
+            own = dev.controller_evaluate_mixed(W, gamma, act, succ, pg.mixtures or NO_MIXTURES, float('inf'), 1)[0]
+            tau = 1e-9 * max(1.0, float(torch.max(torch.abs(W))), float(torch.max(torch.abs(own))))
+            sol = bpi_lps(dev, W, own, gamma, tau)
+            sec = dict(sol['seconds'])
+            t0 = time.perf_counter()
+            status = sol['status']
+            nxt, splits, ok, unchanged = pg._bpi_start_graph(sol, tau)
+            st = dict(nodes_before=N, improved=len(ok), not_improvable=int(np.sum(status == 1)), budget=int(np.sum(status == 3)),
+                      numerical=int(np.sum(status == 4)), failed=len(splits) - len(ok), unchanged=unchanged,
+                      lp_rounds=sol['stats']['rounds'], max_columns=sol['stats']['max_columns'], pivots=sol['stats']['pivots'],
+                      pool_rows=sol['stats']['pool_rows'])
+            if nxt is None:
+                sec.update(build=time.perf_counter() - t0, evaluate=0.0, prune=0.0)
+                st.update(nodes_after=N, mixtures=0 if pg.mixtures is None else len(pg.mixtures[0]) - 1,
+                          nnz=0 if pg.mixtures is None else len(pg.mixtures[1]), value_b0=float(pg.value(B[:1])[0][0]), shift=0.0,
+                          seconds=sec)
+                all_stats.append(st)
+                break
+            sec['build'] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            rows, hist = nxt.evaluate(gamma, eps)
+            sec['evaluate'] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            roots = dev.max_values(B, rows)[1].cpu().numpy()
+            seen = reachable_nodes(nxt.successors, roots, nxt.mixtures)
+            keep, k_act, k_succ, k_mix = compact_graph(nxt.actions, nxt.successors, np.where(seen, np.arange(len(nxt)), -1), nxt.mixtures)
+            pg = PolicyGraph(m, k_act, k_succ, rows=rows[torch.as_tensor(keep, device=d)], mixtures=k_mix)
+            pg.gamma = gamma
+            sec['prune'] = time.perf_counter() - t0
+            st.update(nodes_after=len(pg), mixtures=0 if k_mix is None else len(k_mix[0]) - 1, nnz=0 if k_mix is None else len(k_mix[1]),
+                      value_b0=float(pg.value(B[:1])[0][0]), shift=hist.shift, seconds=sec)
+            all_stats.append(st)
+        return pg, all_stats
+
+    def _bpi_start_graph(self, sol: dict, tau: float) -> tuple:
+        """
+        Steps 2 of `bounded_improve` on the LP solutions `sol` of `bpi_lps`: returns (the improved graph without rows and with `_initial`
+        = X, or None when no node is improved; {n: split} of the improvable nodes; the verified nodes; the nodes whose LP solution is
+        the node itself).  A node is improvable when its LP stopped optimal or at the budget with u < -tau; a split that plays the
+        node's own action on the node's own edges (its solution is its own column) changes nothing and is left out.
+        """
+        m, gamma, W, N = self.model, self.gamma, self.rows, len(self)
+        dev, d = m.device, m.device.device
+        status = sol['status']
+        improvable = np.flatnonzero(((status == 2) | (status == 3)) & (sol['u'] < -tau))
+        splits, unchanged = {}, 0
+        for n in improvable.tolist():
+            cols, columns = sol['columns'][n], []
+            for c in cols[cols > -2].tolist():
+                t = sol['tuples'][c] if c >= 0 else None
+                columns.append((int(self.actions[n]), self.successors[n]) if c == -1 else (int(t[0]), t[1:]))
+            sp = bpi_split(columns, sol['lam'][n][:len(columns)], N, self.mixtures)
+            if len(sp) == 1 and sp[0][0] == self.actions[n] and all(
+                    np.array_equal(nodes, own[0]) and np.array_equal(w, own[1])
+                    for (nodes, w), own in zip(sp[0][2], (combine_members(*successor_distribution(int(e), N, self.mixtures))
+                                                          for e in self.successors[n]))):
+                unchanged += 1
+                continue
+            splits[n] = sp
+        if not splits:
+            return None, splits, [], unchanged
+        a_i, s_i, mix_i, pos_i = bpi_assemble(self.actions, self.successors, self.mixtures, splits, redirect=False)
+        X0 = torch.cat([W, torch.zeros((len(a_i) - N, W.shape[1]), dtype=torch.float64, device=d)])
+        Xi = dev.controller_evaluate_mixed(X0, gamma, a_i, s_i, mix_i or NO_MIXTURES, float('inf'), 1)[0]
+        order = sorted(splits)
+        off = np.concatenate([[0], np.cumsum([len(splits[n]) for n in order])]).astype(np.int64)
+        members = np.asarray([pos_i[(n, j)] for n in order for j in range(len(splits[n]))], np.int64)
+        weights = np.asarray([c for n in order for _, c, _ in splits[n]], np.float64)
+        Z = mixture_rows(Xi, (off, members, weights))
+        good = ((Z - W[torch.as_tensor(order, device=d)]) > tau / 2).all(dim=1).cpu().numpy()
+        ok = [n for n, g in zip(order, good.tolist()) if g]
+        if not ok:
+            return None, splits, ok, unchanged
+        a_f, s_f, mix_f, pos_f = bpi_assemble(self.actions, self.successors, self.mixtures, {n: splits[n] for n in ok}, redirect=True)
+        X = torch.cat([W, torch.zeros((len(a_f) - N, W.shape[1]), dtype=torch.float64, device=d)])
+        dst, src = zip(*[(k, pos_i[key]) for key, k in pos_f.items()])
+        X[torch.as_tensor(dst, device=d)] = Xi[torch.as_tensor(src, device=d)]
+        nxt = PolicyGraph(m, a_f, s_f, mixtures=mix_f)
+        nxt._initial = X
+        return nxt, splits, ok, unchanged
 
     def prune_dominated(self) -> 'PolicyGraph':
         """
