@@ -37,6 +37,27 @@ sum|t| is evaluated in float64 with non-negative terms (relative error below n u
 
 Every computation runs on the support of each belief only, so a belief with 50 non-zero states over S = 20 000 costs 50 R A O V
 multiply-adds.  This module imports nothing from the product package.
+
+Upper bounds (pbvi_sawtooth / pbvi_sawtooth_lists, pbvi_upper_backup, pbvi_gap_trial_step, pbvi_hsvi_level).  Each stage is exact given
+its float64 inputs: the successor rows q and masses P(o|b,a) are the device's own (pinned elsewhere: rows bitwise the reference's update,
+masses bitwise NumPy's pairwise sum), and so is every value a later stage reads.  The results are intervals [lo, hi] that hold every
+float64 evaluation; a minimum or maximum of values known to lie in intervals lies in the interval of the endpoints' minima / maxima, so
+the intervals do not depend on which term a device reduction picks.
+
+  sawtooth term (x_i = v0 + (v_i - d_i) m_i, v0 = q . corner, d_i = b_i . corner, m_i = min_{s: b_i[s] > 0} q[s] / b_i[s]):  m_i is a
+      minimum of correctly rounded quotients, and rounding is monotone, so the device's m_i is the float64 minimum of the float64
+      quotients -- NumPy's, bit for bit, overflow to inf included -- and enters as an input.  A q . corner term passes the v0 dot (n_0
+      roundings) and the final addition: n_0 + 1; v_i m_i passes the subtraction, the product and the addition: 3; a b_i . corner
+      term the d_i dot (n_i), then the same 3: n_i + 3.  With n = n_0 + n_i + 1 that is <= n + 2 -> (n + 3) u, C_SAW = 3.  An absolute
+      (subnormal) error of the d_i dot is multiplied by m_i later: M = max(1, m_i).  The v0 term alone is the n = n_0 case.
+  Q (rb + gamma sum_{o: P > 0} P y_o, rb = b . Rbar_a, y_o = min(max_v F_v . q, saw(q)) known in [y_lo, y_hi]):  Q is increasing in
+      every y_o (P >= 0, gamma > 0), so the exact Q at the device's y lies in [Q(y_lo), Q(y_hi)].  Its float64 evaluation: an rb term
+      passes the n_r dot roundings and the final addition; a P y term the product, O_p - 1 additions, gamma, the final addition: with
+      n = n_r + O_p terms both are <= n + 2 -> C_Q = 3 (sum|t| with |y| <= max(|y_lo|, |y_hi|)).
+  excess e = P ((U - L) - theta):  three roundings per term, n = 3 terms (P U, P L, P theta) -> (n + 1) u, C_EXCESS = 1; e is increasing
+      in U and decreasing in L, so its exact value at the device's U, L lies in [P (U_lo - L_hi - theta), P (U_hi - L_lo - theta)].
+  sampled o* (cdf_j = (sum_{o <= j} w_o) / W, w = max(e, 0), sequential sums, one division):  with w in [w_lo, w_hi] the running sums
+      lie within (O + 1) (u + u_ld) of [cumsum w_lo, cumsum w_hi], and the quotient within one more rounding.
 """
 from __future__ import annotations
 
@@ -54,6 +75,9 @@ ABS_SLACK = 1.0 + 1e-6            # sum|t| is itself evaluated in float64
 C_SCORE = 3
 C_VALUE = 3
 C_GER = 3
+C_SAW = 3
+C_Q = 3
+C_EXCESS = 1
 
 
 def _bound(n, abs_sum, c, scale):
@@ -221,6 +245,139 @@ def ger_eps(beliefs: np.ndarray, successors: np.ndarray, alpha_b: np.ndarray, r_
 
 
 # --------------------------------------------------------------------------------------------------------------------------------
+# Upper bounds
+# --------------------------------------------------------------------------------------------------------------------------------
+def _dots(rows: np.ndarray, vec: np.ndarray):
+    """rows . vec in longdouble, sum |row[s] vec[s]| and the number of non-zero products, per row."""
+    prod_abs = np.abs(rows) * np.abs(vec)[None, :]
+    exact = rows.astype(LD) @ vec.astype(LD)
+    return exact, prod_abs.sum(axis=1), np.count_nonzero(prod_abs, axis=1).astype(np.float64)
+
+
+def sawtooth(corner: np.ndarray, stored_rows: np.ndarray, stored_vals: np.ndarray, queries: np.ndarray):
+    """
+    The sawtooth upper bound of each query (finite, non-negative rows) over the stored pairs: (lo, hi) longdouble [n_q] that hold
+    min(v0, min_i x_i) for every float64 evaluation (module docstring, C_SAW).  A term whose m_i overflows to inf in float64 is +inf or
+    -inf by the sign of its scale (and either, or skipped as NaN, when that sign is not certain).
+    """
+    queries = np.atleast_2d(queries)
+    v0, v0abs, n0 = _dots(queries, corner)
+    lo = v0 - _bound(n0, v0abs, C_SAW, 1.0).astype(LD)
+    hi = v0 + _bound(n0, v0abs, C_SAW, 1.0).astype(LD)
+    for bi, vi in zip(np.atleast_2d(stored_rows), np.atleast_2d(stored_vals).reshape(-1)):
+        sup = np.flatnonzero(bi > 0)
+        if sup.size == 0:
+            m = np.full(len(queries), np.inf)
+        else:
+            with np.errstate(over='ignore', under='ignore'):
+                m = np.min(queries[:, sup] / bi[sup], axis=1)                     # the device's minimum, bit for bit
+        d, dabs, ni = _dots(bi[None, :], corner)
+        sc = LD(vi) - d[0]
+        sc_bound = _bound(ni[0], dabs[0], C_SAW, 1.0)
+        fin = np.isfinite(m)
+        mf = np.where(fin, m, 0.0)
+        x = v0 + sc * mf.astype(LD)
+        tabs = v0abs + (abs(vi) + dabs[0]) * mf
+        e = _bound(n0 + ni[0] + 1, tabs, C_SAW, np.maximum(1.0, mf)).astype(LD)
+        t_lo, t_hi = x - e, x + e
+        if not fin.all():
+            pos = sc > LD(sc_bound)
+            neg = sc < -LD(sc_bound)
+            t_lo = np.where(fin, t_lo, LD(np.inf) if pos else LD(-np.inf))
+            t_hi = np.where(fin, t_hi, LD(-np.inf) if neg else LD(np.inf))
+        lo = np.minimum(lo, t_lo)
+        hi = np.minimum(hi, t_hi)
+    return lo, hi
+
+
+def max_scores(rows: np.ndarray, alphas: np.ndarray):
+    """(lo, hi) longdouble [n] holding max_v rows . alpha_v for every float64 evaluation (pbvi's few-rows and plain score kernels)."""
+    ex, bd, _ = plain_scores(np.atleast_2d(rows), alphas)
+    bd = bd.astype(LD)
+    return np.max(ex - bd, axis=1), np.max(ex + bd, axis=1)
+
+
+def upper_values(rows: np.ndarray, fib_rows, corner, stored_rows, stored_vals):
+    """(lo, hi) of min(max_v F_v . q, sawtooth(q)) per row (no FIB part when fib_rows is None)."""
+    lo, hi = sawtooth(corner, stored_rows, stored_vals, rows)
+    if fib_rows is not None:
+        flo, fhi = max_scores(rows, fib_rows)
+        lo, hi = np.minimum(lo, flo), np.minimum(hi, fhi)
+    return lo, hi
+
+
+def q_values(beliefs: np.ndarray, rbar: np.ndarray, gamma: float, mass: np.ndarray, y_lo: np.ndarray, y_hi: np.ndarray):
+    """
+    (lo, hi) longdouble [n, A] holding Q[b,a] = b . Rbar_a + gamma sum_{o: P > 0} P(o|b,a) y[b,a,o] for every float64 evaluation at
+    every y in [y_lo, y_hi] (C_Q).  mass [n, A, O] are the device's masses; y is read only where they are positive.
+    """
+    n, A, O = mass.shape
+    live = mass > 0
+    rb = beliefs.astype(LD) @ rbar.astype(LD)                                           # [n, A]
+    rb_abs = np.abs(beliefs) @ np.abs(rbar)
+    n_r = np.stack([np.count_nonzero(beliefs * rbar[:, a][None, :], axis=1) for a in range(A)], axis=1).astype(np.float64)
+    g = LD(gamma)
+    p = np.where(live, mass, 0.0)
+    ylo = np.where(live, y_lo, LD(0))
+    yhi = np.where(live, y_hi, LD(0))
+    q_lo = rb + g * np.sum(p.astype(LD) * ylo, axis=2)
+    q_hi = rb + g * np.sum(p.astype(LD) * yhi, axis=2)
+    ymag = np.maximum(np.abs(ylo), np.abs(yhi)).astype(np.float64)
+    tabs = rb_abs + abs(gamma) * np.sum(p * ymag, axis=2)
+    e = _bound(n_r + np.count_nonzero(live, axis=2), tabs, C_Q, max(1.0, abs(gamma))).astype(LD)
+    return q_lo - e, q_hi + e
+
+
+def upper_q(beliefs, rbar, gamma: float, successors, mass, fib_rows, corner, stored_rows, stored_vals, want_cur: bool = True):
+    """
+    The upper-bound backup (pbvi_upper_backup) from the device's successor rows [n, A, O, S] and masses [n, A, O]: a dict of longdouble
+    intervals  Q [n, A],  u = max_a Q [n],  cur = min(max_v F_v . b, sawtooth(b)) [n],  and y [n, A, O] (NaN where P = 0).
+    """
+    n, A, O = mass.shape
+    live = mass > 0
+    y_lo = np.full((n, A, O), LD(np.nan))
+    y_hi = np.full((n, A, O), LD(np.nan))
+    if live.any():
+        y_lo[live], y_hi[live] = upper_values(successors[live], fib_rows, corner, stored_rows, stored_vals)
+    q_lo, q_hi = q_values(beliefs, rbar, gamma, mass, y_lo, y_hi)
+    out = dict(Q=(q_lo, q_hi), u=(np.max(q_lo, axis=1), np.max(q_hi, axis=1)), y=(y_lo, y_hi))
+    if want_cur:
+        out['cur'] = upper_values(beliefs, fib_rows, corner, stored_rows, stored_vals)
+    return out
+
+
+def excess(mass, U, L, theta: float):
+    """(lo, hi) of e = P ((U - L) - theta) for every float64 evaluation at every U in U = (lo, hi) and L in L = (lo, hi) (C_EXCESS);
+    NaN where P = 0."""
+    live = mass > 0
+    p = np.where(live, mass, 0.0)
+    u_lo, u_hi = (np.where(live, x, LD(0)) for x in U)
+    l_lo, l_hi = (np.where(live, x, LD(0)) for x in L)
+    pl, th = p.astype(LD), LD(theta)
+    tabs = p * (np.maximum(np.abs(u_lo), np.abs(u_hi)) + np.maximum(np.abs(l_lo), np.abs(l_hi)) + abs(theta)).astype(np.float64)
+    e = _bound(3, tabs, C_EXCESS, 1.0).astype(LD)
+    lo = np.where(live, pl * (u_lo - l_hi - th) - e, LD(np.nan))
+    hi = np.where(live, pl * (u_hi - l_lo - th) + e, LD(np.nan))
+    return lo, hi
+
+
+def gap_step(successors, mass, fib_rows, corner, stored_rows, stored_vals, lower_rows, theta: float):
+    """
+    One gap-trial level at the chosen actions (pbvi_gap_trial_step): successors [K, O, S] and masses [K, O] of b_k under a*_k.  Returns
+    a dict of longdouble intervals U [K, O] (upper value of the successor), L [K, O] (max_n X_n . q) and e [K, O] (the excess); all three
+    NaN where P = 0.
+    """
+    K, O = mass.shape
+    live = mass > 0
+    U = [np.full((K, O), LD(np.nan)) for _ in range(2)]
+    L = [np.full((K, O), LD(np.nan)) for _ in range(2)]
+    if live.any():
+        U[0][live], U[1][live] = upper_values(successors[live], fib_rows, corner, stored_rows, stored_vals)
+        L[0][live], L[1][live] = max_scores(successors[live], lower_rows)
+    return dict(U=tuple(U), L=tuple(L), e=excess(mass, U, L, theta))
+
+
+# --------------------------------------------------------------------------------------------------------------------------------
 # The contract
 # --------------------------------------------------------------------------------------------------------------------------------
 def check_argmax(exact, bound, picked, no_terms=None, what='argmax'):
@@ -266,6 +423,106 @@ def check_close(got, exact, bound, what='value'):
         i = tuple(np.argwhere(bad)[0])
         raise AssertionError(f'{what}: entry {i} is {float(err[i]):.3e} from the exact value {float(exact[i]):.17g} '
                              f'(bound {float(bound[i]):.3e}, worst ratio {float(np.nanmax(err / np.maximum(bound, 1e-320))):.3g})')
+
+
+def check_interval(got, interval, what='value'):
+    """lo <= got <= hi entrywise; NaN intervals (an impossible observation) take NaN only."""
+    lo, hi = interval
+    got = np.asarray(got, dtype=np.float64)
+    gl = got.astype(LD)
+    nan = np.isnan(lo)
+    bad = np.where(nan, ~np.isnan(got), ~((lo <= gl) & (gl <= hi)))
+    if bad.any():
+        i = tuple(np.argwhere(bad)[0])
+        raise AssertionError(f'{what}: entry {i} is {got[i]!r}, outside [{float(lo[i])!r}, {float(hi[i])!r}] '
+                             f'(width {float(hi[i] - lo[i]):.3e})')
+
+
+def as_center(interval):
+    """(center, half width) of an interval: the (exact, bound) pair `check_argmax` takes."""
+    lo, hi = interval
+    return (lo + hi) / 2, ((hi - lo) / 2).astype(np.float64) * ABS_SLACK
+
+
+def check_interval_argmax(interval, picked, valid=None, what='argmax'):
+    """
+    A first-argmax over the valid entries of the last axis, each known to lie in its interval: `picked` is valid and not certainly below
+    another entry; where one entry lies certainly above every other valid entry, `picked` is that entry.  Returns the decided rows.
+    """
+    lo, hi = interval
+    picked = np.asarray(picked, dtype=np.int64)
+    valid = np.ones(lo.shape, bool) if valid is None else valid
+    lo = np.where(valid, lo, LD(-np.inf))
+    hi = np.where(valid, hi, LD(-np.inf))
+    rows = np.argwhere(valid.any(axis=-1))
+    decided = np.zeros(picked.shape, bool)
+    for i in map(tuple, rows):
+        p = picked[i]
+        assert 0 <= p < lo.shape[-1] and valid[i][p], f'{what}: row {i} picked {p}, not a valid entry'
+        assert hi[i][p] >= np.max(lo[i]), f'{what}: row {i} picked {p}, certainly below entry {int(np.argmax(lo[i]))}'
+        j = int(np.argmax(lo[i]))
+        others = np.delete(hi[i], j)
+        if others.size == 0 or lo[i][j] > np.max(others):
+            decided[i] = True
+            assert p == j, f'{what}: row {i} picked {p}, entry {j} is certainly the largest'
+    return decided
+
+
+def check_gap_choice(e, picked, what='o*'):
+    """o* of the argmax rule: the first argmax of e over {e > 0}, -1 when no excess is positive (e = (lo, hi), NaN: impossible)."""
+    lo, hi = e
+    picked = np.asarray(picked, dtype=np.int64)
+    pos_sure = lo > 0                                           # NaN > 0 is False
+    pos_maybe = hi > 0
+    none = picked < 0
+    bad = none & pos_sure.any(axis=-1)
+    assert not bad.any(), f'{what}: rows {np.flatnonzero(bad)[:5]} picked -1 with a certainly positive excess'
+    bad = ~none & ~pos_maybe.any(axis=-1)
+    assert not bad.any(), f'{what}: rows {np.flatnonzero(bad)[:5]} picked an observation with no excess that may be positive'
+    decided = np.where(none, ~pos_maybe.any(axis=-1), False)
+    live = np.flatnonzero(~none)
+    if live.size:
+        decided[live] = check_interval_argmax((lo[live], hi[live]), picked[live], pos_maybe[live], what=what)
+    return decided
+
+
+def check_sampled_choice(e, uniforms, picked, what='sampled o*'):
+    """
+    o* of the sampled rule (NumPy's searchsorted(cdf, u, 'right') over w = max(e, 0), capped at the last positive weight): where every
+    excess has a certain sign and every cdf edge lies certainly on one side of u, `picked` is the exact pick.  Elsewhere `picked` is an
+    observation whose excess may be positive (or -1 as `check_gap_choice` allows).  Returns the decided rows.
+    """
+    lo, hi = e
+    K, O = lo.shape
+    picked = np.asarray(picked, dtype=np.int64)
+    decided = np.zeros(K, bool)
+    g = LD((O + 1) * (U + U_LD))
+    for k in range(K):
+        l, h = lo[k], hi[k]
+        poss = ~np.isnan(l)
+        if not (h[poss] > 0).any():
+            assert picked[k] == -1, f'{what}: trial {k} picked {picked[k]} with no excess that may be positive'
+            decided[k] = True
+            continue
+        if picked[k] >= 0:
+            assert poss[picked[k]] and h[picked[k]] > 0, f'{what}: trial {k} picked {picked[k]}, whose excess cannot be positive'
+        else:
+            assert not (l[poss] > 0).any(), f'{what}: trial {k} picked -1 with a certainly positive excess'
+        if not np.all((l[poss] > 0) | (h[poss] <= 0)):
+            continue
+        w_lo = np.where(poss & (l > 0), l, LD(0))
+        w_hi = np.where(poss & (h > 0), h, LD(0))
+        r_lo, r_hi = np.cumsum(w_lo) * (1 - g), np.cumsum(w_hi) * (1 + g)
+        c_lo = r_lo / r_hi[-1] * (1 - 2 * LD(U))
+        c_hi = np.minimum(r_hi / r_lo[-1] * (1 + 2 * LD(U)), LD(1))
+        uk = LD(uniforms[k])
+        below, above = c_hi <= uk, c_lo > uk
+        if not np.all(below | above):
+            continue
+        want = min(int(np.sum(below)), int(np.flatnonzero(w_hi > 0)[-1]))
+        decided[k] = True
+        assert picked[k] == want, f'{what}: trial {k} picked {picked[k]}, the exact draw at u = {uniforms[k]!r} is {want}'
+    return decided
 
 
 def check_backup(reach, rto, rbar, gamma: float, beliefs, alphas, vstar, value=None, astar=None, rows=None, sc=None):

@@ -880,6 +880,7 @@ extern "C" int pbvi_sawtooth(pbvi_model* m, const double* d_corner, const double
     PBVI_TAKE(v0, double, (size_t)n_q);
     cudaStream_t st = (cudaStream_t)stream;
     sawtooth_v0_kernel<<<n_q, 256, 0, st>>>(d_corner, d_queries, m->S, v0);
+    m->last_launches = 1;
     PBVI_CUDA(cudaMemcpy2DAsync(terms + n_ub, (size_t)(n_ub + 1) * sizeof(double), v0, sizeof(double), sizeof(double), (size_t)n_q,
                                 cudaMemcpyDeviceToDevice, st));
     if (n_ub > 0) {
@@ -889,10 +890,11 @@ extern "C" int pbvi_sawtooth(pbvi_model* m, const double* d_corner, const double
             const size_t smem = (sizeof(double) + sizeof(int)) * SAW_RANGE + sizeof(double) * (size_t)nq;
             sawtooth_terms_kernel<<<n_ub, 256, smem, st>>>(d_corner, d_ub_beliefs, d_ub_values, n_ub, d_queries + (size_t)q0 * m->S, nq, m->S,
                                                            v0 + q0, terms + (size_t)q0 * (n_ub + 1));
+            m->last_launches++;
         }
     }
     row_min_kernel<<<ceil_div(n_q, 128), 128, 0, (cudaStream_t)stream>>>(terms, n_q, n_ub + 1, d_out);
-    m->last_launches = 3;
+    m->last_launches++;
     PBVI_CUDA(cudaGetLastError());
     return PBVI_OK;
 }
