@@ -86,6 +86,31 @@ PBVI_API int pbvi_backup_select(pbvi_model* m, const double* d_beliefs, int nB, 
 PBVI_API int pbvi_backup_assemble(pbvi_model* m, const double* d_alphas, int nV, double gamma, const int32_t* d_actions,
                          const int32_t* d_vsel, int n, double* d_out, uint64_t* d_hash, void* stream);
 
+/* ---- exact value iteration by incremental pruning (IncrementalPruning_Solver; Cassandra, Littman & Zhang 1997) -------------------
+ * The rows of H V are built as pbvi_backup_assemble builds them, Rbar[s,a] + ((G_0 + G_1) + ...), but as a fold over observations:
+ * pbvi_ip_project gives every G_o, pbvi_ip_cross_sum adds one observation (and, last, Rbar), so a finished row is bitwise
+ * pbvi_backup_assemble of its tuple (a, v_0 .. v_{O-1}).
+ * pbvi_ip_project: d_out [O][nV][S] with d_out[o][v][s] = G_o[s] = gamma * sum_r RTO[s,a,o,r] * alpha_v[reach[s,a,r]] of action a in
+ * pbvi_backup_assemble's order (r ascending, one rounding per operation) and with its zero-RTO skip, which is off at a state whose
+ * Rbar[s,a] is -0.0.  The caller guarantees finite d_alphas [nV][S]; gamma must be finite, 0 <= a < A.  Enqueues, does not synchronise. */
+PBVI_API int pbvi_ip_project(pbvi_model* m, const double* d_alphas, int nV, double gamma, int a, double* d_out, void* stream);
+/* pbvi_ip_cross_sum: d_out[i*ng + j][s] = d_x[i][s] + d_g[j][s] (one __dadd_rn), or, with a >= 0, Rbar[s,a] + (d_x[i][s] + d_g[j][s]).
+ * d_x = NULL means no X (nx is ignored): d_out[j] = d_g[j], or Rbar[s,a] + d_g[j][s] (O = 1).  d_out [nx*ng][S] (rows i-major, j-minor)
+ * must not overlap the inputs; a < A (a < 0: no Rbar).  Enqueues, does not synchronise. */
+PBVI_API int pbvi_ip_cross_sum(pbvi_model* m, const double* d_x, int nx, const double* d_g, int ng, int a, double* d_out, void* stream);
+/* pbvi_ip_residual_lp: how far each row y_i of d_y [ny][S] rises above the max over the rows of d_x [nx][S] (nx >= 1, all rows finite):
+ *   delta_i = max_{b in simplex} min_j b . (y_i - x_j)
+ * by the cutting-plane LP of pbvi_prune_lp (seeded at the corner s maximising y_i[s] - max_j x_j[s]), with only X competing.  Outputs:
+ *   d_u[i]      a verified upper bound u_i = max_s (y_i - sum_q lambda_q x_{J_q})[s] >= delta_i, recomputed in FP64 from the rows
+ *   d_cert_idx [ny][64], d_cert_w [ny][64]   J (rows of X, -1 padded) and lambda (>= 0, summing to 1 up to rounding, 0 padded) of u_i
+ *   d_mstar[i]  a lower bound m*_i = b* . y_i - max_j b* . x_j <= delta_i (up to the rounding of those dot products)
+ *   d_bstar [ny][S]  its belief b* (dense, in the simplex)
+ * Each row keeps the best bounds of its LPs and stops when u_i - m*_i <= tau, or at the 64-competitor or pivot budget (u_i stays a valid
+ * bound: lambda = e_{J_0} of the seed competitor at worst).  h_stats4 (nullable) = {largest competitor set, restricted LPs solved,
+ * simplex pivots, rows stopped by a budget}.  Scratch: (ny + nx) rows of S doubles from the handle's arena.  Synchronises `stream`. */
+PBVI_API int pbvi_ip_residual_lp(pbvi_model* m, const double* d_y, int ny, const double* d_x, int nx, double tau, double* d_u, double* d_mstar,
+                                 double* d_bstar, int32_t* d_cert_idx, double* d_cert_w, int64_t* h_stats4, void* stream);
+
 /* pbvi_controller_sweep: one evaluation sweep of a finite-state controller (PolicyGraph) with n nodes, node i playing d_actions[i] and
  * moving to node d_succ[i][o] on observation o:
  *   d_out[i][s] = Rbar[s,a_i] + ((G_0 + G_1) + ...),  G_o = gamma * sum_r RTO[s,a_i,o,r] * d_in[succ_i[o]][reach[s,a_i,r]]

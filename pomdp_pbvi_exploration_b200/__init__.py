@@ -4,8 +4,8 @@ B200-native PBVI backup engine: a drop-in for the solver of PimLb/POMDP_PBVI_Exp
 Same names as the reference -- `Model`, `Belief`, `BeliefSet`, `AlphaVector`, `ValueFunction`, `PBVI_Solver`,
 `HSVI_Solver`, `FSVI_Solver`, `FSVI_EG_Solver`, `VI_Solver`, `BeliefValueMapping`, `SolverHistory`, `Agent`, `Simulation`,
 `SimulationSet` -- plus certified upper bounds on V* (`FIB_Solver`, `UpperBound`) and finite-state controllers evaluated as
-certified lower bounds (`PolicyGraph`), and a solver that closes the gap between them at b0 (`GapSolver`), none of them in the
-reference, backed by
+certified lower bounds (`PolicyGraph`), a solver that closes the gap between them at b0 (`GapSolver`) and exact value iteration with a
+certified distance to V* (`IncrementalPruning_Solver`), none of them in the reference, backed by
 hand-written sm_100a CUDA kernels in `libpbvi_b200.so` (C ABI: include/pbvi_b200.h).  The library is loaded on first
 device use; without it (or without a CUDA device) the package raises -- there is no CPU fallback.
 """
@@ -22,6 +22,7 @@ _LAZY = {
     'DeviceModel': '_native', 'ShardedBackup': 'parallel', 'ShardedSolveState': 'parallel', 'NativeComm': 'parallel',
     'FIB_Solver': 'bounds', 'UpperBound': 'bounds', 'PolicyGraph': 'policy_graph', 'ControllerOutcomes': 'policy_graph',
     'GapSolver': 'gap_solver', 'GapSolverHistory': 'gap_solver',
+    'IncrementalPruning_Solver': 'incremental_pruning', 'IncrementalPruningHistory': 'incremental_pruning',
 }
 
 

@@ -63,6 +63,9 @@ SIGNATURES = {
     'pbvi_prune_lp_certificates': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_prune_lp_stats': [_P, _P],
     'pbvi_bpi_lp': [_P, _P, c_int, c_int, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P],
+    'pbvi_ip_project': [_P, _P, c_int, c_double, c_int, _P, _P],
+    'pbvi_ip_cross_sum': [_P, _P, c_int, _P, c_int, c_int, _P, _P],
+    'pbvi_ip_residual_lp': [_P, _P, c_int, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth': [_P, _P, _P, _P, c_int, _P, c_int, _P, _P],
     'pbvi_support_lists': [_P, _P, c_int, _P, _P, _P, _P, _P, _P],
     'pbvi_sawtooth_lists': [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int, _P, _P],
@@ -684,6 +687,55 @@ class DeviceModel:
                                          _ptr(ncols), _ptr(bstar), _ptr(delta), _ptr(u), _ptr(lam), _ptr(mstar), _ptr(status),
                                          out.ctypes.data, self._stream))
         return dict(max_columns=int(out[0]), lps=int(out[1]), pivots=int(out[2]), entries=int(out[3]))
+
+    def _finite_rows(self, rows, what: str) -> torch.Tensor:
+        X = self._beliefs(rows)
+        if X.shape[0] and not bool(torch.isfinite(X).all()):
+            raise ValueError(f'{what}: rows must be finite')
+        return X
+
+    def ip_project(self, alphas, gamma: float, action: int) -> torch.Tensor:
+        """The projections of incremental pruning (`pbvi_ip_project`): G [O, nV, S] CUDA float64, G[o, v] = gamma * sum_r RTO[:, a, o, r] *
+        alpha_v[reach[:, a, r]], bitwise the term `backup_assemble` forms for observation o.  The rows must be finite."""
+        al = self._finite_rows(alphas, 'ip_project')
+        if not 0 <= int(action) < self.A:
+            raise ValueError(f'ip_project: action must lie in [0, {self.A})')
+        out = torch.empty((self.O, al.shape[0], self.S), dtype=torch.float64, device=self.device)
+        self._call(self._lib.pbvi_ip_project(self._h, _ptr(al), al.shape[0], float(gamma), int(action), _ptr(out), self._stream))
+        return out
+
+    def ip_cross_sum(self, x, g, action: int = -1) -> torch.Tensor:
+        """The cross sum of incremental pruning (`pbvi_ip_cross_sum`): rows x_i + g_j [nx * ng, S] (i-major), with action >= 0 Rbar[:, a] +
+        (x_i + g_j); x = None gives g_j (or Rbar[:, a] + g_j)."""
+        G = self._beliefs(g)
+        X = None if x is None else self._beliefs(x)
+        if not -1 <= int(action) < self.A:
+            raise ValueError(f'ip_cross_sum: action must lie in [-1, {self.A})')
+        nx = 1 if X is None else X.shape[0]
+        out = torch.empty((nx * G.shape[0], self.S), dtype=torch.float64, device=self.device)
+        self._call(self._lib.pbvi_ip_cross_sum(self._h, _ptr(X), 0 if X is None else X.shape[0], _ptr(G), G.shape[0], int(action), _ptr(out),
+                                               self._stream))
+        return out
+
+    def ip_residual_lp(self, new_rows, old_rows, tau: float) -> dict:
+        """How far each row y_i of `new_rows` rises above the rows of `old_rows` (`pbvi_ip_residual_lp`), delta_i = max_b min_j b . (y_i - x_j):
+        {u [ny] (verified upper bound), mstar [ny] (lower bound), bstar [ny, S], cert_idx [ny, 64] int32, cert_w [ny, 64], stats} as CUDA
+        tensors, stats = {max_competitors, lps, pivots, budget_rows}.  Rows must be finite and old_rows non-empty.  Synchronises."""
+        Y, X = self._finite_rows(new_rows, 'ip_residual_lp'), self._finite_rows(old_rows, 'ip_residual_lp')
+        if X.shape[0] < 1:
+            raise ValueError('ip_residual_lp: need at least one old row')
+        if not (tau >= 0.0 and np.isfinite(tau)):
+            raise ValueError('ip_residual_lp: tau must be finite and >= 0')
+        ny = Y.shape[0]
+        u, mstar = (torch.empty((ny,), dtype=torch.float64, device=self.device) for _ in range(2))
+        bstar = torch.empty((ny, self.S), dtype=torch.float64, device=self.device)
+        idx = torch.empty((ny, 64), dtype=torch.int32, device=self.device)
+        w = torch.empty((ny, 64), dtype=torch.float64, device=self.device)
+        st = np.zeros(4, dtype=np.int64)
+        self._call(self._lib.pbvi_ip_residual_lp(self._h, _ptr(Y), ny, _ptr(X), X.shape[0], float(tau), _ptr(u), _ptr(mstar), _ptr(bstar),
+                                                 _ptr(idx), _ptr(w), st.ctypes.data, self._stream))
+        return dict(u=u, mstar=mstar, bstar=bstar, cert_idx=idx, cert_w=w,
+                    stats=dict(max_competitors=int(st[0]), lps=int(st[1]), pivots=int(st[2]), budget_rows=int(st[3])))
 
     def sawtooth(self, corner, ub_beliefs, ub_values, queries) -> torch.Tensor:
         c, q = _f64(corner, self.device), self._beliefs(queries)

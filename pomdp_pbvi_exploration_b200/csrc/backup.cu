@@ -270,28 +270,63 @@ __device__ __forceinline__ double block_sum_256(double v, double* sh) {
 // Coherent: the alpha rows were written earlier in the same launch (controller_evaluate_kernel), so they are gathered with ld.global.cg
 // instead of through the read-only data cache, which is not kept coherent with writes during a launch.
 // Mixed: a selection v >= nRows names row v - nRows of `mixRows` (the mixture rows of controller_evaluate_kernel<true>).
+// observation_term is G_o at state s for the row `arow` (rtoO = the RTO slice of observation o); pbvi_ip_project writes exactly these terms.
+__device__ __forceinline__ bool zero_term_skip(bool skipZero, double rb) { return skipZero && !(rb == 0.0 && signbit(rb)); }
+
+template <bool Coherent = false>
+__device__ __forceinline__ double observation_term(const double* arow, const double* rtoO, const int32_t* __restrict__ reach,
+                                                   int R, double gamma, int s, bool skip) {
+    double inner = 0.0;
+    for (int r = 0; r < R; r++) {
+        const size_t k = (size_t)s * R + r;
+        const double w = rtoO[k];
+        const double prod = (skip && w == 0.0) ? 0.0 : __dmul_rn(w, Coherent ? __ldcg(arow + reach[k]) : arow[reach[k]]);
+        inner = (r == 0) ? prod : __dadd_rn(inner, prod);
+    }
+    return __dmul_rn(gamma, inner);
+}
+
 template <bool Coherent = false, bool Mixed = false>
 __device__ __forceinline__ double alpha_a_entry(const double* __restrict__ alphas, int S, int R, int O, const int* vsel,
                                                 const int32_t* __restrict__ reach, const double* __restrict__ rtoA,
                                                 const double* __restrict__ rbarA, double gamma, int s, bool skipZero,
                                                 const double* mixRows = nullptr, int nRows = 0) {
     const double rb = rbarA[s];
-    const bool skip = skipZero && !(rb == 0.0 && signbit(rb));
+    const bool skip = zero_term_skip(skipZero, rb);
     double tot = 0.0;
     for (int o = 0; o < O; o++) {
         const double* arow = (Mixed && vsel[o] >= nRows) ? mixRows + (size_t)(vsel[o] - nRows) * S : alphas + (size_t)vsel[o] * S;
-        const double* rto = rtoA + (size_t)o * S * R;
-        double inner = 0.0;
-        for (int r = 0; r < R; r++) {
-            const size_t k = (size_t)s * R + r;
-            const double w = rto[k];
-            const double prod = (skip && w == 0.0) ? 0.0 : __dmul_rn(w, Coherent ? __ldcg(arow + reach[k]) : arow[reach[k]]);
-            inner = (r == 0) ? prod : __dadd_rn(inner, prod);
-        }
-        const double term = __dmul_rn(gamma, inner);
+        const double term = observation_term<Coherent>(arow, rtoA + (size_t)o * S * R, reach, R, gamma, s, skip);
         tot = (o == 0) ? term : __dadd_rn(tot, term);
     }
     return __dadd_rn(rb, tot);
+}
+
+// ---- incremental pruning (IncrementalPruning_Solver): the projections G_o of alpha_a_entry, and the left fold over o as cross sums ----
+// out[o][v][s] = observation_term(alpha_v, o) of action a (zero-RTO skip on: the caller's alphas are finite).  grid (S tiles, v slab, o)
+__global__ void __launch_bounds__(256) ip_project_kernel(const double* __restrict__ alphas, int nV, int v0, const int32_t* __restrict__ reach,
+                                                         const double* __restrict__ rtoA, const double* __restrict__ rbarA, double gamma,
+                                                         int S, int R, double* __restrict__ out) {
+    const int s = blockIdx.x * 256 + threadIdx.x;
+    const int v = v0 + blockIdx.y, o = blockIdx.z;
+    if (s >= S) return;
+    const bool skip = zero_term_skip(true, rbarA[s]);
+    out[((size_t)o * nV + v) * S + s] = observation_term(alphas + (size_t)v * S, rtoA + (size_t)o * S * R, reach, R, gamma, s, skip);
+}
+
+// out[i*ng + j][s] = x_i[s] + g_j[s] (g_j alone without x), then rbarA[s] + that when rbarA is given: alpha_a_entry's last additions
+__global__ void __launch_bounds__(256) ip_cross_sum_kernel(const double* __restrict__ x, const double* __restrict__ g, int ng, size_t rows,
+                                                           const double* __restrict__ rbarA, int S, double* __restrict__ out) {
+    const size_t total = rows * (size_t)S;
+    for (size_t e = (size_t)blockIdx.x * 256 + threadIdx.x; e < total; e += (size_t)gridDim.x * 256) {
+        const size_t row = e / S;
+        const int s = (int)(e - row * S);
+        const size_t i = row / ng, j = row - i * ng;
+        double v = g[j * S + s];
+        if (x) v = __dadd_rn(x[i * S + s], v);
+        if (rbarA) v = __dadd_rn(rbarA[s], v);
+        out[e] = v;
+    }
 }
 
 // sets *flag when some entry is NaN or +-inf (the zero-skip of the assemble kernels needs finite alphas)
@@ -1320,6 +1355,46 @@ extern "C" int pbvi_backup_assemble(pbvi_model* m, const double* d_alphas, int n
     PBVI_TRY(enter_call(m, (cudaStream_t)stream));
     m->last_launches = 0;
     return assemble_impl(m, d_alphas, nV, gamma, d_actions, d_vsel, (size_t)m->O, 0, n, d_out, d_hash, (cudaStream_t)stream);
+}
+
+extern "C" int pbvi_ip_project(pbvi_model* m, const double* d_alphas, int nV, double gamma, int a, double* d_out, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_REQUIRE(nV >= 0, "nV must be non-negative");
+    PBVI_REQUIRE(a >= 0 && a < m->A, "action out of range");
+    PBVI_REQUIRE(std::isfinite(gamma), "gamma must be finite (zero-RTO terms are skipped)");
+    m->last_launches = 0;
+    if (nV == 0) return PBVI_OK;
+    PBVI_REQUIRE(d_alphas && d_out, "NULL pointer argument");
+    PBVI_REQUIRE(m->O <= 65535, "too many observations for one launch");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    const int S = m->S, R = m->R;
+    for (int v0 = 0; v0 < nV; v0 += 65535) {
+        ip_project_kernel<<<dim3(ceil_div(S, 256), std::min(65535, nV - v0), m->O), 256, 0, st>>>(
+            d_alphas, nV, v0, m->reachK + (size_t)a * S * R, m->rtoK + (size_t)a * m->O * S * R, m->rbarT + (size_t)a * S, gamma, S, R, d_out);
+        m->last_launches++;
+    }
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_ip_cross_sum(pbvi_model* m, const double* d_x, int nx, const double* d_g, int ng, int a, double* d_out, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_REQUIRE(ng >= 0 && (d_x == nullptr || nx >= 0), "counts must be non-negative");
+    PBVI_REQUIRE(a < m->A, "action out of range");
+    m->last_launches = 0;
+    const size_t rows = (size_t)(d_x ? nx : 1) * (size_t)ng;
+    if (rows == 0) return PBVI_OK;
+    PBVI_REQUIRE(d_g && d_out, "NULL pointer argument");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    const size_t blocks = std::min(ceil_div_sz(rows * (size_t)m->S, 256), (size_t)m->sm_count * 16);
+    ip_cross_sum_kernel<<<(unsigned)blocks, 256, 0, st>>>(d_x, d_g, ng, rows, a >= 0 ? m->rbarT + (size_t)a * m->S : nullptr, m->S, d_out);
+    m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    return PBVI_OK;
 }
 
 extern "C" int pbvi_controller_sweep(pbvi_model* m, const double* d_in, int n, double gamma, const int32_t* d_actions, const int32_t* d_succ,

@@ -155,6 +155,26 @@ __global__ void __launch_bounds__(PL_THREADS) prune_lp_corner_kernel(const doubl
     }
 }
 
+// residual LP seed, block per row y_i of the pool's first rows: the corner s maximising y_i[s] - max_j x_j[s] (lowest s on a tie), its best
+// row of X (pool index off + i1[s]) and that margin, which is m* at b = e_s
+__global__ void __launch_bounds__(PL_THREADS) residual_corner_kernel(const double* __restrict__ A, int S, int off, const double* __restrict__ v1,
+                                                                     const int32_t* __restrict__ i1, int32_t* __restrict__ cornerS,
+                                                                     int32_t* __restrict__ cornerJ, double* __restrict__ bound) {
+    __shared__ double sv[PL_THREADS / 32 + 1];
+    __shared__ int si[PL_THREADS / 32 + 1];
+    const int i = blockIdx.x;
+    const double* a = A + (size_t)i * S;
+    double best = -INFINITY;
+    int bestS = INT_MAX;
+    for (int s = threadIdx.x; s < S; s += PL_THREADS) arg_better(best, bestS, a[s] - v1[s], s);
+    block_argmax(best, bestS, sv, si);
+    if (threadIdx.x == 0) {
+        cornerS[i] = bestS;
+        cornerJ[i] = off + i1[bestS];
+        bound[i] = best;
+    }
+}
+
 // Cutting-plane LP, a block per undecided row (rows handed out by an atomic counter).  Restricted LP in equality form, rows q < k for the
 // competitors J[q], row k the simplex row:
 //     sum_s b_s d_q[s] - delta - t_q = 0,   sum_s b_s = 1,   b, t >= 0,   delta free,   maximise delta       (d_q = (alpha_i - alpha_J[q]) / scl)
@@ -188,6 +208,26 @@ template <typename... T>
 constexpr bool kIsBpi = (false || ... || std::is_same<T, BpiArgs>::value);
 
 __device__ __forceinline__ const BpiArgs& bpi_args(const BpiArgs& a) { return a; }
+
+// The residual LP of incremental pruning (pbvi_ip_residual_lp) is the instantiation whose pack is one ResidualArgs: A is the pool [Y; X]
+// (ny rows of the new set, then the nx rows of the old one), the rows i < ny are tested and only X competes.  A row keeps the best
+// verified bounds over its LPs -- u (with its J / lambda) and m* (with its b*), both valid for any LP -- and stops when u - m* <= tol.
+struct ResidualArgs {
+    int off, nx;                // X = pool rows [off, off + nx)
+    double tol;                 // stop at u - m* <= tol
+    double* u;                  // [ny] verified upper bound on delta_i
+    double* mstar;              // [ny] lower bound b* . y_i - max_j b* . x_j
+    double* bstar;              // [ny, S] its belief (dense)
+    int32_t* certIdx;           // [ny, J_MAX] J of u as rows of X (-1 padded)
+    double* certW;              // [ny, J_MAX] lambda of u (0 padded)
+    double uBest, mBest;        // per thread: the best bounds of the current row (state kept here, so the other instantiations
+                                // declare nothing new and keep their code)
+};
+
+template <typename... T>
+constexpr bool kIsResidual = (false || ... || std::is_same<T, ResidualArgs>::value);
+
+__device__ __forceinline__ ResidualArgs& residual_args(ResidualArgs& a) { return a; }
 
 // sum of v over the block in a fixed order (warp shuffles, then the warps in order); every thread receives the result
 __device__ double block_sum(double v, double* sv) {
@@ -238,6 +278,22 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
         int verdict = -1;                                   // 0 pruned, 1 kept by an LP witness, 3 undecided
         double bnd = 0.0;
         unsigned long long pivots = 0, rounds = 0;
+        if constexpr (kIsResidual<Cert...>) {
+            // the start: m* at the seed corner, u of lambda = e_{J0}; both are valid bounds whatever the LPs below do
+            ResidualArgs& g = residual_args(cert...);
+            const double* x0 = A + (size_t)cornerJ[i] * S;
+            double uv = -INFINITY;
+            int us = INT_MAX;
+            for (int s = tid; s < S; s += PL_THREADS) {
+                arg_better(uv, us, ai[s] - x0[s], s);
+                g.bstar[(size_t)i * S + s] = s == s0 ? 1.0 : 0.0;
+            }
+            block_argmax(uv, us, sv, si);
+            g.uBest = uv;
+            g.mBest = bound[i];
+            if (tid == 0) { g.certIdx[(size_t)i * J_MAX] = cornerJ[i] - g.off; g.certW[(size_t)i * J_MAX] = 1.0; }
+            if (g.uBest - g.mBest <= g.tol) verdict = 0;
+        }
         if constexpr (kIsBpi<Cert...>) {
             // the column priced at the last b*: m* = b* . (W_n - C_price) <= delta over every column <= delta_J
             const BpiArgs& g = bpi_args(cert...);
@@ -395,7 +451,16 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
             // ---- verified lower bound: m* = min over every finite j != i of b* . (alpha_i - alpha_j) ----
             double mv = -INFINITY;
             int mj = INT_MAX;
-            if constexpr (!kIsBpi<Cert...>) {
+            if constexpr (kIsResidual<Cert...>) {
+                ResidualArgs& g = residual_args(cert...);
+                for (int j = g.off + tid; j < g.off + g.nx; j += PL_THREADS) {
+                    const double* aj = A + (size_t)j * S;
+                    double v = 0.0;
+                    for (int p = 0; p < ns; p++) v = fma(suppB[p], ai[suppS[p]] - aj[suppS[p]], v);
+                    arg_better(mv, mj, -v, j);
+                }
+                block_argmax(mv, mj, sv, si);
+            } else if constexpr (!kIsBpi<Cert...>) {
                 for (int j = tid; j < n; j += PL_THREADS) {
                     if (j == i || !finite[j]) continue;
                     const double* aj = A + (size_t)j * S;
@@ -406,7 +471,7 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
                 block_argmax(mv, mj, sv, si);
             }
             const double mstar = -mv;
-            if constexpr (!kIsBpi<Cert...>) {
+            if constexpr (!kIsBpi<Cert...> && !kIsResidual<Cert...>) {
                 if (mstar > -tau) { verdict = 1; bnd = mstar; break; }
             }
             // ---- verified upper bound: u = max_s (alpha_i - sum_q lambda_q alpha_J[q])[s] ----
@@ -423,6 +488,29 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
             }
             block_argmax(uv, us, sv, si);
             if constexpr (kIsBpi<Cert...>) { verdict = 0; bnd = uv; break; }          // one LP per launch: the host prices at b*
+            if constexpr (kIsResidual<Cert...>) {
+                ResidualArgs& g = residual_args(cert...);
+                if (uv < g.uBest) {                          // k only grows: the first k entries replace the previous certificate
+                    g.uBest = uv;
+                    if (tid < k) { g.certIdx[(size_t)i * J_MAX + tid] = J[tid] - g.off; g.certW[(size_t)i * J_MAX + tid] = lam[tid]; }
+                }
+                if (mstar > g.mBest) {
+                    g.mBest = mstar;
+                    double* b = g.bstar + (size_t)i * S;
+                    for (int s = tid; s < S; s += PL_THREADS) b[s] = 0.0;
+                    __syncthreads();
+                    if (tid < ns) b[suppS[tid]] = suppB[tid];
+                }
+                if (g.uBest - g.mBest <= g.tol) { verdict = 0; break; }
+                bool inJ = false;
+                for (int q = 0; q < k; q++) inJ |= J[q] == mj;
+                if (inJ || k == J_MAX || mj == INT_MAX) { verdict = 3; break; }
+                __syncthreads();
+                if (tid == 0) J[k] = mj;
+                k++;
+                __syncthreads();
+                continue;
+            }
             if (uv < -tau) { verdict = 0; bnd = uv; break; }
             // ---- cut: the row that beats alpha_i most at b* joins J ----
             bool inJ = false;
@@ -435,6 +523,20 @@ __global__ void __launch_bounds__(PL_THREADS, 2) prune_lp_kernel(const double* _
         }
         if constexpr (kCert) {
             if (verdict == 0 && tid < k) write_certificate(cert..., i, tid, J[tid], lam[tid]);   // J and lambda of the LP that gave u
+        }
+        if constexpr (kIsResidual<Cert...>) {
+            ResidualArgs& g = residual_args(cert...);
+            if (tid == 0) {
+                g.u[i] = g.uBest;
+                g.mstar[i] = g.mBest;
+                keep[i] = verdict;
+                if (verdict != 0) atomicAdd(counts + 3, 1);
+                atomicMax(stats + 0, (unsigned long long)k);
+                atomicAdd(stats + 1, rounds);
+                atomicAdd(stats + 2, pivots);
+                atomicAdd(stats + 3, verdict != 0 ? 1ull : 0ull);
+            }
+            continue;
         }
         if constexpr (kIsBpi<Cert...>) {
             // an LP that ran out of pivots (3) or into numerical trouble (4) leaves the previous LP's outputs as they were
@@ -576,6 +678,62 @@ extern "C" int pbvi_bpi_lp(pbvi_model* m, const double* d_pool, int nP, int n, d
     prune_lp_kernel<false><<<grid, PL_THREADS, 0, st>>>(d_pool, n, m->S, nullptr, tauD, d_corner, nullptr, d_status, d_delta, counters,
                                                         counters + 1, stats, args);
     m->last_launches = 1;
+    PBVI_CUDA(cudaGetLastError());
+    unsigned long long sv[4];
+    PBVI_CUDA(cudaMemcpyAsync(sv, stats, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    PBVI_CUDA(cudaStreamSynchronize(st));
+    if (h_stats4)
+        for (int k = 0; k < 4; k++) h_stats4[k] = (long long)sv[k];
+    return PBVI_OK;
+}
+
+extern "C" int pbvi_ip_residual_lp(pbvi_model* m, const double* d_y, int ny, const double* d_x, int nx, double tau, double* d_u, double* d_mstar,
+                                   double* d_bstar, int32_t* d_cert_idx, double* d_cert_w, int64_t* h_stats4, void* stream) {
+    PBVI_REQUIRE(m != nullptr, "model handle is NULL");
+    PBVI_REQUIRE(ny >= 0 && nx >= 1, "need ny >= 0 rows to test and nx >= 1 rows to test them against");
+    PBVI_REQUIRE(tau >= 0.0 && std::isfinite(tau), "tau must be finite and >= 0");
+    if (h_stats4) std::fill(h_stats4, h_stats4 + 4, 0ll);
+    m->last_launches = 0;
+    if (ny == 0) return PBVI_OK;
+    PBVI_REQUIRE(d_y && d_x && d_u && d_mstar && d_bstar && d_cert_idx && d_cert_w, "NULL pointer argument");
+    PBVI_CUDA(cudaSetDevice(m->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PBVI_TRY(enter_call(m, st));
+    const int S = m->S, n = ny + nx;
+    PBVI_REQUIRE(n > ny, "ny + nx overflows");
+    PBVI_TAKE(pool, double, (size_t)n * S);
+    PBVI_TAKE(finite, int32_t, (size_t)n);
+    PBVI_TAKE(rowMax, double, (size_t)n);
+    PBVI_TAKE(scale, double, 1);
+    PBVI_TAKE(v1, double, (size_t)S);
+    PBVI_TAKE(v2, double, (size_t)S);
+    PBVI_TAKE(i1, int32_t, (size_t)S);
+    PBVI_TAKE(i2, int32_t, (size_t)S);
+    PBVI_TAKE(cornerS, int32_t, (size_t)ny);
+    PBVI_TAKE(cornerJ, int32_t, (size_t)ny);
+    PBVI_TAKE(verdict, int32_t, (size_t)ny);
+    PBVI_TAKE(bound, double, (size_t)ny);
+    PBVI_TAKE(counters, int, 8);                          // [0] row queue, [1..4] counts
+    PBVI_TAKE(stats, unsigned long long, 4);
+    PBVI_CUDA(cudaMemcpyAsync(pool, d_y, (size_t)ny * S * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    PBVI_CUDA(cudaMemcpyAsync(pool + (size_t)ny * S, d_x, (size_t)nx * S * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    PBVI_CUDA(cudaMemsetAsync(verdict, 0xff, (size_t)ny * sizeof(int32_t), st));        // -1: every row runs
+    PBVI_CUDA(cudaMemsetAsync(counters, 0, 8 * sizeof(int), st));
+    PBVI_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), st));
+    PBVI_CUDA(cudaMemsetAsync(d_cert_idx, 0xff, (size_t)ny * J_MAX * sizeof(int32_t), st));   // -1
+    PBVI_CUDA(cudaMemsetAsync(d_cert_w, 0, (size_t)ny * J_MAX * sizeof(double), st));
+    // the simplex works on rows scaled by max(1, max |pool|), as pbvi_prune_lp's does (its tau kernel gives 1e-9 times that)
+    prune_lp_row_stats_kernel<<<n, PL_THREADS, 0, st>>>(pool, S, finite, rowMax);
+    prune_lp_tau_kernel<<<1, PL_THREADS, 0, st>>>(rowMax, n, scale);
+    prune_lp_columns_kernel<<<ceil_div(S, PL_THREADS), PL_THREADS, 0, st>>>(pool + (size_t)ny * S, nx, S, finite + ny, v1, i1, v2, i2);
+    residual_corner_kernel<<<ny, PL_THREADS, 0, st>>>(pool, S, ny, v1, i1, cornerS, cornerJ, bound);
+    const ResidualArgs args{ny, nx, tau, d_u, d_mstar, d_bstar, d_cert_idx, d_cert_w, INFINITY, -INFINITY};
+    int perSM = 1;
+    PBVI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, prune_lp_kernel<false, ResidualArgs>, PL_THREADS, 0));
+    const int grid = std::max(1, std::min(ny, m->sm_count * std::max(perSM, 1)));
+    prune_lp_kernel<false><<<grid, PL_THREADS, 0, st>>>(pool, ny, S, finite, scale, cornerS, cornerJ, verdict, bound, counters, counters + 1,
+                                                        stats, args);
+    m->last_launches = 5;
     PBVI_CUDA(cudaGetLastError());
     unsigned long long sv[4];
     PBVI_CUDA(cudaMemcpyAsync(sv, stats, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
